@@ -3,6 +3,7 @@
 "UPOLS channel-Msamples/s (B=1024, 2^20 taps); batched FFT GB/s vs HBM peak".
 
     python bench.py --gpus N --steps K --warmup W [--frame T | --frame 0 --blocks T] [--layout GcxGp] [--impl reference]
+                    [--dump-outputs DIR]
 
 A step is one call of the convolver bank: T consecutive blocks of 1024 samples for each of the 1024 channels, each channel convolved
 with its own 2^20-tap impulse response (P = 1024 partitions) -- BASELINE config 5. T = 1 is the reference's streaming call (one block
@@ -47,6 +48,7 @@ METRIC = "UPOLS channel-Msamples/s (B=1024, 2^20 taps); batched FFT GB/s vs HBM 
 UNIT = "channel-Msamples/s"
 WORKLOAD = "C5: 1024 channels x 2^20-tap IR each, UPOLS B=1024 (P=1024, K=1025), white-noise input"
 PARITY_TOL = 1e-5  # north_star: relative L2 vs neo's own convolver, float32
+DUMP_BYTES = 32 << 20  # --dump-outputs writes at most this much output
 
 
 def measured_peaks():
@@ -532,6 +534,8 @@ def run_single(args, pkg, torch, emit, peak, peak_src):
         stop.record()
         torch.cuda.synchronize()
     ms_total = start.elapsed_time(stop)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, torch, ys)
     ms_r2c, ms_mac, ms_c2r, mac_launches = conv.profile_read()
     conv.profile(False)
     launches = pkg.kernel_launches() - launches0
@@ -676,6 +680,17 @@ def run_single(args, pkg, torch, emit, peak, peak_src):
     if configs is not None:
         line["configs"] = configs
     emit(line)
+
+
+def dump_outputs(directory: str, torch, y) -> None:
+    """--dump-outputs: what the last timed step handed back, y[channels][T*B] float32, as `directory`/output.npy. Above DUMP_BYTES
+    a fixed seeded sample of whole channel rows (ascending order) is written, and where one row alone exceeds it, each row's leading
+    samples. The inputs are seeded, so two builds run with the same arguments can be compared output for output."""
+    rows = max(1, min(y.shape[0], DUMP_BYTES // (y.shape[1] * y.element_size())))
+    cols = min(y.shape[1], DUMP_BYTES // (rows * y.element_size()))
+    pick = np.sort(np.random.default_rng(0).choice(y.shape[0], rows, replace=False))
+    os.makedirs(directory, exist_ok=True)
+    np.save(os.path.join(directory, "output.npy"), y[torch.as_tensor(pick, device=y.device), :cols].cpu().numpy())
 
 
 def ncu_traffic(key: str, scale: int = 1):
@@ -1047,7 +1062,12 @@ def main():
     ap.add_argument("--fft-only", action="store_true")
     ap.add_argument("--no-modes", action="store_true", help="skip the other call shapes / layouts")
     ap.add_argument("--no-configs", action="store_true", help="skip BASELINE configs 1, 3, 4 and the unchanged-driver run")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the convolver output of the last timed step to DIR/output.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.gpus != 1 or args.impl != "ours" or args.fft_only):
+        ap.error("--dump-outputs writes the one-GPU convolver's output: use it with --gpus 1 and --impl ours, without --fft-only")
     if args.impl == "reference":
         run_reference(args, int(os.environ.get("RANK", "0")))
     else:

@@ -159,6 +159,7 @@ def test_sparse_filters_csr_device_layout(gpu, orc, golden, block, taps, channel
     conv.reset()
     import torch
 
+    conv.set_stream(torch.cuda.current_stream())  # device buffers: the input copies and the read-backs below are on torch's stream
     x = torch.from_numpy(sigw).cuda()
     y = torch.empty_like(x[:, : 4 * 32])
     outs = []

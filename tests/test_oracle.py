@@ -1,10 +1,12 @@
 """CPU: pins the oracle (oracle/neo_oracle.c) against the reference's own known-answer tests, against golden vectors
 produced by the unmodified reference (tests/golden/neo_ref_golden.npz, oracle/make_golden.py) and, where the prebuilt
 oracle/_ref library is present, against the reference side by side."""
+import os
+
 import numpy as np
 import pytest
 
-from conftest import rel_l2
+from conftest import ROOT, rel_l2
 
 KINDS = ("upols", "upola", "split_upols", "split_upola", "upola_v2")
 
@@ -341,21 +343,15 @@ def test_overlap_policies_identity(golden):
     assert np.allclose(golden["overlap/add"], golden["overlap/signal"], atol=1e-5)
 
 
-# ---- side by side with the compiled reference, when it travelled ------------------------------------------------------------------
+# ---- side by side with the compiled reference: its stored outputs, and the library itself when it travelled ---------------------------
 def test_oracle_vs_compiled_reference(orc, ref):
-    if ref is None:
-        pytest.skip("oracle/_ref/libneo_ref.so not present")
-    for order in range(0, 13):
-        assert np.array_equal(orc.bitrev_table(order), ref.bitrev_table(order))
-    for order in (1, 4, 9, 13):
-        x = orc.noise(1 << order, 21, np.complex64)
-        assert np.array_equal(orc.fft(x, -1), ref.fft(x, -1))
-        xr = orc.noise(1 << order, 22, np.float32)
-        assert np.array_equal(orc.rfft(xr), ref.rfft(xr))
-    ir = orc.normalize_impulse(np.stack([orc.noise(700, 31 + c, np.float32) for c in range(2)]))
-    assert np.array_equal(ir, ref.normalize_impulse(np.stack([orc.noise(700, 31 + c, np.float32) for c in range(2)])))
-    H = orc.uniform_partition(ir, 64)
-    assert np.array_equal(H, ref.uniform_partition(ir, 64))
-    sig = np.stack([orc.noise(64 * 16, 41 + c, np.float32) for c in range(2)])
-    for kind in (0, 1, 4):
-        assert np.array_equal(orc.convolve_blocks(kind, H, sig), ref.convolve_blocks(kind, H, sig))
+    # tests/golden/neo_ref_side_by_side.npz holds the inputs and the compiled reference's outputs (oracle/make_golden_side_by_side.py);
+    # the oracle must reproduce them bit for bit, and so must the reference library where it is present
+    from oracle.make_golden_side_by_side import side_by_side
+
+    want = np.load(os.path.join(ROOT, "tests", "golden", "neo_ref_side_by_side.npz"))
+    for name, chk in [("oracle", orc)] + ([("reference", ref)] if ref is not None else []):
+        got = side_by_side(chk, orc.noise)
+        assert sorted(got) == sorted(want.files), name
+        for key in want.files:
+            assert np.array_equal(got[key], want[key]), (name, key)
