@@ -320,6 +320,46 @@ NEO_B200_API int neo_b200_conv_profile_read(neo_b200_conv* conv, double* phase_m
 /* bytes of device memory held by the handle (filter + FDL + scratch) */
 NEO_B200_API size_t neo_b200_conv_device_bytes(neo_b200_conv const* conv);
 
+/* ---- one-block-latency convolver: what upols_convolver computes (overlap-save, diagonal bank), at one block of latency for long
+ *      impulse responses, through non-uniform partitioning (Gardner 1995; Garcia 2002). With levels T_1 < ... < T_n (powers of two
+ *      in [2, 512], n <= 4) and P partitions:
+ *        head     partitions [0, min(2 T_1, P)): direct form, one fused kernel per block for the whole bank;
+ *        level i  partitions [2 T_i, 2 T_{i+1}) (the last one ends at P): frame mode with frame_blocks = T_i on its own stream, started
+ *                 when a frame of T_i input blocks is complete and due 2 T_i blocks after the frame began -- one frame period of slack.
+ *      Levels that would start at or past P are dropped. Results are the reference's up to rounding (a regrouping of the same sum over
+ *      partitions), independent of timing: fixed summation order, no atomics; n-block calls give the bits of n one-block calls.
+ *      Environment, read at creation: NEO_B200_LOWLAT_SYNC runs the level work on the handle's stream (same bits);
+ *      NEO_B200_LOWLAT_UNFUSED runs the head through the direct-form kernels plus a combine kernel (what block sizes outside
+ *      2^6 .. 2^12 (float) / 2^11 (double) always use). ----------------------------------------------------------------------- */
+typedef struct neo_b200_lowlat neo_b200_lowlat;
+
+typedef struct neo_b200_lowlat_config
+{
+    int dtype;               /* neo_b200_dtype */
+    size_t channels;         /* C, each with its own filter */
+    size_t block;            /* B, power of two >= 2 (the single-CTA transform range: 8192 float, 4096 double) */
+    size_t partitions;       /* P of the whole filter */
+    size_t levels;           /* 0 = library default: T_1 = 8, then x4 while 2 T_i < P */
+    size_t frame_blocks[4];  /* T_1 < ... < T_levels */
+} neo_b200_lowlat_config;
+
+/* validates `config` and resolves the schedule without touching a device: the live levels, their T, and [begin, end) partition ranges
+ * (ranges[0] = head, ranges[1 + i] = level i; unused entries 0) */
+NEO_B200_API int neo_b200_lowlat_layout(neo_b200_lowlat_config const* config, size_t* levels, size_t frame_blocks[4], size_t ranges[5][2]);
+NEO_B200_API int neo_b200_lowlat_create(neo_b200_lowlat** handle, neo_b200_lowlat_config const* config);
+NEO_B200_API void neo_b200_lowlat_destroy(neo_b200_lowlat* handle);
+/* H [channels][P][block+1] complex (uniform_partition layout) / ir [channels][taps] reals; both zero all state */
+NEO_B200_API int neo_b200_lowlat_set_filter(neo_b200_lowlat* handle, void const* H, int memspace);
+NEO_B200_API int neo_b200_lowlat_set_impulse(neo_b200_lowlat* handle, void const* ir, size_t taps, int memspace);
+NEO_B200_API int neo_b200_lowlat_reset(neo_b200_lowlat* handle);
+/* `convolver(block)` for every channel, `blocks` >= 1 consecutive blocks: in [channels][blocks*B] -> out, in == out allowed. HOST:
+ * returns with the result in `out`; DEVICE: enqueued on the handle's stream, level work continues on the handle's side streams. */
+NEO_B200_API int neo_b200_lowlat_process(neo_b200_lowlat* handle, void const* in, void* out, size_t blocks, int memspace);
+NEO_B200_API int neo_b200_lowlat_set_stream(neo_b200_lowlat* handle, void* cuda_stream);
+/* waits for the handle's stream and its side streams */
+NEO_B200_API int neo_b200_lowlat_synchronize(neo_b200_lowlat* handle);
+NEO_B200_API size_t neo_b200_lowlat_device_bytes(neo_b200_lowlat const* handle);
+
 /* ---- multi-GPU bank: one convolver bank spread over the GPUs of one box -----------------------------------------------------------
  * What a caller of the reference does with N host threads -- one private convolver per channel
  * (convolution/uniform_partitioned_convolver.hpp:28-34; extra/cli/src/convolver.cpp:37-40 builds one per channel) -- and, for one very

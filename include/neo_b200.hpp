@@ -727,6 +727,71 @@ using upols_convolver = uniform_partitioned_convolver<Complex, NEO_B200_UPOLS>;
 template<typename Complex>
 using upola_convolver = uniform_partitioned_convolver<Complex, NEO_B200_UPOLA>;
 
+/// upols_convolver<Complex>'s duck type (`filter(H[P][K])`, `operator()(block[B])` in place) at one block of latency for long impulse
+/// responses: the first partitions run per block, later stretches in frame mode on side streams (neo_b200_lowlat_*, non-uniform
+/// partitioning). Same results up to rounding. One instance = one channel; `frame_blocks` = the level frame sizes, empty = the
+/// library default.
+template<typename Complex>
+struct low_latency_convolver
+{
+    using value_type = Complex;
+    using real_type  = detail::real_of<Complex>;
+
+    low_latency_convolver() = default;
+    explicit low_latency_convolver(std::vector<std::size_t> frame_blocks) : _frame_blocks(std::move(frame_blocks)) {}
+    low_latency_convolver(low_latency_convolver const&)                    = delete;
+    auto operator=(low_latency_convolver const&) -> low_latency_convolver& = delete;
+    ~low_latency_convolver() { neo_b200_lowlat_destroy(_conv); }
+
+    template<typename Mat>
+    auto filter(Mat h) -> void
+    {
+        static_assert(std::is_same_v<detail::element_of<Mat>, Complex>);
+        auto const parts = static_cast<std::size_t>(h.extent(0));
+        auto const bins  = static_cast<std::size_t>(h.extent(1));
+        _copy.resize(parts * bins);
+        for (std::size_t p = 0; p < parts; ++p) {
+            for (std::size_t k = 0; k < bins; ++k) {
+                auto const v        = h(p, k);
+                _copy[p * bins + k] = std::complex<real_type>{v.real(), v.imag()};
+            }
+        }
+        neo_b200_lowlat_config cfg{detail::dtype_of<real_type>, 1, bins - 1, parts, _frame_blocks.size(), {0, 0, 0, 0}};
+        for (std::size_t i = 0; i < _frame_blocks.size() && i < 4; ++i) { cfg.frame_blocks[i] = _frame_blocks[i]; }
+        neo_b200_lowlat_destroy(_conv);
+        _conv = nullptr;
+        detail::check(neo_b200_lowlat_create(&_conv, &cfg));
+        detail::check(neo_b200_lowlat_set_filter(_conv, _copy.data(), NEO_B200_HOST));
+        _block = bins - 1;
+    }
+
+    template<typename Vec>
+    auto operator()(Vec block) -> void
+    {
+        static_assert(std::is_same_v<detail::element_of<Vec>, real_type>);
+        auto const n = static_cast<std::size_t>(block.extent(0));
+        if (_conv == nullptr) { throw std::invalid_argument{"neo::b200::low_latency_convolver: filter() has not been called"}; }
+        if (n != _block) { throw std::invalid_argument{"neo::b200::low_latency_convolver: block extent differs from the filter's block size"}; }
+        if (detail::is_contiguous(block)) {
+            detail::check(neo_b200_lowlat_process(_conv, block.data_handle(), block.data_handle(), 1, NEO_B200_HOST));
+        } else {
+            _tmp.resize(n);
+            for (std::size_t i = 0; i < n; ++i) { _tmp[i] = block[i]; }
+            detail::check(neo_b200_lowlat_process(_conv, _tmp.data(), _tmp.data(), 1, NEO_B200_HOST));
+            for (std::size_t i = 0; i < n; ++i) { block[i] = _tmp[i]; }
+        }
+    }
+
+    [[nodiscard]] auto device_bytes() const noexcept -> std::size_t { return _conv == nullptr ? 0 : neo_b200_lowlat_device_bytes(_conv); }
+
+private:
+    neo_b200_lowlat* _conv{nullptr};
+    std::vector<std::size_t> _frame_blocks;
+    std::size_t _block{0};
+    std::vector<std::complex<real_type>> _copy;
+    std::vector<real_type> _tmp;
+};
+
 /// Drop-in for neo::convolution::overlap_add_convolver / upola_convolver_v2 (convolution/overlap_add_convolver.hpp:21-136,
 /// dense_convolver.hpp:28): `operator()(inout)` takes ANY number of samples >= one block (:74 asserts that).
 ///   - Calls of whole blocks on a clean window -- what its test and benchmark use (uniform_partitioned_convolver_test.cpp:40,

@@ -71,6 +71,17 @@ class BankRankInfo(C.Structure):
     ]
 
 
+class LowLatConfig(C.Structure):
+    _fields_ = [
+        ("dtype", _i),
+        ("channels", _sz),
+        ("block", _sz),
+        ("partitions", _sz),
+        ("levels", _sz),
+        ("frame_blocks", _sz * 4),
+    ]
+
+
 BANK_ID_BYTES = 128
 _pp = C.POINTER(_vp)
 
@@ -146,6 +157,16 @@ SIGNATURES = {
     "neo_b200_conv_profile_enable": (_i, [_vp, _i]),
     "neo_b200_conv_profile_read": (_i, [_vp, C.POINTER(C.c_double), C.POINTER(C.c_uint64)]),
     "neo_b200_conv_device_bytes": (_sz, [_vp]),
+    "neo_b200_lowlat_layout": (_i, [C.POINTER(LowLatConfig), C.POINTER(_sz), C.POINTER(_sz), C.POINTER(_sz)]),
+    "neo_b200_lowlat_create": (_i, [C.POINTER(_vp), C.POINTER(LowLatConfig)]),
+    "neo_b200_lowlat_destroy": (None, [_vp]),
+    "neo_b200_lowlat_set_filter": (_i, [_vp, _vp, _i]),
+    "neo_b200_lowlat_set_impulse": (_i, [_vp, _vp, _sz, _i]),
+    "neo_b200_lowlat_reset": (_i, [_vp]),
+    "neo_b200_lowlat_process": (_i, [_vp, _vp, _vp, _sz, _i]),
+    "neo_b200_lowlat_set_stream": (_i, [_vp, _vp]),
+    "neo_b200_lowlat_synchronize": (_i, [_vp]),
+    "neo_b200_lowlat_device_bytes": (_sz, [_vp]),
     "neo_b200_bank_unique_id": (_i, [_vp]),
     "neo_b200_bank_create": (_i, [C.POINTER(_vp), C.POINTER(ConvConfig), C.POINTER(BankLayout), C.POINTER(_i), _sz]),
     "neo_b200_bank_create_rank": (_i, [C.POINTER(_vp), C.POINTER(ConvConfig), C.POINTER(BankLayout), _i, _i, _i, _vp]),
@@ -730,6 +751,105 @@ class Convolver:
     def close(self) -> None:
         if self._h:
             library().neo_b200_conv_destroy(self._h)
+            self._h = _vp()
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
+
+
+class LowLatencyConvolver:
+    """A bank of upols_convolver instances at ONE block of latency for long impulse responses (include/neo_b200.h:
+    neo_b200_lowlat_*): the first partitions run per block, later stretches in frame mode on side streams (non-uniform
+    partitioning). `filter(H)` / `impulse(ir, block)` then call on any whole number of blocks.
+
+    frame_blocks: the level frame sizes T_1 < ... < T_n (powers of two in [2, 512], n <= 4); None = the library default.
+    """
+
+    def __init__(self, dtype="float32", frame_blocks=None):
+        self.real = _REAL_OF[str(np.dtype(dtype))]
+        self.frame_blocks = tuple(int(t) for t in frame_blocks) if frame_blocks else ()
+        self._h = _vp()
+        self.cfg = None
+        self._stream = None
+
+    @staticmethod
+    def _config(dtype_code: int, channels: int, block: int, partitions: int, frame_blocks) -> LowLatConfig:
+        fb = tuple(frame_blocks or ())
+        arr = (_sz * 4)(*(list(fb[:4]) + [0] * (4 - len(fb[:4]))))  # more than 4 levels: the library reports it
+        return LowLatConfig(dtype_code, channels, block, partitions, len(fb), arr)
+
+    @staticmethod
+    def layout(partitions: int, block: int, frame_blocks=None, dtype="float32") -> dict:
+        """The schedule the library builds, without a device: {"frame_blocks": (T_1, ...), "head": (0, e),
+        "levels": [(begin, end), ...]} -- levels that would start at or past `partitions` are dropped."""
+        cfg = LowLatencyConvolver._config(_DTYPE_CODE[_REAL_OF[str(np.dtype(dtype))]], 1, block, partitions, frame_blocks)
+        n = _sz(0)
+        fb = (_sz * 4)()
+        ranges = (_sz * 10)()
+        _check(library().neo_b200_lowlat_layout(C.byref(cfg), C.byref(n), fb, ranges))
+        n = int(n.value)
+        return {
+            "frame_blocks": tuple(int(fb[i]) for i in range(n)),
+            "head": (int(ranges[0]), int(ranges[1])),
+            "levels": [(int(ranges[2 + 2 * i]), int(ranges[3 + 2 * i])) for i in range(n)],
+        }
+
+    def _create(self, channels, block, partitions):
+        self.close()
+        self.cfg = self._config(_DTYPE_CODE[self.real], channels, block, partitions, self.frame_blocks)
+        _check(library().neo_b200_lowlat_create(C.byref(self._h), C.byref(self.cfg)))
+        if self._stream is not None:
+            _check(library().neo_b200_lowlat_set_stream(self._h, self._stream))
+
+    def filter(self, H) -> None:
+        """H [C][P][B+1] (uniform_partition layout): deep copy, state zeroed."""
+        if H.ndim != 3:
+            raise ValueError("filter must be [channels][partitions][block+1]")
+        if _dtype_name(H) != ("complex64" if self.real == "float32" else "complex128"):
+            raise ValueError("filter dtype does not match the convolver")
+        self._create(int(H.shape[0]), int(H.shape[2]) - 1, int(H.shape[1]))
+        _check(library().neo_b200_lowlat_set_filter(self._h, _ptr(H), _space(H)))
+
+    def impulse(self, ir, block: int) -> None:
+        """filter(uniform_partition(ir, block)) without materialising H on the host. ir: [C][L]."""
+        if ir.ndim != 2 or _dtype_name(ir) != self.real:
+            raise ValueError("impulse response shape/dtype mismatch")
+        taps = int(ir.shape[1])
+        self._create(int(ir.shape[0]), block, num_partitions(taps, block))
+        _check(library().neo_b200_lowlat_set_impulse(self._h, _ptr(ir), taps, _space(ir)))
+
+    def set_stream(self, stream) -> None:
+        self._stream = _stream_ptr(stream)
+        if self._h:
+            _check(library().neo_b200_lowlat_set_stream(self._h, self._stream))
+
+    def synchronize(self) -> None:
+        _check(library().neo_b200_lowlat_synchronize(self._h))
+
+    def reset(self) -> None:
+        _check(library().neo_b200_lowlat_reset(self._h))
+
+    def device_bytes(self) -> int:
+        return int(library().neo_b200_lowlat_device_bytes(self._h))
+
+    def __call__(self, x, out=None):
+        """convolver(block) for every channel: x [C][n*B] processed as n blocks; in place when out is None."""
+        if self.cfg is None:
+            raise RuntimeError("no filter set")
+        block = int(self.cfg.block)
+        if x.ndim != 2 or x.shape[0] != self.cfg.channels or x.shape[1] % block != 0 or _dtype_name(x) != self.real:
+            raise ValueError(f"expected {self.real}[{self.cfg.channels}][n*{block}]")
+        if out is None:
+            out = x
+        _check(library().neo_b200_lowlat_process(self._h, _ptr(x), _ptr(out), x.shape[1] // block, _space(x)))
+        return out
+
+    def close(self) -> None:
+        if self._h:
+            library().neo_b200_lowlat_destroy(self._h)
             self._h = _vp()
 
     def __del__(self):

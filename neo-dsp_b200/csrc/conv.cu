@@ -3,6 +3,7 @@
 // (src/neo/convolution/uniform_partitioned_convolver.hpp:14-65, dense_convolver.hpp:20-25) and
 // neo::convolution::uniform_partition (uniform_partition.hpp:13-26).
 #include "conv_frame.cuh"
+#include "conv_lowlat.cuh"
 #include "fft_wide.cuh"
 
 #include <algorithm>
@@ -1685,6 +1686,394 @@ int neo_b200_fdl_index_sequence(size_t parts, size_t calls, uint32_t* write_pos,
     NEO_TRY(check_launch("fdl_index_kernel"));
     NEO_TRY(table_to_host(wp, write_pos, calls));
     return table_to_host(pr, pairs, n * 2);
+}
+
+}  // extern "C"
+
+// ---- one-block-latency convolver (neo_b200_lowlat_*): head kernel per block, frame-mode levels on side streams ----------------------
+namespace neo_b200 {
+namespace {
+
+constexpr size_t k_lowlat_default_t1    = 8;
+constexpr size_t k_lowlat_default_ratio = 4;  // T_1 x {4, 8} x {2, 4, 8, 16} on C5: 8, 32, 128 was fastest (DESIGN §4.7)
+
+// validates the configuration, resolves the default schedule and yields the head range (ranges[0]) and one range per live level
+int lowlat_resolve(neo_b200_lowlat_config const* c, size_t* levels, size_t fb[k_lowlat_max_levels], size_t ranges[k_lowlat_max_levels + 1][2])
+{
+    if (c == nullptr) { return fail(NEO_B200_ERR_INVALID, "null argument"); }
+    if (c->dtype != NEO_B200_F32 && c->dtype != NEO_B200_F64) { return fail(NEO_B200_ERR_INVALID, "bad dtype %d", c->dtype); }
+    if (c->channels == 0 || c->channels > 65535) { return fail(NEO_B200_ERR_INVALID, "channels must be in [1, 65535], got %zu", c->channels); }
+    size_t const max_block = size_t(1) << (c->dtype == NEO_B200_F32 ? max_cta_logm<float>() : max_cta_logm<double>());
+    if (!is_pow2(c->block) || c->block < 2 || c->block > max_block) {
+        return fail(NEO_B200_ERR_INVALID, "block size must be a power of two in [2, %zu], got %zu", max_block, c->block);
+    }
+    if (c->partitions == 0 || c->partitions > (size_t(1) << 30)) { return fail(NEO_B200_ERR_INVALID, "partitions must be in [1, 2^30]"); }
+    if (c->levels > size_t(k_lowlat_max_levels)) {
+        return fail(NEO_B200_ERR_INVALID, "at most %d levels, got %zu", k_lowlat_max_levels, c->levels);
+    }
+    size_t const P = c->partitions;
+    size_t t[k_lowlat_max_levels] = {};
+    size_t n                      = c->levels;
+    if (n == 0) {  // library default: T_1 = 8, times 4 while the level would start inside the filter
+        for (size_t v = k_lowlat_default_t1; v <= k_max_frame_blocks && n < size_t(k_lowlat_max_levels) && 2 * v < P; v *= k_lowlat_default_ratio) {
+            t[n++] = v;
+        }
+    } else {
+        for (size_t i = 0; i < n; ++i) {
+            t[i] = c->frame_blocks[i];
+            if (!is_pow2(t[i]) || t[i] < 2 || t[i] > k_max_frame_blocks) {
+                return fail(NEO_B200_ERR_INVALID, "frame_blocks[%zu] must be a power of two in [2, %zu], got %zu", i, k_max_frame_blocks, t[i]);
+            }
+            if (i > 0 && t[i] <= t[i - 1]) {
+                return fail(NEO_B200_ERR_INVALID, "frame_blocks must increase: frame_blocks[%zu]=%zu after %zu", i, t[i], t[i - 1]);
+            }
+        }
+    }
+    size_t live = 0;
+    while (live < n && 2 * t[live] < P) { ++live; }  // levels that would start at or past the end of the filter are dropped
+    size_t const t1 = n > 0 ? t[0] : k_lowlat_default_t1;
+    ranges[0][0]    = 0;
+    ranges[0][1]    = std::min(2 * t1, P);
+    for (size_t i = 0; i < size_t(k_lowlat_max_levels); ++i) {
+        fb[i]            = i < live ? t[i] : 0;
+        ranges[i + 1][0] = i < live ? 2 * t[i] : 0;
+        ranges[i + 1][1] = i < live ? (i + 1 < live ? 2 * t[i + 1] : P) : 0;
+    }
+    *levels = live;
+    return NEO_B200_OK;
+}
+
+template<typename T>
+struct lowlat_state
+{
+    conv_engine<T> head;                       // direct form over the head partitions (filter, delay line, half-window)
+    conv_engine<T> level[k_lowlat_max_levels];  // frame mode, input_delayed, partitions [2 T_i, end_i)
+    device_buffer in_ring;                     // [C][2 T_n][B] the last 2 T_n input blocks: every level's frame is contiguous
+    device_buffer plane[k_lowlat_max_levels];  // [C][2 T_i][B] level i's partial output of block t at slot t mod 2 T_i
+    device_buffer head_y, stage_in, stage_out; // unfused head output; HOST staging
+
+    size_t device_bytes(size_t levels) const
+    {
+        size_t n = head.device_bytes() + in_ring.bytes + head_y.bytes + stage_in.bytes + stage_out.bytes;
+        for (size_t i = 0; i < levels; ++i) { n += level[i].device_bytes() + plane[i].bytes; }
+        return n;
+    }
+};
+
+}  // namespace
+}  // namespace neo_b200
+
+struct neo_b200_lowlat
+{
+    neo_b200_lowlat_config cfg{};
+    size_t levels{0};
+    size_t t[k_lowlat_max_levels]{};
+    size_t ranges[k_lowlat_max_levels + 1][2]{};
+    size_t ring_blocks{1};  // 2 T_n
+    int device{0};
+    stream_ref stream;      // the head's stream (highest priority when the handle creates it)
+    cudaStream_t side[k_lowlat_max_levels]{};
+    cudaEvent_t ready[k_lowlat_max_levels]{};    // recorded on the head's stream when a level's frame is complete
+    cudaEvent_t done[k_lowlat_max_levels][2]{};  // level i's frame f is in its plane: done[i][f % 2]
+    bool sync{false};       // NEO_B200_LOWLAT_SYNC: level work on the head's stream
+    bool fused{false};      // lowlat_head_kernel; else the head engine + lowlat_combine_kernel (NEO_B200_LOWLAT_UNFUSED)
+    bool has_filter{false};
+    size_t block_pos{0};    // blocks since the last reset
+    lowlat_state<float> f32;
+    lowlat_state<double> f64;
+
+    int sync_all()
+    {
+        NEO_CUDA_TRY(cudaStreamSynchronize(stream.stream));
+        for (size_t i = 0; i < levels; ++i) { NEO_CUDA_TRY(cudaStreamSynchronize(side[i])); }
+        return NEO_B200_OK;
+    }
+
+    ~neo_b200_lowlat()
+    {
+        if (stream.stream != nullptr) { cudaStreamSynchronize(stream.stream); }
+        for (size_t i = 0; i < size_t(k_lowlat_max_levels); ++i) {
+            if (side[i] != nullptr) {
+                cudaStreamSynchronize(side[i]);
+                cudaStreamDestroy(side[i]);
+            }
+            for (cudaEvent_t ev : {ready[i], done[i][0], done[i][1]}) {
+                if (ev != nullptr) { cudaEventDestroy(ev); }
+            }
+        }
+    }
+};
+
+namespace neo_b200 {
+namespace {
+
+template<typename T>
+lowlat_state<T>& lowlat_of(neo_b200_lowlat* h);
+template<>
+lowlat_state<float>& lowlat_of<float>(neo_b200_lowlat* h) { return h->f32; }
+template<>
+lowlat_state<double>& lowlat_of<double>(neo_b200_lowlat* h) { return h->f64; }
+
+template<typename T>
+int lowlat_init(neo_b200_lowlat* h)
+{
+    lowlat_state<T>& s   = lowlat_of<T>(h);
+    cudaStream_t const st = h->stream.stream;
+    size_t const C = h->cfg.channels, B = h->cfg.block;
+    neo_b200_conv_config hc{NEO_B200_UPOLS, h->cfg.dtype, NEO_B200_DIAGONAL, C, C, B, h->cfg.partitions, 1, 0, h->ranges[0][1], 0, 0};
+    NEO_TRY(validate(hc));
+    NEO_TRY(s.head.init(hc, st));
+    for (size_t i = 0; i < h->levels; ++i) {
+        neo_b200_conv_config lc{NEO_B200_UPOLS, h->cfg.dtype, NEO_B200_DIAGONAL, C, C, B, h->cfg.partitions, h->t[i],
+                                h->ranges[i + 1][0], h->ranges[i + 1][1], h->t[i], 1};
+        NEO_TRY(validate(lc));
+        NEO_TRY(s.level[i].init(lc, st));
+        NEO_TRY(s.plane[i].reserve(C * 2 * h->t[i] * B * sizeof(T)));
+    }
+    NEO_TRY(s.in_ring.reserve(C * h->ring_blocks * B * sizeof(T)));
+    if (!h->fused) { NEO_TRY(s.head_y.reserve(C * B * sizeof(T))); }
+    return NEO_B200_OK;
+}
+
+// zero every piece of stream state; the caller has synchronised the side streams
+template<typename T>
+int lowlat_clear(neo_b200_lowlat* h)
+{
+    lowlat_state<T>& s   = lowlat_of<T>(h);
+    cudaStream_t const st = h->stream.stream;
+    NEO_TRY(s.head.clear_state(st));
+    for (size_t i = 0; i < h->levels; ++i) {
+        NEO_TRY(s.level[i].clear_state(st));
+        NEO_CUDA_TRY(cudaMemsetAsync(s.plane[i].ptr, 0, s.plane[i].bytes, st));
+    }
+    NEO_CUDA_TRY(cudaMemsetAsync(s.in_ring.ptr, 0, s.in_ring.bytes, st));
+    h->block_pos = 0;
+    NEO_CUDA_TRY(cudaStreamSynchronize(st));
+    return NEO_B200_OK;
+}
+
+template<typename T, int LOGM>
+int lowlat_launch_head(lowlat_head_args<T> const& a, conv_engine<T> const& head, cudaStream_t st)
+{
+    using cfg   = fft_cfg<T, LOGM>;
+    auto kernel = lowlat_head_kernel<T, LOGM>;
+    NEO_TRY(enable_smem(kernel, cfg::SMEM));
+    kernel<<<unsigned((a.channels + cfg::G - 1) / cfg::G), cfg::THREADS, cfg::SMEM, st>>>(a, head.tables.tw(), head.tables.rtw());
+    return check_launch("lowlat_head_kernel");
+}
+
+// one block for every channel: `in` / `out` point at the block of channel 0
+template<typename T>
+int lowlat_block(neo_b200_lowlat* h, T const* in, size_t in_stride, T* out, size_t out_stride)
+{
+    lowlat_state<T>& s   = lowlat_of<T>(h);
+    cudaStream_t const st = h->stream.stream;
+    size_t const C = h->cfg.channels, B = h->cfg.block, tb = h->block_pos;
+
+    // the partial output of level i for block tb comes from its frame tb / T_i - 2
+    lowlat_levels<T> lv{};
+    lv.count = int(h->levels);
+    for (size_t i = 0; i < h->levels; ++i) {
+        size_t const ti = h->t[i];
+        if (!h->sync && tb % ti == 0 && tb >= 2 * ti) { NEO_CUDA_TRY(cudaStreamWaitEvent(st, h->done[i][(tb / ti - 2) & 1], 0)); }
+        lv.plane[i]  = s.plane[i].template as<T>() + (tb % (2 * ti)) * B;
+        lv.stride[i] = 2 * ti * B;
+    }
+    T* const ring_slot       = s.in_ring.template as<T>() + (tb % h->ring_blocks) * B;
+    size_t const ring_stride = h->ring_blocks * B;
+
+    if (h->fused) {
+        conv_engine<T>& e = s.head;
+        lowlat_head_args<T> a{in, in_stride, out, out_stride, e.prev[e.prev_flip].template as<T>(), e.prev[e.prev_flip ^ 1].template as<T>(),
+                              ring_slot, ring_stride, e.fdl.template as<cx<T>>(), e.filter.template as<cx<T>>(), e.ring, int(e.write_pos),
+                              e.parts, e.logw, C, lv};
+        int status = NEO_B200_ERR_UNSUPPORTED;
+        NEO_DISPATCH_LOGM(T, e.logb, {
+            if constexpr (LOGM >= 6 && LOGM <= (sizeof(T) == 4 ? 12 : 11)) { status = lowlat_launch_head<T, LOGM>(a, e, st); }
+        });
+        if (status != NEO_B200_OK) { return status == NEO_B200_ERR_UNSUPPORTED ? fail(status, "fused head: block %zu not covered", B) : status; }
+        e.advance(1);
+    } else {
+        conv_engine<T>& e = s.head;
+        NEO_TRY(e.forward(in, in_stride, 1, st));
+        NEO_TRY(e.inverse(static_cast<cx<T> const*>(e.acc_r()), 0, 1, s.head_y.template as<T>(), B, 0, C, 1, st));
+        dim3 const grid(unsigned((B + 255) / 256), unsigned(C));
+        lowlat_combine_kernel<T><<<grid, 256, 0, st>>>(s.head_y.template as<T>(), int(B), in, in_stride, out, out_stride, ring_slot, ring_stride, lv);
+        NEO_TRY(check_launch("lowlat_combine_kernel"));
+    }
+    h->block_pos = tb + 1;
+
+    // Levels whose frame this block completes. Frame f of level i (blocks f T_i .. f T_i + T_i - 1) runs on side stream i behind
+    // `ready` and yields the partial output of blocks (f + 2) T_i .. (f + 3) T_i - 1 into plane slots (f % 2) T_i ..; the head waits for
+    // done[i][f % 2] before block (f + 2) T_i. No slot is overwritten while it is still being read:
+    //   - input ring: the head rewrites the slot of block b at block b + 2 T_n >= (f + 2) T_i, i.e. after its wait for the reader;
+    //   - plane slot (f % 2): its previous readers are the head blocks f T_i .. f T_i + T_i - 1 (frame f - 2's output), all enqueued on
+    //     the head's stream before `ready`;
+    //   - done[i][f % 2] is re-recorded for frame f + 2 only after the head's wait for frame f has been enqueued.
+    // Every kernel sums in a fixed order and none uses atomics, so the bits do not depend on how the streams interleave
+    // (NEO_B200_LOWLAT_SYNC runs the same kernels on the head's stream).
+    for (size_t i = 0; i < h->levels; ++i) {
+        size_t const ti = h->t[i];
+        if ((tb + 1) % ti != 0) { continue; }
+        size_t const f      = tb / ti;
+        cudaStream_t const ls = h->sync ? st : h->side[i];
+        if (!h->sync) {
+            NEO_CUDA_TRY(cudaEventRecord(h->ready[i], st));
+            NEO_CUDA_TRY(cudaStreamWaitEvent(ls, h->ready[i], 0));
+        }
+        conv_engine<T>& e = s.level[i];
+        NEO_TRY(e.forward(s.in_ring.template as<T>() + ((f * ti) % h->ring_blocks) * B, ring_stride, ti, ls));
+        NEO_TRY(e.inverse(static_cast<cx<T> const*>(e.acc_r()), 0, 1, s.plane[i].template as<T>() + (f % 2) * ti * B, 2 * ti * B, 0, C, ti, ls));
+        if (!h->sync) { NEO_CUDA_TRY(cudaEventRecord(h->done[i][f & 1], ls)); }
+    }
+    return NEO_B200_OK;
+}
+
+template<typename T>
+int lowlat_process(neo_b200_lowlat* h, void const* in, void* out, size_t blocks, int memspace)
+{
+    lowlat_state<T>& s   = lowlat_of<T>(h);
+    cudaStream_t const st = h->stream.stream;
+    size_t const B = h->cfg.block, stride = blocks * B, bytes = h->cfg.channels * stride * sizeof(T);
+    T const* din = static_cast<T const*>(in);
+    T* dout      = static_cast<T*>(out);
+    if (memspace == NEO_B200_HOST) {
+        NEO_TRY(s.stage_in.reserve(bytes));
+        NEO_TRY(s.stage_out.reserve(bytes));
+        NEO_CUDA_TRY(cudaMemcpyAsync(s.stage_in.ptr, in, bytes, cudaMemcpyHostToDevice, st));
+        din  = s.stage_in.template as<T>();
+        dout = s.stage_out.template as<T>();
+    }
+    for (size_t b = 0; b < blocks; ++b) { NEO_TRY(lowlat_block<T>(h, din + b * B, stride, dout + b * B, stride)); }
+    if (memspace == NEO_B200_HOST) {
+        NEO_CUDA_TRY(cudaMemcpyAsync(out, dout, bytes, cudaMemcpyDeviceToHost, st));
+        NEO_CUDA_TRY(cudaStreamSynchronize(st));
+    }
+    return NEO_B200_OK;
+}
+
+}  // namespace
+}  // namespace neo_b200
+
+extern "C" {
+
+int neo_b200_lowlat_layout(neo_b200_lowlat_config const* config, size_t* levels, size_t frame_blocks[4], size_t ranges[5][2])
+{
+    if (levels == nullptr || frame_blocks == nullptr || ranges == nullptr) { return fail(NEO_B200_ERR_INVALID, "null argument"); }
+    return lowlat_resolve(config, levels, frame_blocks, ranges);
+}
+
+int neo_b200_lowlat_create(neo_b200_lowlat** handle, neo_b200_lowlat_config const* config)
+{
+    if (handle == nullptr) { return fail(NEO_B200_ERR_INVALID, "null argument"); }
+    *handle = nullptr;
+    auto p  = std::unique_ptr<neo_b200_lowlat>(new (std::nothrow) neo_b200_lowlat{});
+    if (!p) { return fail(NEO_B200_ERR_ALLOC, "out of host memory"); }
+    NEO_TRY(lowlat_resolve(config, &p->levels, p->t, p->ranges));
+    p->cfg         = *config;
+    p->ring_blocks = p->levels > 0 ? 2 * p->t[p->levels - 1] : 1;
+    p->sync        = std::getenv("NEO_B200_LOWLAT_SYNC") != nullptr;
+    int const logb = int(log2_exact(config->block));
+    p->fused       = logb >= 6 && logb <= (config->dtype == NEO_B200_F32 ? 12 : 11) && std::getenv("NEO_B200_LOWLAT_UNFUSED") == nullptr;
+    NEO_TRY(require_device());
+    NEO_CUDA_TRY(cudaGetDevice(&p->device));
+    // the head is due every block, so its stream has the highest priority; smaller levels (due sooner) above larger ones
+    int least = 0, greatest = 0;
+    NEO_CUDA_TRY(cudaDeviceGetStreamPriorityRange(&least, &greatest));
+    NEO_CUDA_TRY(cudaStreamCreateWithPriority(&p->stream.stream, cudaStreamNonBlocking, greatest));
+    p->stream.owned = true;
+    for (size_t i = 0; i < p->levels; ++i) {
+        int const prio = std::min(least, greatest + 1 + int(i));
+        NEO_CUDA_TRY(cudaStreamCreateWithPriority(&p->side[i], cudaStreamNonBlocking, prio));
+        for (cudaEvent_t* ev : {&p->ready[i], &p->done[i][0], &p->done[i][1]}) { NEO_CUDA_TRY(cudaEventCreateWithFlags(ev, cudaEventDisableTiming)); }
+    }
+    NEO_TRY(config->dtype == NEO_B200_F32 ? lowlat_init<float>(p.get()) : lowlat_init<double>(p.get()));
+    NEO_CUDA_TRY(cudaStreamSynchronize(p->stream.stream));
+    *handle = p.release();
+    return NEO_B200_OK;
+}
+
+void neo_b200_lowlat_destroy(neo_b200_lowlat* handle) { delete handle; }
+
+extern "C++" template<typename T>
+int lowlat_set_filter_impl(neo_b200_lowlat* h, void const* H, void const* ir, size_t taps, int memspace)
+{
+    lowlat_state<T>& s   = lowlat_of<T>(h);
+    cudaStream_t const st = h->stream.stream;
+    NEO_TRY(h->sync_all());
+    h->has_filter = false;
+    if (ir != nullptr) {
+        NEO_TRY(s.head.set_impulse(ir, taps, memspace, st));
+        for (size_t i = 0; i < h->levels; ++i) { NEO_TRY(s.level[i].set_impulse(ir, taps, memspace, st)); }
+    } else {
+        NEO_TRY(s.head.set_filter(H, memspace, st));
+        for (size_t i = 0; i < h->levels; ++i) { NEO_TRY(s.level[i].set_filter(H, memspace, st)); }
+    }
+    NEO_TRY(lowlat_clear<T>(h));
+    h->has_filter = true;
+    return NEO_B200_OK;
+}
+
+int neo_b200_lowlat_set_filter(neo_b200_lowlat* handle, void const* H, int memspace)
+{
+    if (handle == nullptr || H == nullptr) { return fail(NEO_B200_ERR_INVALID, "null argument"); }
+    NEO_CUDA_TRY(cudaSetDevice(handle->device));
+    if (handle->cfg.dtype == NEO_B200_F32) { return lowlat_set_filter_impl<float>(handle, H, nullptr, 0, memspace); }
+    return lowlat_set_filter_impl<double>(handle, H, nullptr, 0, memspace);
+}
+
+int neo_b200_lowlat_set_impulse(neo_b200_lowlat* handle, void const* ir, size_t taps, int memspace)
+{
+    if (handle == nullptr || ir == nullptr) { return fail(NEO_B200_ERR_INVALID, "null argument"); }
+    if (taps < handle->cfg.block) { return fail(NEO_B200_ERR_INVALID, "impulse response shorter than one block"); }
+    if (neo_b200_num_partitions(taps, handle->cfg.block) != handle->cfg.partitions) {
+        return fail(NEO_B200_ERR_INVALID, "taps=%zu gives %zu partitions, handle was created for %zu", taps,
+                    neo_b200_num_partitions(taps, handle->cfg.block), handle->cfg.partitions);
+    }
+    NEO_CUDA_TRY(cudaSetDevice(handle->device));
+    if (handle->cfg.dtype == NEO_B200_F32) { return lowlat_set_filter_impl<float>(handle, nullptr, ir, taps, memspace); }
+    return lowlat_set_filter_impl<double>(handle, nullptr, ir, taps, memspace);
+}
+
+int neo_b200_lowlat_reset(neo_b200_lowlat* handle)
+{
+    if (handle == nullptr) { return fail(NEO_B200_ERR_INVALID, "null argument"); }
+    NEO_CUDA_TRY(cudaSetDevice(handle->device));
+    NEO_TRY(handle->sync_all());
+    return handle->cfg.dtype == NEO_B200_F32 ? lowlat_clear<float>(handle) : lowlat_clear<double>(handle);
+}
+
+int neo_b200_lowlat_process(neo_b200_lowlat* handle, void const* in, void* out, size_t blocks, int memspace)
+{
+    if (handle == nullptr) { return fail(NEO_B200_ERR_INVALID, "null argument"); }
+    if (!handle->has_filter) { return fail(NEO_B200_ERR_INVALID, "no filter set"); }
+    if (in == nullptr || out == nullptr) { return fail(NEO_B200_ERR_INVALID, "null buffer"); }
+    if (blocks == 0) { return fail(NEO_B200_ERR_INVALID, "blocks must be >= 1"); }
+    NEO_CUDA_TRY(cudaSetDevice(handle->device));
+    if (handle->cfg.dtype == NEO_B200_F32) { return lowlat_process<float>(handle, in, out, blocks, memspace); }
+    return lowlat_process<double>(handle, in, out, blocks, memspace);
+}
+
+int neo_b200_lowlat_set_stream(neo_b200_lowlat* handle, void* cuda_stream)
+{
+    if (handle == nullptr) { return fail(NEO_B200_ERR_INVALID, "null argument"); }
+    NEO_CUDA_TRY(cudaSetDevice(handle->device));
+    NEO_CUDA_TRY(cudaStreamSynchronize(handle->stream.stream));  // work already enqueued stays ordered before the new stream's
+    handle->stream.adopt(cuda_stream);
+    return NEO_B200_OK;
+}
+
+int neo_b200_lowlat_synchronize(neo_b200_lowlat* handle)
+{
+    if (handle == nullptr) { return fail(NEO_B200_ERR_INVALID, "null argument"); }
+    NEO_CUDA_TRY(cudaSetDevice(handle->device));
+    return handle->sync_all();
+}
+
+size_t neo_b200_lowlat_device_bytes(neo_b200_lowlat const* handle)
+{
+    if (handle == nullptr) { return 0; }
+    return handle->cfg.dtype == NEO_B200_F32 ? handle->f32.device_bytes(handle->levels) : handle->f64.device_bytes(handle->levels);
 }
 
 }  // extern "C"
