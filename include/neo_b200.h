@@ -348,13 +348,24 @@ typedef struct neo_b200_lowlat_config
 NEO_B200_API int neo_b200_lowlat_layout(neo_b200_lowlat_config const* config, size_t* levels, size_t frame_blocks[4], size_t ranges[5][2]);
 NEO_B200_API int neo_b200_lowlat_create(neo_b200_lowlat** handle, neo_b200_lowlat_config const* config);
 NEO_B200_API void neo_b200_lowlat_destroy(neo_b200_lowlat* handle);
-/* H [channels][P][block+1] complex (uniform_partition layout) / ir [channels][taps] reals; both zero all state */
+/* H [channels][P][block+1] complex (uniform_partition layout) / ir [channels][taps] reals; both zero all state (reset too, including the
+ * samples of a block that neo_b200_lowlat_process_samples left pending) */
 NEO_B200_API int neo_b200_lowlat_set_filter(neo_b200_lowlat* handle, void const* H, int memspace);
 NEO_B200_API int neo_b200_lowlat_set_impulse(neo_b200_lowlat* handle, void const* ir, size_t taps, int memspace);
 NEO_B200_API int neo_b200_lowlat_reset(neo_b200_lowlat* handle);
 /* `convolver(block)` for every channel, `blocks` >= 1 consecutive blocks: in [channels][blocks*B] -> out, in == out allowed. HOST:
- * returns with the result in `out`; DEVICE: enqueued on the handle's stream, level work continues on the handle's side streams. */
+ * returns with the result in `out`; DEVICE: enqueued on the handle's stream, level work continues on the handle's side streams.
+ * Exactly neo_b200_lowlat_process_samples(handle, in, out, blocks*B, memspace): on a handle that process_samples left inside a block
+ * the calls stay aligned to the stream, not to blocks (the first block of the call completes the pending one). */
 NEO_B200_API int neo_b200_lowlat_process(neo_b200_lowlat* handle, void const* in, void* out, size_t blocks, int memspace);
+/* any `samples` >= 1 for every channel: in [channels][samples] -> out, in == out allowed, memory kinds as neo_b200_lowlat_process.
+ * out[c][t] = sum_k h[c][k] in[c][t - k] over the whole stream since the last reset / set_filter / set_impulse, up to rounding, returned
+ * by the call that delivers in[c][t]: no latency beyond the call itself. The handle keeps its position inside the current block; a call
+ * that ends inside a block costs one head kernel whatever its length (no level work; DESIGN §4.7 has the measured cost). Bits: whole-block
+ * calls give the bits of neo_b200_lowlat_process; the segment of a call that completes a block is the whole-block computation, so its
+ * samples and all state at every block boundary are those of whole-block calls however the block was split; outputs of a segment that
+ * ends inside a block match to rounding only. */
+NEO_B200_API int neo_b200_lowlat_process_samples(neo_b200_lowlat* handle, void const* in, void* out, size_t samples, int memspace);
 NEO_B200_API int neo_b200_lowlat_set_stream(neo_b200_lowlat* handle, void* cuda_stream);
 /* waits for the handle's stream and its side streams */
 NEO_B200_API int neo_b200_lowlat_synchronize(neo_b200_lowlat* handle);

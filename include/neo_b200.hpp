@@ -730,7 +730,8 @@ using upola_convolver = uniform_partitioned_convolver<Complex, NEO_B200_UPOLA>;
 /// upols_convolver<Complex>'s duck type (`filter(H[P][K])`, `operator()(block[B])` in place) at one block of latency for long impulse
 /// responses: the first partitions run per block, later stretches in frame mode on side streams (neo_b200_lowlat_*, non-uniform
 /// partitioning). Same results up to rounding. One instance = one channel; `frame_blocks` = the level frame sizes, empty = the
-/// library default.
+/// library default. `process(samples)` takes any number of samples >= 1 in place and returns each output in the call that delivers
+/// its input (neo_b200_lowlat_process_samples): what a plugin host's varying buffer size needs, with no FIFO in front.
 template<typename Complex>
 struct low_latency_convolver
 {
@@ -779,6 +780,23 @@ struct low_latency_convolver
             for (std::size_t i = 0; i < n; ++i) { _tmp[i] = block[i]; }
             detail::check(neo_b200_lowlat_process(_conv, _tmp.data(), _tmp.data(), 1, NEO_B200_HOST));
             for (std::size_t i = 0; i < n; ++i) { block[i] = _tmp[i]; }
+        }
+    }
+
+    template<typename Vec>
+    auto process(Vec samples) -> void
+    {
+        static_assert(std::is_same_v<detail::element_of<Vec>, real_type>);
+        auto const n = static_cast<std::size_t>(samples.extent(0));
+        if (_conv == nullptr) { throw std::invalid_argument{"neo::b200::low_latency_convolver: filter() has not been called"}; }
+        if (n == 0) { throw std::invalid_argument{"neo::b200::low_latency_convolver: process() needs at least one sample"}; }
+        if (detail::is_contiguous(samples)) {
+            detail::check(neo_b200_lowlat_process_samples(_conv, samples.data_handle(), samples.data_handle(), n, NEO_B200_HOST));
+        } else {
+            _tmp.resize(n);
+            for (std::size_t i = 0; i < n; ++i) { _tmp[i] = samples[i]; }
+            detail::check(neo_b200_lowlat_process_samples(_conv, _tmp.data(), _tmp.data(), n, NEO_B200_HOST));
+            for (std::size_t i = 0; i < n; ++i) { samples[i] = _tmp[i]; }
         }
     }
 

@@ -164,6 +164,7 @@ SIGNATURES = {
     "neo_b200_lowlat_set_impulse": (_i, [_vp, _vp, _sz, _i]),
     "neo_b200_lowlat_reset": (_i, [_vp]),
     "neo_b200_lowlat_process": (_i, [_vp, _vp, _vp, _sz, _i]),
+    "neo_b200_lowlat_process_samples": (_i, [_vp, _vp, _vp, _sz, _i]),
     "neo_b200_lowlat_set_stream": (_i, [_vp, _vp]),
     "neo_b200_lowlat_synchronize": (_i, [_vp]),
     "neo_b200_lowlat_device_bytes": (_sz, [_vp]),
@@ -763,7 +764,8 @@ class Convolver:
 class LowLatencyConvolver:
     """A bank of upols_convolver instances at ONE block of latency for long impulse responses (include/neo_b200.h:
     neo_b200_lowlat_*): the first partitions run per block, later stretches in frame mode on side streams (non-uniform
-    partitioning). `filter(H)` / `impulse(ir, block)` then call on any whole number of blocks.
+    partitioning). `filter(H)` / `impulse(ir, block)`, then call on any whole number of blocks, or `process_samples` on any
+    number of samples (each output returned by the call that delivers its input).
 
     frame_blocks: the level frame sizes T_1 < ... < T_n (powers of two in [2, 512], n <= 4); None = the library default.
     """
@@ -845,6 +847,19 @@ class LowLatencyConvolver:
         if out is None:
             out = x
         _check(library().neo_b200_lowlat_process(self._h, _ptr(x), _ptr(out), x.shape[1] // block, _space(x)))
+        return out
+
+    def process_samples(self, x, out=None):
+        """x [C][n], any n >= 1, returned in the same call: the handle keeps its position inside the current block, so a host
+        whose buffer size changes from call to call needs no FIFO in front (neo_b200_lowlat_process_samples). In place when out
+        is None."""
+        if self.cfg is None:
+            raise RuntimeError("no filter set")
+        if x.ndim != 2 or x.shape[0] != self.cfg.channels or x.shape[1] < 1 or _dtype_name(x) != self.real:
+            raise ValueError(f"expected {self.real}[{self.cfg.channels}][n], n >= 1")
+        if out is None:
+            out = x
+        _check(library().neo_b200_lowlat_process_samples(self._h, _ptr(x), _ptr(out), x.shape[1], _space(x)))
         return out
 
     def close(self) -> None:

@@ -1751,10 +1751,13 @@ struct lowlat_state
     device_buffer in_ring;                     // [C][2 T_n][B] the last 2 T_n input blocks: every level's frame is contiguous
     device_buffer plane[k_lowlat_max_levels];  // [C][2 T_i][B] level i's partial output of block t at slot t mod 2 T_i
     device_buffer head_y, stage_in, stage_out; // unfused head output; HOST staging
+    device_buffer pending;                     // [C][B] the current block's samples delivered so far (sample-granular calls)
+    device_buffer window, window_y;            // unfused head: [C][2B] a segment's window and its inverse transform
 
     size_t device_bytes(size_t levels) const
     {
-        size_t n = head.device_bytes() + in_ring.bytes + head_y.bytes + stage_in.bytes + stage_out.bytes;
+        size_t n = head.device_bytes() + in_ring.bytes + head_y.bytes + stage_in.bytes + stage_out.bytes + pending.bytes + window.bytes
+                 + window_y.bytes;
         for (size_t i = 0; i < levels; ++i) { n += level[i].device_bytes() + plane[i].bytes; }
         return n;
     }
@@ -1779,6 +1782,7 @@ struct neo_b200_lowlat
     bool fused{false};      // lowlat_head_kernel; else the head engine + lowlat_combine_kernel (NEO_B200_LOWLAT_UNFUSED)
     bool has_filter{false};
     size_t block_pos{0};    // blocks since the last reset
+    size_t sample_pos{0};   // samples of block block_pos delivered so far (in the pending buffer); 0 after whole-block calls
     lowlat_state<float> f32;
     lowlat_state<double> f64;
 
@@ -1831,7 +1835,12 @@ int lowlat_init(neo_b200_lowlat* h)
         NEO_TRY(s.plane[i].reserve(C * 2 * h->t[i] * B * sizeof(T)));
     }
     NEO_TRY(s.in_ring.reserve(C * h->ring_blocks * B * sizeof(T)));
-    if (!h->fused) { NEO_TRY(s.head_y.reserve(C * B * sizeof(T))); }
+    NEO_TRY(s.pending.reserve(C * B * sizeof(T)));
+    if (!h->fused) {
+        NEO_TRY(s.head_y.reserve(C * B * sizeof(T)));
+        NEO_TRY(s.window.reserve(C * 2 * B * sizeof(T)));
+        NEO_TRY(s.window_y.reserve(C * 2 * B * sizeof(T)));
+    }
     return NEO_B200_OK;
 }
 
@@ -1847,7 +1856,8 @@ int lowlat_clear(neo_b200_lowlat* h)
         NEO_CUDA_TRY(cudaMemsetAsync(s.plane[i].ptr, 0, s.plane[i].bytes, st));
     }
     NEO_CUDA_TRY(cudaMemsetAsync(s.in_ring.ptr, 0, s.in_ring.bytes, st));
-    h->block_pos = 0;
+    h->block_pos  = 0;
+    h->sample_pos = 0;  // the pending samples are discarded
     NEO_CUDA_TRY(cudaStreamSynchronize(st));
     return NEO_B200_OK;
 }
@@ -1862,20 +1872,29 @@ int lowlat_launch_head(lowlat_head_args<T> const& a, conv_engine<T> const& head,
     return check_launch("lowlat_head_kernel");
 }
 
-// one block for every channel: `in` / `out` point at the block of channel 0
+// rows of `p`, `stride` reals apart, all start on a complex pair (the fused head's 8- / 16-byte accesses, the r2c kernels' loads)
 template<typename T>
-int lowlat_block(neo_b200_lowlat* h, T const* in, size_t in_stride, T* out, size_t out_stride)
+bool lowlat_pairs(T const* p, size_t stride)
+{
+    return reinterpret_cast<std::uintptr_t>(p) % (2 * sizeof(T)) == 0 && stride % 2 == 0;
+}
+
+// positions [pos, end) of block block_pos for every channel: `in` / `out` point at position pos of channel 0. pos == 0, end == B is a
+// whole block; end == B completes the block (advances the head and releases level frames); end < B leaves the handle mid-block.
+template<typename T>
+int lowlat_segment(neo_b200_lowlat* h, T const* in, size_t in_stride, T* out, size_t out_stride, size_t pos, size_t end)
 {
     lowlat_state<T>& s   = lowlat_of<T>(h);
     cudaStream_t const st = h->stream.stream;
     size_t const C = h->cfg.channels, B = h->cfg.block, tb = h->block_pos;
+    bool const completes = end == B;
 
-    // the partial output of level i for block tb comes from its frame tb / T_i - 2
+    // the partial output of level i for block tb comes from its frame tb / T_i - 2; the first segment of the block waits for it
     lowlat_levels<T> lv{};
     lv.count = int(h->levels);
     for (size_t i = 0; i < h->levels; ++i) {
         size_t const ti = h->t[i];
-        if (!h->sync && tb % ti == 0 && tb >= 2 * ti) { NEO_CUDA_TRY(cudaStreamWaitEvent(st, h->done[i][(tb / ti - 2) & 1], 0)); }
+        if (!h->sync && pos == 0 && tb % ti == 0 && tb >= 2 * ti) { NEO_CUDA_TRY(cudaStreamWaitEvent(st, h->done[i][(tb / ti - 2) & 1], 0)); }
         lv.plane[i]  = s.plane[i].template as<T>() + (tb % (2 * ti)) * B;
         lv.stride[i] = 2 * ti * B;
     }
@@ -1884,24 +1903,54 @@ int lowlat_block(neo_b200_lowlat* h, T const* in, size_t in_stride, T* out, size
 
     if (h->fused) {
         conv_engine<T>& e = s.head;
+        bool const vec    = pos == 0 && completes && lowlat_pairs(in, in_stride) && lowlat_pairs<T>(out, out_stride);
         lowlat_head_args<T> a{in, in_stride, out, out_stride, e.prev[e.prev_flip].template as<T>(), e.prev[e.prev_flip ^ 1].template as<T>(),
                               ring_slot, ring_stride, e.fdl.template as<cx<T>>(), e.filter.template as<cx<T>>(), e.ring, int(e.write_pos),
-                              e.parts, e.logw, C, lv};
+                              e.parts, e.logw, C, lv, s.pending.template as<T>(), int(pos), int(end), vec ? 1 : 0};
         int status = NEO_B200_ERR_UNSUPPORTED;
         NEO_DISPATCH_LOGM(T, e.logb, {
             if constexpr (LOGM >= 6 && LOGM <= (sizeof(T) == 4 ? 12 : 11)) { status = lowlat_launch_head<T, LOGM>(a, e, st); }
         });
         if (status != NEO_B200_OK) { return status == NEO_B200_ERR_UNSUPPORTED ? fail(status, "fused head: block %zu not covered", B) : status; }
-        e.advance(1);
-    } else {
+        if (completes) { e.advance(1); }
+    } else if (completes) {
+        // a whole pair-aligned block straight from `in`; otherwise pending + `in` assembled into the window's right half first
         conv_engine<T>& e = s.head;
-        NEO_TRY(e.forward(in, in_stride, 1, st));
+        T const* blk      = in;
+        size_t blk_stride = in_stride;
+        if (!(pos == 0 && lowlat_pairs(in, in_stride))) {
+            dim3 const wgrid(unsigned((2 * B + 255) / 256), unsigned(C));
+            lowlat_window_kernel<T><<<wgrid, 256, 0, st>>>(e.prev[e.prev_flip].template as<T>(), s.pending.template as<T>(), in, in_stride, int(B),
+                                                           int(pos), int(end), s.window.template as<T>());
+            NEO_TRY(check_launch("lowlat_window_kernel"));
+            blk        = s.window.template as<T>() + B;
+            blk_stride = 2 * B;
+        }
+        NEO_TRY(e.forward(blk, blk_stride, 1, st));
         NEO_TRY(e.inverse(static_cast<cx<T> const*>(e.acc_r()), 0, 1, s.head_y.template as<T>(), B, 0, C, 1, st));
         dim3 const grid(unsigned((B + 255) / 256), unsigned(C));
-        lowlat_combine_kernel<T><<<grid, 256, 0, st>>>(s.head_y.template as<T>(), int(B), in, in_stride, out, out_stride, ring_slot, ring_stride, lv);
+        lowlat_combine_kernel<T><<<grid, 256, 0, st>>>(s.head_y.template as<T>(), B, int(pos), int(B), blk, blk_stride, out, out_stride, ring_slot,
+                                                       ring_stride, lv);
+        NEO_TRY(check_launch("lowlat_combine_kernel"));
+    } else {
+        // partial: the head engine's window step replaces the newest delay-line row without advancing
+        conv_engine<T>& e = s.head;
+        dim3 const wgrid(unsigned((2 * B + 255) / 256), unsigned(C));
+        lowlat_window_kernel<T><<<wgrid, 256, 0, st>>>(e.prev[e.prev_flip].template as<T>(), s.pending.template as<T>(), in, in_stride, int(B),
+                                                       int(pos), int(end), s.window.template as<T>());
+        NEO_TRY(check_launch("lowlat_window_kernel"));
+        NEO_TRY(e.window_step(s.window.template as<T>(), s.window_y.template as<T>(), false, st));
+        dim3 const grid(unsigned((end + 255) / 256), unsigned(C));
+        lowlat_combine_kernel<T><<<grid, 256, 0, st>>>(s.window_y.template as<T>() + B, 2 * B, int(pos), int(end), nullptr, 0, out, out_stride,
+                                                       nullptr, 0, lv);
         NEO_TRY(check_launch("lowlat_combine_kernel"));
     }
-    h->block_pos = tb + 1;
+    if (!completes) {
+        h->sample_pos = end;
+        return NEO_B200_OK;
+    }
+    h->block_pos  = tb + 1;
+    h->sample_pos = 0;
 
     // Levels whose frame this block completes. Frame f of level i (blocks f T_i .. f T_i + T_i - 1) runs on side stream i behind
     // `ready` and yields the partial output of blocks (f + 2) T_i .. (f + 3) T_i - 1 into plane slots (f % 2) T_i ..; the head waits for
@@ -1910,6 +1959,9 @@ int lowlat_block(neo_b200_lowlat* h, T const* in, size_t in_stride, T* out, size
     //   - plane slot (f % 2): its previous readers are the head blocks f T_i .. f T_i + T_i - 1 (frame f - 2's output), all enqueued on
     //     the head's stream before `ready`;
     //   - done[i][f % 2] is re-recorded for frame f + 2 only after the head's wait for frame f has been enqueued.
+    // Sample-granular calls keep this: every segment of block b reads plane slot b mod 2 T_i, which only a frame released after block b
+    // completes rewrites, so after every segment of block b in stream order; the wait for block b is enqueued before its first segment
+    // (pos == 0); partial segments write neither the input ring nor the half-window, and the pending buffer is the head stream's alone.
     // Every kernel sums in a fixed order and none uses atomics, so the bits do not depend on how the streams interleave
     // (NEO_B200_LOWLAT_SYNC runs the same kernels on the head's stream).
     for (size_t i = 0; i < h->levels; ++i) {
@@ -1929,12 +1981,13 @@ int lowlat_block(neo_b200_lowlat* h, T const* in, size_t in_stride, T* out, size
     return NEO_B200_OK;
 }
 
+// `samples` consecutive samples of every channel: [channels][samples] rows, cut into segments at block boundaries
 template<typename T>
-int lowlat_process(neo_b200_lowlat* h, void const* in, void* out, size_t blocks, int memspace)
+int lowlat_process(neo_b200_lowlat* h, void const* in, void* out, size_t samples, int memspace)
 {
     lowlat_state<T>& s   = lowlat_of<T>(h);
     cudaStream_t const st = h->stream.stream;
-    size_t const B = h->cfg.block, stride = blocks * B, bytes = h->cfg.channels * stride * sizeof(T);
+    size_t const B = h->cfg.block, stride = samples, bytes = h->cfg.channels * stride * sizeof(T);
     T const* din = static_cast<T const*>(in);
     T* dout      = static_cast<T*>(out);
     if (memspace == NEO_B200_HOST) {
@@ -1944,7 +1997,11 @@ int lowlat_process(neo_b200_lowlat* h, void const* in, void* out, size_t blocks,
         din  = s.stage_in.template as<T>();
         dout = s.stage_out.template as<T>();
     }
-    for (size_t b = 0; b < blocks; ++b) { NEO_TRY(lowlat_block<T>(h, din + b * B, stride, dout + b * B, stride)); }
+    for (size_t done = 0; done < samples;) {
+        size_t const pos = h->sample_pos, n = std::min(B - pos, samples - done);
+        NEO_TRY(lowlat_segment<T>(h, din + done, stride, dout + done, stride, pos, pos + n));
+        done += n;
+    }
     if (memspace == NEO_B200_HOST) {
         NEO_CUDA_TRY(cudaMemcpyAsync(out, dout, bytes, cudaMemcpyDeviceToHost, st));
         NEO_CUDA_TRY(cudaStreamSynchronize(st));
@@ -2050,8 +2107,20 @@ int neo_b200_lowlat_process(neo_b200_lowlat* handle, void const* in, void* out, 
     if (in == nullptr || out == nullptr) { return fail(NEO_B200_ERR_INVALID, "null buffer"); }
     if (blocks == 0) { return fail(NEO_B200_ERR_INVALID, "blocks must be >= 1"); }
     NEO_CUDA_TRY(cudaSetDevice(handle->device));
-    if (handle->cfg.dtype == NEO_B200_F32) { return lowlat_process<float>(handle, in, out, blocks, memspace); }
-    return lowlat_process<double>(handle, in, out, blocks, memspace);
+    size_t const samples = blocks * handle->cfg.block;
+    if (handle->cfg.dtype == NEO_B200_F32) { return lowlat_process<float>(handle, in, out, samples, memspace); }
+    return lowlat_process<double>(handle, in, out, samples, memspace);
+}
+
+int neo_b200_lowlat_process_samples(neo_b200_lowlat* handle, void const* in, void* out, size_t samples, int memspace)
+{
+    if (handle == nullptr) { return fail(NEO_B200_ERR_INVALID, "null argument"); }
+    if (!handle->has_filter) { return fail(NEO_B200_ERR_INVALID, "no filter set"); }
+    if (in == nullptr || out == nullptr) { return fail(NEO_B200_ERR_INVALID, "null buffer"); }
+    if (samples == 0) { return fail(NEO_B200_ERR_INVALID, "samples must be >= 1"); }
+    NEO_CUDA_TRY(cudaSetDevice(handle->device));
+    if (handle->cfg.dtype == NEO_B200_F32) { return lowlat_process<float>(handle, in, out, samples, memspace); }
+    return lowlat_process<double>(handle, in, out, samples, memspace);
 }
 
 int neo_b200_lowlat_set_stream(neo_b200_lowlat* handle, void* cuda_stream)

@@ -7,6 +7,15 @@
 //   Hermitian pre-pass -> c2r -> 1/2B, keep the last B samples -> + each level's partial output (level order) -> store,
 // and saves the block as the next left half-window and into the levels' input ring.
 //
+// Calls of any sample count (neo_b200_lowlat_process_samples) cut the stream into segments [pos, end) of a block. Overlap-save is
+// causal: output j of a block depends on input <= j only, so the window [previous block | samples [0, end), zeros] gives the exact
+// outputs [0, end), and the levels' planes already hold their part of the whole block. A segment that ends inside the block (end < B)
+// runs the same kernel with the new half assembled from the pending buffer ([0, pos), earlier calls), `in` ([pos, end), also kept in
+// the pending buffer) and zeros, stores outputs [pos, end) only, and leaves the half-window, the delay line and the input ring alone:
+// nothing reads delay-line slot wp (partition 0 comes from registers) before the segment that completes the block writes it. The
+// completing segment (end == B) is the whole-block computation on the whole block. Only a whole, pair-aligned block uses 8- / 16-byte
+// accesses on `in` / `out`; every other segment reads and writes them one real at a time, as its rows may start at any sample.
+//
 // Layouts (shared with conv_engine, whose head-range handle owns filter, delay line and half-window buffers):
 //   fdl    [C][B/W][R][W]    ring of head spectra, R = 2*T_1 rows, bin 0 packed as (Re X[0], Re X[B])
 //   filter [C][B/W][Ph][W]   head partitions, same packing
@@ -42,7 +51,17 @@ struct lowlat_head_args
     int ring, wp, parts, logw;
     size_t channels;
     lowlat_levels<T> levels;
+    T* pending;    // [C][B] samples [0, pos) of the current block, delivered by earlier calls
+    int pos, end;  // this segment covers block positions [pos, end); `in` / `out` point at position pos
+    int vec;       // pos == 0, end == B and every row of `in` / `out` starts on a complex pair: 8- / 16-byte accesses
 };
+
+// sample j of the new half-window of a segment: pending, then `in`, then zeros
+template<typename T>
+__device__ __forceinline__ T lowlat_sample(lowlat_head_args<T> const& a, T const* pend, T const* src, int j)
+{
+    return j < a.pos ? pend[j] : j < a.end ? src[j - a.pos] : T(0);
+}
 
 // register budget: the MAC keeps E accumulators next to the transform's E points. 128 registers leave no spills (-Xptxas -v) except
 // for double at 2^10 and 2^11 points (100 bytes spilled at 128, 4 at 168), which get the whole 255
@@ -97,19 +116,35 @@ __global__ void __launch_bounds__(fft_cfg<T, LOGM>::THREADS, lowlat_min_ctas<T, 
     size_t const row = live ? ch : 0;
 
     // 1. window [previous block | this block]: points e < E/2 are the left half, the rest this block (H = M/2 = HALF * TN pairs)
-    C const* lo = reinterpret_cast<C const*>(a.prev + row * M);
-    C const* hi = reinterpret_cast<C const*>(a.in + row * a.in_stride);
+    bool const whole = a.end == M;
+    C const* lo      = reinterpret_cast<C const*>(a.prev + row * M);
+    T const* src     = a.in + row * a.in_stride;
+    T* const pend    = a.pending + row * M;
     C v[E];
 #pragma unroll
-    for (int e = 0; e < E; ++e) { v[e] = !live ? mk<T>(0, 0) : e < HALF ? lo[t + e * TN] : hi[t + (e - HALF) * TN]; }
-    // 9. this block is the next left half-window and the levels' input (both buffers are distinct from in / out)
-    if (live) {
+    for (int e = 0; e < E; ++e) {
+        int const j = t + (e - HALF) * TN;
+        if (!live) { v[e] = mk<T>(0, 0); }
+        else if (e < HALF) { v[e] = lo[t + e * TN]; }
+        else if (a.vec) { v[e] = reinterpret_cast<C const*>(src)[j]; }
+        else { v[e] = mk<T>(lowlat_sample(a, pend, src, 2 * j), lowlat_sample(a, pend, src, 2 * j + 1)); }
+    }
+    // 9. a completed block is the next left half-window and the levels' input (both buffers are distinct from in / out); a partial
+    // segment keeps its samples for the segments that follow
+    if (live && whole) {
         C* const keep = reinterpret_cast<C*>(a.prev_next + row * M);
         C* const ring = reinterpret_cast<C*>(a.in_ring + row * a.ring_stride);
 #pragma unroll
         for (int e = HALF; e < E; ++e) {
             keep[t + (e - HALF) * TN] = v[e];
             ring[t + (e - HALF) * TN] = v[e];
+        }
+    } else if (live) {
+#pragma unroll
+        for (int e = HALF; e < E; ++e) {
+            int const j = 2 * (t + (e - HALF) * TN);
+            if (j >= a.pos && j < a.end) { pend[j] = v[e].x; }
+            if (j + 1 >= a.pos && j + 1 < a.end) { pend[j + 1] = v[e].y; }
         }
     }
 
@@ -131,7 +166,7 @@ __global__ void __launch_bounds__(fft_cfg<T, LOGM>::THREADS, lowlat_min_ctas<T, 
     }
     __syncthreads();  // the tile is reused by the c2r pre-pass
 
-    // 3. delay-line insert into slot wp; 4. MAC over the head partitions, partition 0 from registers, fixed partition order
+    // 3. delay-line insert into slot wp (completed blocks only); 4. MAC over the head partitions, partition 0 from registers, fixed partition order
     C* const x_row       = a.fdl + tiled_offset(row, M >> a.logw, a.logw, size_t(a.ring), 0, 0);
     C const* const h_row = a.filter + tiled_offset(row, M >> a.logw, a.logw, size_t(a.parts), 0, 0);
     C ak[HALF], am[HALF];
@@ -139,7 +174,7 @@ __global__ void __launch_bounds__(fft_cfg<T, LOGM>::THREADS, lowlat_min_ctas<T, 
     for (int e = 0; e < HALF; ++e) {
         int const k  = t + e * TN;
         int const km = k == 0 ? M / 2 : M - k;
-        if (live) {
+        if (live && whole) {
             x_row[lowlat_tiled(a.ring, a.logw, k) + (size_t(a.wp) << a.logw)]  = xk[e];
             x_row[lowlat_tiled(a.ring, a.logw, km) + (size_t(a.wp) << a.logw)] = xm[e];
         }
@@ -194,10 +229,11 @@ __global__ void __launch_bounds__(fft_cfg<T, LOGM>::THREADS, lowlat_min_ctas<T, 
     __syncthreads();
     cta_fft<T, LOGM, +1>::run(v, sm, tw, t);
 
-    // 6.-8. scale, keep samples [B, 2B), add the levels in level order, store
+    // 6.-8. scale, keep samples [B, 2B), add the levels in level order, store positions [pos, end)
     if (live) {
         T const scale = T(1) / T(2 * M);
-        C* const dst  = reinterpret_cast<C*>(a.out + row * a.out_stride);
+        T* const o    = a.out + row * a.out_stride;
+        C* const dst  = reinterpret_cast<C*>(o);
 #pragma unroll
         for (int e = HALF; e < E; ++e) {
             int const j = t + (e - HALF) * TN;
@@ -210,27 +246,52 @@ __global__ void __launch_bounds__(fft_cfg<T, LOGM>::THREADS, lowlat_min_ctas<T, 
                     y.y += l.y;
                 }
             }
-            dst[j] = y;
+            if (a.vec) { dst[j] = y; }
+            else {
+                if (2 * j >= a.pos && 2 * j < a.end) { o[2 * j - a.pos] = y.x; }
+                if (2 * j + 1 >= a.pos && 2 * j + 1 < a.end) { o[2 * j + 1 - a.pos] = y.y; }
+            }
         }
     }
 }
 
-// the unfused form's tail: out = head + levels (level order), and the block into the levels' input ring. grid (ceil(B/256), C)
+// the unfused form's tail over block positions [0, end): with an input ring, the block (`in` from position 0) into it; for positions
+// [first, end), out = head + levels (level order), `out` pointing at position `first`. grid (ceil(end/256), C)
 template<typename T>
-__global__ void __launch_bounds__(256) lowlat_combine_kernel(T const* __restrict__ head, int block, T const* in, size_t in_stride, T* out,
-                                                             size_t out_stride, T* __restrict__ in_ring, size_t ring_stride,
-                                                             lowlat_levels<T> levels)
+__global__ void __launch_bounds__(256) lowlat_combine_kernel(T const* __restrict__ head, size_t head_stride, int first, int end, T const* in,
+                                                             size_t in_stride, T* out, size_t out_stride, T* __restrict__ in_ring,
+                                                             size_t ring_stride, lowlat_levels<T> levels)
 {
     size_t const ch = blockIdx.y;
     int const i     = blockIdx.x * blockDim.x + threadIdx.x;
-    if (i >= block) { return; }
-    in_ring[ch * ring_stride + i] = in[ch * in_stride + i];  // read before the store below: in == out is allowed
-    T y = head[ch * size_t(block) + i];
+    if (i >= end) { return; }
+    if (in_ring != nullptr) { in_ring[ch * ring_stride + i] = in[ch * in_stride + i]; }  // read before the store below: in == out is allowed
+    if (i < first) { return; }
+    T y = head[ch * head_stride + i];
 #pragma unroll
     for (int l = 0; l < k_lowlat_max_levels; ++l) {
         if (l < levels.count) { y += levels.plane[l][ch * levels.stride[l] + i]; }
     }
-    out[ch * out_stride + i] = y;
+    out[ch * out_stride + (i - first)] = y;
+}
+
+// the unfused head's window of a segment, [C][2B] = [previous block | pending [0, pos), in [pos, end), zeros] (`in` pointing at position
+// pos); a partial segment (end < B) also keeps its samples in the pending buffer. grid (ceil(2B/256), C)
+template<typename T>
+__global__ void __launch_bounds__(256) lowlat_window_kernel(T const* __restrict__ prev, T* __restrict__ pending, T const* in, size_t in_stride,
+                                                            int block, int pos, int end, T* __restrict__ window)
+{
+    size_t const ch = blockIdx.y;
+    int const i     = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= 2 * block) { return; }
+    T v;
+    if (i < block) { v = prev[ch * block + i]; }
+    else {
+        int const j = i - block;
+        v           = j < pos ? pending[ch * block + j] : j < end ? in[ch * in_stride + (j - pos)] : T(0);
+        if (end < block && j >= pos && j < end) { pending[ch * block + j] = v; }
+    }
+    window[ch * 2 * block + i] = v;
 }
 
 }  // namespace neo_b200
