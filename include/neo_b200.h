@@ -366,6 +366,25 @@ NEO_B200_API int neo_b200_lowlat_process(neo_b200_lowlat* handle, void const* in
  * samples and all state at every block boundary are those of whole-block calls however the block was split; outputs of a segment that
  * ends inside a block match to rounding only. */
 NEO_B200_API int neo_b200_lowlat_process_samples(neo_b200_lowlat* handle, void const* in, void* out, size_t samples, int memspace);
+/* switch to a new filter mid-stream with a sample-accurate linear crossfade, keeping every delay line (DESIGN §4.7).
+ * stage_filter / stage_impulse build a second filter set B next to the current set A, on the handle's own lowest-priority stream after any
+ * enqueued work that may still read the spare set, and return when B is ready. They change no output and touch no delay line, block
+ * position or pending sample. H has the set_filter layout; ir is [channels][taps] with block <= taps and num_partitions(taps, block) <=
+ * P, shorter responses zero-padded to P partitions. Staging again before a crossfade replaces B. NEO_B200_ERR_INVALID before any filter
+ * is set, while a crossfade is pending or running, or on a taps mismatch. Device bytes grow by the spare set at the first stage. */
+NEO_B200_API int neo_b200_lowlat_stage_filter(neo_b200_lowlat* handle, void const* H, int memspace);
+NEO_B200_API int neo_b200_lowlat_stage_impulse(neo_b200_lowlat* handle, void const* ir, size_t taps, int memspace);
+/* starts the switch to the staged set and returns in *start (may be NULL) the absolute index, in samples delivered since the last
+ * reset / set_filter / set_impulse, of the first sample of the fade. Every channel's output at sample t is y_A(t) for t < start,
+ * y_A(t) + g (y_B(t) - y_A(t)) with g = (t - start) / fade (computed in double, rounded to the handle's type) for start <= t < start +
+ * fade, and y_B(t) itself from start + fade on (fade = 0: a hard switch at start); y_B is the output of B over the whole stream. Once every
+ * sample before start + fade has been delivered, B is the current filter and A the spare. start is the next sample with no levels;
+ * otherwise start = b0 * block with b0 = max_i (floor(b / T_i) + 2) T_i, b the block holding the next sample: level work under B starts
+ * with the first frame released after this call, so the switch comes 1 to 2 frames of the largest level later. Bits: samples before
+ * start are those of the handle without the crossfade, samples from start + fade on those of a handle given B at its last reset and fed
+ * the same calls. NEO_B200_ERR_INVALID with nothing staged or a crossfade already pending or running. reset, set_filter and set_impulse
+ * cancel a pending or running crossfade and drop the staged set (reset keeps the current filter, A until the fade has ended). */
+NEO_B200_API int neo_b200_lowlat_crossfade(neo_b200_lowlat* handle, size_t fade, size_t* start);
 NEO_B200_API int neo_b200_lowlat_set_stream(neo_b200_lowlat* handle, void* cuda_stream);
 /* waits for the handle's stream and its side streams */
 NEO_B200_API int neo_b200_lowlat_synchronize(neo_b200_lowlat* handle);

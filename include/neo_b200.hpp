@@ -732,6 +732,8 @@ using upola_convolver = uniform_partitioned_convolver<Complex, NEO_B200_UPOLA>;
 /// partitioning). Same results up to rounding. One instance = one channel; `frame_blocks` = the level frame sizes, empty = the
 /// library default. `process(samples)` takes any number of samples >= 1 in place and returns each output in the call that delivers
 /// its input (neo_b200_lowlat_process_samples): what a plugin host's varying buffer size needs, with no FIFO in front.
+/// `crossfade_to(H, fade)` swaps in a new impulse response mid-stream with a linear crossfade of `fade` samples and keeps the reverb
+/// tail of everything played so far (neo_b200_lowlat_stage_filter + neo_b200_lowlat_crossfade).
 template<typename Complex>
 struct low_latency_convolver
 {
@@ -747,16 +749,9 @@ struct low_latency_convolver
     template<typename Mat>
     auto filter(Mat h) -> void
     {
-        static_assert(std::is_same_v<detail::element_of<Mat>, Complex>);
         auto const parts = static_cast<std::size_t>(h.extent(0));
         auto const bins  = static_cast<std::size_t>(h.extent(1));
-        _copy.resize(parts * bins);
-        for (std::size_t p = 0; p < parts; ++p) {
-            for (std::size_t k = 0; k < bins; ++k) {
-                auto const v        = h(p, k);
-                _copy[p * bins + k] = std::complex<real_type>{v.real(), v.imag()};
-            }
-        }
+        copy_filter(h);
         neo_b200_lowlat_config cfg{detail::dtype_of<real_type>, 1, bins - 1, parts, _frame_blocks.size(), {0, 0, 0, 0}};
         for (std::size_t i = 0; i < _frame_blocks.size() && i < 4; ++i) { cfg.frame_blocks[i] = _frame_blocks[i]; }
         neo_b200_lowlat_destroy(_conv);
@@ -764,6 +759,24 @@ struct low_latency_convolver
         detail::check(neo_b200_lowlat_create(&_conv, &cfg));
         detail::check(neo_b200_lowlat_set_filter(_conv, _copy.data(), NEO_B200_HOST));
         _block = bins - 1;
+        _parts = parts;
+    }
+
+    /// switches to `h` (the H[P][B+1] view filter() takes, same P and B) with a linear crossfade of `fade` samples, keeping every delay
+    /// line; returns the index of the fade's first sample, counted from the last filter() call. Throws while an earlier crossfade has
+    /// not ended (DESIGN §4.7: the fade starts one to two of the largest level's frames after the call).
+    template<typename Mat>
+    auto crossfade_to(Mat h, std::size_t fade) -> std::size_t
+    {
+        if (_conv == nullptr) { throw std::invalid_argument{"neo::b200::low_latency_convolver: filter() has not been called"}; }
+        if (static_cast<std::size_t>(h.extent(0)) != _parts || static_cast<std::size_t>(h.extent(1)) != _block + 1) {
+            throw std::invalid_argument{"neo::b200::low_latency_convolver: crossfade_to() needs the shape filter() was given"};
+        }
+        copy_filter(h);
+        detail::check(neo_b200_lowlat_stage_filter(_conv, _copy.data(), NEO_B200_HOST));
+        std::size_t start = 0;
+        detail::check(neo_b200_lowlat_crossfade(_conv, fade, &start));
+        return start;
     }
 
     template<typename Vec>
@@ -803,9 +816,24 @@ struct low_latency_convolver
     [[nodiscard]] auto device_bytes() const noexcept -> std::size_t { return _conv == nullptr ? 0 : neo_b200_lowlat_device_bytes(_conv); }
 
 private:
+    template<typename Mat>
+    auto copy_filter(Mat h) -> void
+    {
+        static_assert(std::is_same_v<detail::element_of<Mat>, Complex>);
+        auto const parts = static_cast<std::size_t>(h.extent(0));
+        auto const bins  = static_cast<std::size_t>(h.extent(1));
+        _copy.resize(parts * bins);
+        for (std::size_t p = 0; p < parts; ++p) {
+            for (std::size_t k = 0; k < bins; ++k) {
+                auto const v        = h(p, k);
+                _copy[p * bins + k] = std::complex<real_type>{v.real(), v.imag()};
+            }
+        }
+    }
+
     neo_b200_lowlat* _conv{nullptr};
     std::vector<std::size_t> _frame_blocks;
-    std::size_t _block{0};
+    std::size_t _block{0}, _parts{0};
     std::vector<std::complex<real_type>> _copy;
     std::vector<real_type> _tmp;
 };

@@ -165,6 +165,9 @@ SIGNATURES = {
     "neo_b200_lowlat_reset": (_i, [_vp]),
     "neo_b200_lowlat_process": (_i, [_vp, _vp, _vp, _sz, _i]),
     "neo_b200_lowlat_process_samples": (_i, [_vp, _vp, _vp, _sz, _i]),
+    "neo_b200_lowlat_stage_filter": (_i, [_vp, _vp, _i]),
+    "neo_b200_lowlat_stage_impulse": (_i, [_vp, _vp, _sz, _i]),
+    "neo_b200_lowlat_crossfade": (_i, [_vp, _sz, C.POINTER(_sz)]),
     "neo_b200_lowlat_set_stream": (_i, [_vp, _vp]),
     "neo_b200_lowlat_synchronize": (_i, [_vp]),
     "neo_b200_lowlat_device_bytes": (_sz, [_vp]),
@@ -765,7 +768,8 @@ class LowLatencyConvolver:
     """A bank of upols_convolver instances at ONE block of latency for long impulse responses (include/neo_b200.h:
     neo_b200_lowlat_*): the first partitions run per block, later stretches in frame mode on side streams (non-uniform
     partitioning). `filter(H)` / `impulse(ir, block)`, then call on any whole number of blocks, or `process_samples` on any
-    number of samples (each output returned by the call that delivers its input).
+    number of samples (each output returned by the call that delivers its input). `stage_filter(H)` / `stage_impulse(ir)` then
+    `crossfade(fade)` switch to a new response mid-stream with a linear crossfade, keeping every delay line.
 
     frame_blocks: the level frame sizes T_1 < ... < T_n (powers of two in [2, 512], n <= 4); None = the library default.
     """
@@ -822,6 +826,41 @@ class LowLatencyConvolver:
         taps = int(ir.shape[1])
         self._create(int(ir.shape[0]), block, num_partitions(taps, block))
         _check(library().neo_b200_lowlat_set_impulse(self._h, _ptr(ir), taps, _space(ir)))
+
+    def stage_filter(self, H) -> None:
+        """H [C][P][B+1] of this handle's shape, prepared next to the current filter for `crossfade`: no output, delay line or
+        position changes (neo_b200_lowlat_stage_filter)."""
+        if self.cfg is None:
+            raise RuntimeError("no filter set")
+        shape = (int(self.cfg.channels), int(self.cfg.partitions), int(self.cfg.block) + 1)
+        if H.ndim != 3 or tuple(int(n) for n in H.shape) != shape:
+            raise ValueError(f"filter must be [{shape[0]}][{shape[1]}][{shape[2]}]")
+        if _dtype_name(H) != ("complex64" if self.real == "float32" else "complex128"):
+            raise ValueError("filter dtype does not match the convolver")
+        _check(library().neo_b200_lowlat_stage_filter(self._h, _ptr(H), _space(H)))
+
+    def stage_impulse(self, ir) -> None:
+        """stage_filter(uniform_partition(ir, B)) for ir [C][taps], B <= taps, num_partitions(taps, B) <= P; a shorter response
+        is zero-padded to the handle's P partitions."""
+        if self.cfg is None:
+            raise RuntimeError("no filter set")
+        if ir.ndim != 2 or ir.shape[0] != self.cfg.channels or _dtype_name(ir) != self.real:
+            raise ValueError("impulse response shape/dtype mismatch")
+        taps, block = int(ir.shape[1]), int(self.cfg.block)
+        if taps < block or num_partitions(taps, block) > self.cfg.partitions:
+            raise ValueError(f"impulse response of {taps} taps does not fit {self.cfg.partitions} partitions of {block}")
+        _check(library().neo_b200_lowlat_stage_impulse(self._h, _ptr(ir), taps, _space(ir)))
+
+    def crossfade(self, fade: int) -> int:
+        """Switch to the staged filter with a linear fade of `fade` samples (0: hard switch). Returns `start`, the absolute index
+        (samples since the last reset / filter / impulse) of the fade's first sample (neo_b200_lowlat_crossfade)."""
+        if self.cfg is None:
+            raise RuntimeError("no filter set")
+        if int(fade) < 0:
+            raise ValueError("fade must be >= 0")
+        start = _sz(0)
+        _check(library().neo_b200_lowlat_crossfade(self._h, int(fade), C.byref(start)))
+        return int(start.value)
 
     def set_stream(self, stream) -> None:
         self._stream = _stream_ptr(stream)

@@ -13,6 +13,7 @@
 #include <cstring>
 #include <new>
 #include <string>
+#include <utility>
 
 namespace neo_b200 {
 
@@ -96,6 +97,12 @@ struct device_buffer
     U* as() const
     {
         return static_cast<U*>(ptr);
+    }
+
+    void swap(device_buffer& o) noexcept
+    {
+        std::swap(ptr, o.ptr);
+        std::swap(bytes, o.bytes);
     }
 };
 

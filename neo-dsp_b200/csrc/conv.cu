@@ -306,7 +306,7 @@ struct conv_engine
         return NEO_B200_OK;
     }
 
-    // frame mode: the level-1 filter exists only between begin_filter and finish_filter
+    // frame mode: the level-1 filter exists only between begin_filter and build_filter
     int begin_filter()
     {
         if (frame > 0 || filter.ptr == nullptr) { NEO_TRY(filter.reserve(filters * parts * m * sizeof(cx<T>))); }
@@ -386,6 +386,14 @@ struct conv_engine
 
     int finish_filter(cudaStream_t stream)
     {
+        NEO_TRY(build_filter(stream));
+        return clear_state(stream);
+    }
+
+    // the filter's last step (frame mode: the level-1 filter transformed along block time into filter2); the delay line is not touched,
+    // so a filter can be built into a spare buffer while the stream keeps running (neo_b200_lowlat_stage_filter)
+    int build_filter(cudaStream_t stream)
+    {
         if (frame > 0) {
             frame_geom const fg{logb, logw, nt, frame, tiles2};
             int status = NEO_B200_ERR_UNSUPPORTED;
@@ -403,7 +411,7 @@ struct conv_engine
             filter.release();
         }
         has_filter = true;
-        return clear_state(stream);
+        return NEO_B200_OK;
     }
 
     // H in the reference layout [filters][P][B+1]; device pointer
@@ -420,6 +428,13 @@ struct conv_engine
     }
 
     int set_filter(void const* h, int memspace, cudaStream_t stream)
+    {
+        NEO_TRY(load_filter(h, memspace, stream));
+        return clear_state(stream);
+    }
+
+    // set_filter without zeroing the state
+    int load_filter(void const* h, int memspace, cudaStream_t stream)
     {
         size_t const p_total = cfg.partitions;
         size_t const k       = size_t(m) + 1;
@@ -441,7 +456,7 @@ struct conv_engine
                 NEO_CUDA_TRY(cudaStreamSynchronize(stream));  // staging buffer is reused
             }
         }
-        return finish_filter(stream);
+        return build_filter(stream);
     }
 
     int partition_into(T const* ir_dev, size_t taps, size_t first_filter, size_t count, cudaStream_t stream)
@@ -459,6 +474,13 @@ struct conv_engine
 
     int set_impulse(void const* ir, size_t taps, int memspace, cudaStream_t stream)
     {
+        NEO_TRY(load_impulse(ir, taps, memspace, stream));
+        return clear_state(stream);
+    }
+
+    // set_impulse without zeroing the state; partitions past `taps` are zero
+    int load_impulse(void const* ir, size_t taps, int memspace, cudaStream_t stream)
+    {
         NEO_TRY(begin_filter());
         if (memspace == NEO_B200_DEVICE) {
             NEO_TRY(partition_into(static_cast<T const*>(ir), taps, 0, filters, stream));
@@ -474,7 +496,7 @@ struct conv_engine
                 NEO_CUDA_TRY(cudaStreamSynchronize(stream));
             }
         }
-        return finish_filter(stream);
+        return build_filter(stream);
     }
 
     // the wide kernels move the real rows with 128-bit accesses
@@ -1753,14 +1775,38 @@ struct lowlat_state
     device_buffer head_y, stage_in, stage_out; // unfused head output; HOST staging
     device_buffer pending;                     // [C][B] the current block's samples delivered so far (sample-granular calls)
     device_buffer window, window_y;            // unfused head: [C][2B] a segment's window and its inverse transform
+    // the spare filter set (neo_b200_lowlat_stage_*), allocated by the first stage: the head's filter, each level's filter2, each level's
+    // B-side planes [C][2 T_i][B], and the head's B-side outputs of a segment inside a crossfade ([C][B] fused, [C][2B] unfused)
+    device_buffer spare_head, spare_level[k_lowlat_max_levels], plane_b[k_lowlat_max_levels], fade_y;
 
     size_t device_bytes(size_t levels) const
     {
         size_t n = head.device_bytes() + in_ring.bytes + head_y.bytes + stage_in.bytes + stage_out.bytes + pending.bytes + window.bytes
-                 + window_y.bytes;
-        for (size_t i = 0; i < levels; ++i) { n += level[i].device_bytes() + plane[i].bytes; }
+                 + window_y.bytes + spare_head.bytes + fade_y.bytes;
+        for (size_t i = 0; i < levels; ++i) { n += level[i].device_bytes() + plane[i].bytes + spare_level[i].bytes + plane_b[i].bytes; }
         return n;
     }
+
+    // the staged set becomes the current one, and the current one the spare
+    void swap_sets(size_t levels)
+    {
+        head.filter.swap(spare_head);
+        for (size_t i = 0; i < levels; ++i) {
+            level[i].filter2.swap(spare_level[i]);
+            plane[i].swap(plane_b[i]);
+        }
+    }
+};
+
+// an engine runs with the spare filter for the lifetime of this guard
+struct lowlat_use_spare
+{
+    device_buffer& a;
+    device_buffer& b;
+    lowlat_use_spare(device_buffer& filter, device_buffer& spare) : a(filter), b(spare) { a.swap(b); }
+    ~lowlat_use_spare() { a.swap(b); }
+    lowlat_use_spare(lowlat_use_spare const&)            = delete;
+    lowlat_use_spare& operator=(lowlat_use_spare const&) = delete;
 };
 
 }  // namespace
@@ -1783,8 +1829,17 @@ struct neo_b200_lowlat
     bool has_filter{false};
     size_t block_pos{0};    // blocks since the last reset
     size_t sample_pos{0};   // samples of block block_pos delivered so far (in the pending buffer); 0 after whole-block calls
+    // crossfade (neo_b200_lowlat_stage_* / _crossfade): the spare set holds B; while `fading`, samples [fade_start, fade_end) blend A into
+    // B and B becomes the current set once every sample before fade_end has been delivered
+    bool staged{false};
+    bool fading{false};
+    size_t fade_start{0}, fade_end{0};
+    cudaStream_t stage_stream{nullptr};                // lowest priority: staging runs behind the stream's work
+    cudaEvent_t stage_after[k_lowlat_max_levels + 1]{};  // staging waits for the head's stream and each side stream
     lowlat_state<float> f32;
     lowlat_state<double> f64;
+
+    size_t position() const { return block_pos * cfg.block + sample_pos; }  // samples delivered since the last reset
 
     int sync_all()
     {
@@ -1804,6 +1859,13 @@ struct neo_b200_lowlat
             for (cudaEvent_t ev : {ready[i], done[i][0], done[i][1]}) {
                 if (ev != nullptr) { cudaEventDestroy(ev); }
             }
+        }
+        if (stage_stream != nullptr) {
+            cudaStreamSynchronize(stage_stream);
+            cudaStreamDestroy(stage_stream);
+        }
+        for (cudaEvent_t ev : stage_after) {
+            if (ev != nullptr) { cudaEventDestroy(ev); }
         }
     }
 };
@@ -1844,7 +1906,7 @@ int lowlat_init(neo_b200_lowlat* h)
     return NEO_B200_OK;
 }
 
-// zero every piece of stream state; the caller has synchronised the side streams
+// zero every piece of stream state and drop a staged set or a pending / running crossfade; the caller has synchronised the side streams
 template<typename T>
 int lowlat_clear(neo_b200_lowlat* h)
 {
@@ -1858,6 +1920,8 @@ int lowlat_clear(neo_b200_lowlat* h)
     NEO_CUDA_TRY(cudaMemsetAsync(s.in_ring.ptr, 0, s.in_ring.bytes, st));
     h->block_pos  = 0;
     h->sample_pos = 0;  // the pending samples are discarded
+    h->staged     = false;
+    h->fading     = false;
     NEO_CUDA_TRY(cudaStreamSynchronize(st));
     return NEO_B200_OK;
 }
@@ -1866,7 +1930,7 @@ template<typename T, int LOGM>
 int lowlat_launch_head(lowlat_head_args<T> const& a, conv_engine<T> const& head, cudaStream_t st)
 {
     using cfg   = fft_cfg<T, LOGM>;
-    auto kernel = lowlat_head_kernel<T, LOGM>;
+    auto kernel = a.commit == 0 || a.fade_y != nullptr ? lowlat_head_kernel<T, LOGM, true> : lowlat_head_kernel<T, LOGM, false>;
     NEO_TRY(enable_smem(kernel, cfg::SMEM));
     kernel<<<unsigned((a.channels + cfg::G - 1) / cfg::G), cfg::THREADS, cfg::SMEM, st>>>(a, head.tables.tw(), head.tables.rtw());
     return check_launch("lowlat_head_kernel");
@@ -1879,8 +1943,20 @@ bool lowlat_pairs(T const* p, size_t stride)
     return reinterpret_cast<std::uintptr_t>(p) % (2 * sizeof(T)) == 0 && stride % 2 == 0;
 }
 
+// the staged set becomes the current one once every sample before the end of the fade has been delivered
+template<typename T>
+void lowlat_finish_fade(neo_b200_lowlat* h)
+{
+    if (!h->fading || h->position() < h->fade_end) { return; }
+    lowlat_of<T>(h).swap_sets(h->levels);
+    h->fading = false;
+    h->staged = false;
+}
+
 // positions [pos, end) of block block_pos for every channel: `in` / `out` point at position pos of channel 0. pos == 0, end == B is a
 // whole block; end == B completes the block (advances the head and releases level frames); end < B leaves the handle mid-block.
+// A segment with samples on both sides of a crossfade's start ... end runs the head twice: the B side outputs only, then the A side,
+// which commits the state as always and blends the two per sample.
 template<typename T>
 int lowlat_segment(neo_b200_lowlat* h, T const* in, size_t in_stride, T* out, size_t out_stride, size_t pos, size_t end)
 {
@@ -1888,15 +1964,18 @@ int lowlat_segment(neo_b200_lowlat* h, T const* in, size_t in_stride, T* out, si
     cudaStream_t const st = h->stream.stream;
     size_t const C = h->cfg.channels, B = h->cfg.block, tb = h->block_pos;
     bool const completes = end == B;
+    bool const both      = h->fading && tb * B + pos < h->fade_end && tb * B + end > h->fade_start;
+    lowlat_fade const fade{tb * B, h->fade_start, h->fade_end - h->fade_start};
 
     // the partial output of level i for block tb comes from its frame tb / T_i - 2; the first segment of the block waits for it
-    lowlat_levels<T> lv{};
-    lv.count = int(h->levels);
+    lowlat_levels<T> lv{}, lvb{};
+    lv.count = lvb.count = int(h->levels);
     for (size_t i = 0; i < h->levels; ++i) {
         size_t const ti = h->t[i];
         if (!h->sync && pos == 0 && tb % ti == 0 && tb >= 2 * ti) { NEO_CUDA_TRY(cudaStreamWaitEvent(st, h->done[i][(tb / ti - 2) & 1], 0)); }
         lv.plane[i]  = s.plane[i].template as<T>() + (tb % (2 * ti)) * B;
-        lv.stride[i] = 2 * ti * B;
+        lv.stride[i] = lvb.stride[i] = 2 * ti * B;
+        if (both) { lvb.plane[i] = s.plane_b[i].template as<T>() + (tb % (2 * ti)) * B; }
     }
     T* const ring_slot       = s.in_ring.template as<T>() + (tb % h->ring_blocks) * B;
     size_t const ring_stride = h->ring_blocks * B;
@@ -1906,12 +1985,25 @@ int lowlat_segment(neo_b200_lowlat* h, T const* in, size_t in_stride, T* out, si
         bool const vec    = pos == 0 && completes && lowlat_pairs(in, in_stride) && lowlat_pairs<T>(out, out_stride);
         lowlat_head_args<T> a{in, in_stride, out, out_stride, e.prev[e.prev_flip].template as<T>(), e.prev[e.prev_flip ^ 1].template as<T>(),
                               ring_slot, ring_stride, e.fdl.template as<cx<T>>(), e.filter.template as<cx<T>>(), e.ring, int(e.write_pos),
-                              e.parts, e.logw, C, lv, s.pending.template as<T>(), int(pos), int(end), vec ? 1 : 0};
-        int status = NEO_B200_ERR_UNSUPPORTED;
-        NEO_DISPATCH_LOGM(T, e.logb, {
-            if constexpr (LOGM >= 6 && LOGM <= (sizeof(T) == 4 ? 12 : 11)) { status = lowlat_launch_head<T, LOGM>(a, e, st); }
-        });
-        if (status != NEO_B200_OK) { return status == NEO_B200_ERR_UNSUPPORTED ? fail(status, "fused head: block %zu not covered", B) : status; }
+                              e.parts, e.logw, C, lv, s.pending.template as<T>(), int(pos), int(end), vec ? 1 : 0, 1, nullptr, fade};
+        auto const launch = [&](lowlat_head_args<T> const& args) {
+            int status = NEO_B200_ERR_UNSUPPORTED;
+            NEO_DISPATCH_LOGM(T, e.logb, {
+                if constexpr (LOGM >= 6 && LOGM <= (sizeof(T) == 4 ? 12 : 11)) { status = lowlat_launch_head<T, LOGM>(args, e, st); }
+            });
+            return status == NEO_B200_ERR_UNSUPPORTED ? fail(status, "fused head: block %zu not covered", B) : status;
+        };
+        if (both) {  // B side: filter B and the B planes, outputs [pos, end) into fade_y by block position, nothing committed
+            lowlat_head_args<T> b = a;
+            b.out                 = s.fade_y.template as<T>() + pos;
+            b.out_stride          = B;
+            b.filter              = s.spare_head.template as<cx<T>>();
+            b.levels              = lvb;
+            b.commit              = 0;
+            NEO_TRY(launch(b));
+            a.fade_y = s.fade_y.template as<T>();
+        }
+        NEO_TRY(launch(a));
         if (completes) { e.advance(1); }
     } else if (completes) {
         // a whole pair-aligned block straight from `in`; otherwise pending + `in` assembled into the window's right half first
@@ -1926,27 +2018,44 @@ int lowlat_segment(neo_b200_lowlat* h, T const* in, size_t in_stride, T* out, si
             blk        = s.window.template as<T>() + B;
             blk_stride = 2 * B;
         }
-        NEO_TRY(e.forward(blk, blk_stride, 1, st));
+        if (both) {  // one insert, the B side's MAC and inverse transform into fade_y, then the A side's MAC as forward() runs it
+            NEO_TRY(e.forward_r2c(blk, blk_stride, 1, 0, C, st));
+            {
+                lowlat_use_spare const use_b(e.filter, s.spare_head);
+                NEO_TRY(e.forward_mac(1, 0, C, st));
+            }
+            NEO_TRY(e.inverse(e.acc_w(), 0, 1, s.fade_y.template as<T>(), B, 0, C, 1, st));
+            NEO_TRY(e.forward_mac(1, 0, C, st));
+            e.advance(1);
+        } else {
+            NEO_TRY(e.forward(blk, blk_stride, 1, st));
+        }
         NEO_TRY(e.inverse(static_cast<cx<T> const*>(e.acc_r()), 0, 1, s.head_y.template as<T>(), B, 0, C, 1, st));
         dim3 const grid(unsigned((B + 255) / 256), unsigned(C));
         lowlat_combine_kernel<T><<<grid, 256, 0, st>>>(s.head_y.template as<T>(), B, int(pos), int(B), blk, blk_stride, out, out_stride, ring_slot,
-                                                       ring_stride, lv);
+                                                       ring_stride, lv, both ? s.fade_y.template as<T>() : nullptr, lvb, fade);
         NEO_TRY(check_launch("lowlat_combine_kernel"));
     } else {
-        // partial: the head engine's window step replaces the newest delay-line row without advancing
+        // partial: the head engine's window step replaces the newest delay-line row without advancing (the B side's step stores the
+        // same row again)
         conv_engine<T>& e = s.head;
         dim3 const wgrid(unsigned((2 * B + 255) / 256), unsigned(C));
         lowlat_window_kernel<T><<<wgrid, 256, 0, st>>>(e.prev[e.prev_flip].template as<T>(), s.pending.template as<T>(), in, in_stride, int(B),
                                                        int(pos), int(end), s.window.template as<T>());
         NEO_TRY(check_launch("lowlat_window_kernel"));
         NEO_TRY(e.window_step(s.window.template as<T>(), s.window_y.template as<T>(), false, st));
+        if (both) {
+            lowlat_use_spare const use_b(e.filter, s.spare_head);
+            NEO_TRY(e.window_step(s.window.template as<T>(), s.fade_y.template as<T>(), false, st));
+        }
         dim3 const grid(unsigned((end + 255) / 256), unsigned(C));
         lowlat_combine_kernel<T><<<grid, 256, 0, st>>>(s.window_y.template as<T>() + B, 2 * B, int(pos), int(end), nullptr, 0, out, out_stride,
-                                                       nullptr, 0, lv);
+                                                       nullptr, 0, lv, both ? s.fade_y.template as<T>() + B : nullptr, lvb, fade);
         NEO_TRY(check_launch("lowlat_combine_kernel"));
     }
     if (!completes) {
         h->sample_pos = end;
+        lowlat_finish_fade<T>(h);
         return NEO_B200_OK;
     }
     h->block_pos  = tb + 1;
@@ -1962,6 +2071,11 @@ int lowlat_segment(neo_b200_lowlat* h, T const* in, size_t in_stride, T* out, si
     // Sample-granular calls keep this: every segment of block b reads plane slot b mod 2 T_i, which only a frame released after block b
     // completes rewrites, so after every segment of block b in stream order; the wait for block b is enqueued before its first segment
     // (pos == 0); partial segments write neither the input ring nor the half-window, and the pending buffer is the head stream's alone.
+    // A crossfade keeps it too. During a fade a frame runs the A side into `plane` while any of its blocks precedes the fade's end, and the
+    // B side into `plane_b` while any follows its start; both sides are on the same side stream before done[i][f % 2], and the plane_b
+    // slots have the same readers at the same blocks as the plane slots. When the fade ends the two plane sets trade places: the new
+    // `plane` holds B for every block the head reads from then on, and the old A planes are next written by a B side released after the
+    // next crossfade call, behind a `ready` recorded after every head block that read them.
     // Every kernel sums in a fixed order and none uses atomics, so the bits do not depend on how the streams interleave
     // (NEO_B200_LOWLAT_SYNC runs the same kernels on the head's stream).
     for (size_t i = 0; i < h->levels; ++i) {
@@ -1973,11 +2087,32 @@ int lowlat_segment(neo_b200_lowlat* h, T const* in, size_t in_stride, T* out, si
             NEO_CUDA_TRY(cudaEventRecord(h->ready[i], st));
             NEO_CUDA_TRY(cudaStreamWaitEvent(ls, h->ready[i], 0));
         }
-        conv_engine<T>& e = s.level[i];
-        NEO_TRY(e.forward(s.in_ring.template as<T>() + ((f * ti) % h->ring_blocks) * B, ring_stride, ti, ls));
-        NEO_TRY(e.inverse(static_cast<cx<T> const*>(e.acc_r()), 0, 1, s.plane[i].template as<T>() + (f % 2) * ti * B, 2 * ti * B, 0, C, ti, ls));
+        conv_engine<T>& e   = s.level[i];
+        T const* const frm  = s.in_ring.template as<T>() + ((f * ti) % h->ring_blocks) * B;
+        size_t const first  = (f + 2) * ti * B, last = (f + 3) * ti * B;  // the samples this frame's output covers
+        bool const side_a   = !h->fading || first < h->fade_end;
+        bool const side_b   = h->fading && last > h->fade_start;
+        size_t const slot   = (f % 2) * ti * B;
+        if (!side_b) {
+            NEO_TRY(e.forward(frm, ring_stride, ti, ls));
+            NEO_TRY(e.inverse(static_cast<cx<T> const*>(e.acc_r()), 0, 1, s.plane[i].template as<T>() + slot, 2 * ti * B, 0, C, ti, ls));
+        } else {
+            // one insert; the second forward_mac stores the same ring slot with the same bits; one advance
+            NEO_TRY(e.forward_r2c(frm, ring_stride, ti, 0, C, ls));
+            if (side_a) {
+                NEO_TRY(e.forward_mac(ti, 0, C, ls));
+                NEO_TRY(e.inverse(e.acc_w(), 0, 1, s.plane[i].template as<T>() + slot, 2 * ti * B, 0, C, ti, ls));
+            }
+            {
+                lowlat_use_spare const use_b(e.filter2, s.spare_level[i]);
+                NEO_TRY(e.forward_mac(ti, 0, C, ls));
+            }
+            NEO_TRY(e.inverse(e.acc_w(), 0, 1, s.plane_b[i].template as<T>() + slot, 2 * ti * B, 0, C, ti, ls));
+            e.advance(ti);
+        }
         if (!h->sync) { NEO_CUDA_TRY(cudaEventRecord(h->done[i][f & 1], ls)); }
     }
+    lowlat_finish_fade<T>(h);
     return NEO_B200_OK;
 }
 
@@ -2068,6 +2203,99 @@ int lowlat_set_filter_impl(neo_b200_lowlat* h, void const* H, void const* ir, si
     }
     NEO_TRY(lowlat_clear<T>(h));
     h->has_filter = true;
+    return NEO_B200_OK;
+}
+
+// builds H / ir into the spare set on the staging stream; the current set, the delay lines and the position are not touched
+extern "C++" template<typename T>
+int lowlat_stage_impl(neo_b200_lowlat* h, void const* H, void const* ir, size_t taps, int memspace)
+{
+    lowlat_state<T>& s   = lowlat_of<T>(h);
+    size_t const C = h->cfg.channels, B = h->cfg.block;
+    if (h->stage_stream == nullptr) {
+        int least = 0, greatest = 0;
+        NEO_CUDA_TRY(cudaDeviceGetStreamPriorityRange(&least, &greatest));
+        NEO_CUDA_TRY(cudaStreamCreateWithPriority(&h->stage_stream, cudaStreamNonBlocking, least));
+        for (cudaEvent_t& ev : h->stage_after) { NEO_CUDA_TRY(cudaEventCreateWithFlags(&ev, cudaEventDisableTiming)); }
+    }
+    cudaStream_t const ss = h->stage_stream;
+    NEO_TRY(s.spare_head.reserve(s.head.filter.bytes));
+    NEO_TRY(s.fade_y.reserve(C * (h->fused ? 1 : 2) * B * sizeof(T)));
+    for (size_t i = 0; i < h->levels; ++i) {
+        NEO_TRY(s.spare_level[i].reserve(s.level[i].filter2.bytes));
+        NEO_TRY(s.plane_b[i].reserve(s.plane[i].bytes));
+    }
+    // the spare set may still be read by enqueued work: the A side of a fade that has just ended
+    NEO_CUDA_TRY(cudaEventRecord(h->stage_after[0], h->stream.stream));
+    NEO_CUDA_TRY(cudaStreamWaitEvent(ss, h->stage_after[0], 0));
+    for (size_t i = 0; i < h->levels && !h->sync; ++i) {
+        NEO_CUDA_TRY(cudaEventRecord(h->stage_after[1 + i], h->side[i]));
+        NEO_CUDA_TRY(cudaStreamWaitEvent(ss, h->stage_after[1 + i], 0));
+    }
+    h->staged = false;
+    {
+        lowlat_use_spare const use(s.head.filter, s.spare_head);
+        NEO_TRY(ir != nullptr ? s.head.load_impulse(ir, taps, memspace, ss) : s.head.load_filter(H, memspace, ss));
+    }
+    for (size_t i = 0; i < h->levels; ++i) {
+        lowlat_use_spare const use(s.level[i].filter2, s.spare_level[i]);
+        NEO_TRY(ir != nullptr ? s.level[i].load_impulse(ir, taps, memspace, ss) : s.level[i].load_filter(H, memspace, ss));
+    }
+    NEO_CUDA_TRY(cudaStreamSynchronize(ss));
+    h->staged = true;
+    return NEO_B200_OK;
+}
+
+extern "C++" static int lowlat_stage_check(neo_b200_lowlat* h)
+{
+    if (!h->has_filter) { return fail(NEO_B200_ERR_INVALID, "no filter set: stage needs a current filter to fade from"); }
+    if (h->fading) { return fail(NEO_B200_ERR_INVALID, "a crossfade is pending or running"); }
+    NEO_CUDA_TRY(cudaSetDevice(h->device));
+    return NEO_B200_OK;
+}
+
+int neo_b200_lowlat_stage_filter(neo_b200_lowlat* handle, void const* H, int memspace)
+{
+    if (handle == nullptr || H == nullptr) { return fail(NEO_B200_ERR_INVALID, "null argument"); }
+    NEO_TRY(lowlat_stage_check(handle));
+    if (handle->cfg.dtype == NEO_B200_F32) { return lowlat_stage_impl<float>(handle, H, nullptr, 0, memspace); }
+    return lowlat_stage_impl<double>(handle, H, nullptr, 0, memspace);
+}
+
+int neo_b200_lowlat_stage_impulse(neo_b200_lowlat* handle, void const* ir, size_t taps, int memspace)
+{
+    if (handle == nullptr || ir == nullptr) { return fail(NEO_B200_ERR_INVALID, "null argument"); }
+    if (taps < handle->cfg.block) { return fail(NEO_B200_ERR_INVALID, "impulse response shorter than one block"); }
+    if (neo_b200_num_partitions(taps, handle->cfg.block) > handle->cfg.partitions) {
+        return fail(NEO_B200_ERR_INVALID, "taps=%zu gives %zu partitions, the handle holds %zu", taps, neo_b200_num_partitions(taps, handle->cfg.block),
+                    handle->cfg.partitions);
+    }
+    NEO_TRY(lowlat_stage_check(handle));
+    if (handle->cfg.dtype == NEO_B200_F32) { return lowlat_stage_impl<float>(handle, nullptr, ir, taps, memspace); }
+    return lowlat_stage_impl<double>(handle, nullptr, ir, taps, memspace);
+}
+
+int neo_b200_lowlat_crossfade(neo_b200_lowlat* handle, size_t fade, size_t* start)
+{
+    if (handle == nullptr) { return fail(NEO_B200_ERR_INVALID, "null argument"); }
+    if (handle->fading) { return fail(NEO_B200_ERR_INVALID, "a crossfade is already pending or running"); }
+    if (!handle->staged) { return fail(NEO_B200_ERR_INVALID, "nothing staged: call neo_b200_lowlat_stage_filter / _stage_impulse first"); }
+    // level i's B side starts with the first frame released after this call, floor(b / T_i), whose output begins at block
+    // (floor(b / T_i) + 2) T_i; b is the block holding the next sample. With no levels the head alone starts at the next sample.
+    size_t at = handle->position();
+    if (handle->levels > 0) {
+        size_t b0 = 0;
+        for (size_t i = 0; i < handle->levels; ++i) { b0 = std::max(b0, (handle->block_pos / handle->t[i] + 2) * handle->t[i]); }
+        at = b0 * handle->cfg.block;
+    }
+    if (fade > SIZE_MAX - at) { return fail(NEO_B200_ERR_INVALID, "fade of %zu samples overflows the stream position", fade); }
+    NEO_CUDA_TRY(cudaSetDevice(handle->device));
+    handle->fading     = true;
+    handle->fade_start = at;
+    handle->fade_end   = at + fade;
+    if (start != nullptr) { *start = at; }
+    if (handle->cfg.dtype == NEO_B200_F32) { lowlat_finish_fade<float>(handle); }
+    else { lowlat_finish_fade<double>(handle); }
     return NEO_B200_OK;
 }
 

@@ -16,6 +16,10 @@
 // completing segment (end == B) is the whole-block computation on the whole block. Only a whole, pair-aligned block uses 8- / 16-byte
 // accesses on `in` / `out`; every other segment reads and writes them one real at a time, as its rows may start at any sample.
 //
+// A crossfade to a staged filter (neo_b200_lowlat_crossfade) runs the kernel twice for a segment with samples on both sides of the
+// fade's start .. end: first with filter B and B's level planes in an outputs-only mode (commit = 0: no half-window, delay-line,
+// input-ring or pending write) into a [C][B] scratch, then with filter A as always, blending with the scratch per sample at the store.
+//
 // Layouts (shared with conv_engine, whose head-range handle owns filter, delay line and half-window buffers):
 //   fdl    [C][B/W][R][W]    ring of head spectra, R = 2*T_1 rows, bin 0 packed as (Re X[0], Re X[B])
 //   filter [C][B/W][Ph][W]   head partitions, same packing
@@ -34,6 +38,22 @@ struct lowlat_levels
     T const* plane[k_lowlat_max_levels];   // level i's partial output of THIS block, channel 0
     size_t stride[k_lowlat_max_levels];    // reals between channels of a plane
 };
+
+// a crossfade (neo_b200_lowlat_crossfade): out = y_A before `start`, y_A + g (y_B - y_A) with g = (t - start) / len inside, y_B after
+struct lowlat_fade
+{
+    unsigned long long t0;          // absolute sample index of block position 0
+    unsigned long long start, len;  // the fade covers samples [start, start + len)
+};
+
+template<typename T>
+__device__ __forceinline__ T lowlat_blend(T ya, T yb, unsigned long long t, lowlat_fade const& f)
+{
+    if (t < f.start) { return ya; }
+    if (t - f.start >= f.len) { return yb; }
+    T const g = T(double(t - f.start) / double(f.len));
+    return ya + g * (yb - ya);
+}
 
 template<typename T>
 struct lowlat_head_args
@@ -54,6 +74,9 @@ struct lowlat_head_args
     T* pending;    // [C][B] samples [0, pos) of the current block, delivered by earlier calls
     int pos, end;  // this segment covers block positions [pos, end); `in` / `out` point at position pos
     int vec;       // pos == 0, end == B and every row of `in` / `out` starts on a complex pair: 8- / 16-byte accesses
+    int commit;    // 0: outputs only (the B side of a crossfade): no half-window, delay-line, input-ring or pending writes
+    T const* fade_y;  // [C][B] the B side's outputs of this segment by block position, blended in by `fade`; nullptr: no crossfade
+    lowlat_fade fade;
 };
 
 // sample j of the new half-window of a segment: pending, then `in`, then zeros
@@ -98,8 +121,8 @@ __device__ __forceinline__ size_t lowlat_tiled(int ring_rows, int logw, int k)
 
 // One CTA holds G channels (fft_cfg); thread t owns the Hermitian pairs (k, M-k), k = t + e*TN for e < E/2 -- the same bins in the
 // r2c post-pass, the MAC and the c2r pre-pass, so the accumulators never leave registers. Thread 0's pair e = 0 is (packed bin 0,
-// bin M/2).
-template<typename T, int LOGM>
+// bin M/2). XF: a segment inside a crossfade (a.commit and a.fade_y are read); the instantiation every other segment runs is free of both.
+template<typename T, int LOGM, bool XF>
 __global__ void __launch_bounds__(fft_cfg<T, LOGM>::THREADS, lowlat_min_ctas<T, LOGM>())
     lowlat_head_kernel(lowlat_head_args<T> a, cx<T> const* __restrict__ tw, cx<T> const* __restrict__ rtw)
 {
@@ -130,8 +153,9 @@ __global__ void __launch_bounds__(fft_cfg<T, LOGM>::THREADS, lowlat_min_ctas<T, 
         else { v[e] = mk<T>(lowlat_sample(a, pend, src, 2 * j), lowlat_sample(a, pend, src, 2 * j + 1)); }
     }
     // 9. a completed block is the next left half-window and the levels' input (both buffers are distinct from in / out); a partial
-    // segment keeps its samples for the segments that follow
-    if (live && whole) {
+    // segment keeps its samples for the segments that follow. An outputs-only run writes none of them
+    bool const keep = live && (!XF || a.commit);
+    if (keep && whole) {
         C* const keep = reinterpret_cast<C*>(a.prev_next + row * M);
         C* const ring = reinterpret_cast<C*>(a.in_ring + row * a.ring_stride);
 #pragma unroll
@@ -139,7 +163,7 @@ __global__ void __launch_bounds__(fft_cfg<T, LOGM>::THREADS, lowlat_min_ctas<T, 
             keep[t + (e - HALF) * TN] = v[e];
             ring[t + (e - HALF) * TN] = v[e];
         }
-    } else if (live) {
+    } else if (keep) {
 #pragma unroll
         for (int e = HALF; e < E; ++e) {
             int const j = 2 * (t + (e - HALF) * TN);
@@ -174,7 +198,7 @@ __global__ void __launch_bounds__(fft_cfg<T, LOGM>::THREADS, lowlat_min_ctas<T, 
     for (int e = 0; e < HALF; ++e) {
         int const k  = t + e * TN;
         int const km = k == 0 ? M / 2 : M - k;
-        if (live && whole) {
+        if (keep && whole) {
             x_row[lowlat_tiled(a.ring, a.logw, k) + (size_t(a.wp) << a.logw)]  = xk[e];
             x_row[lowlat_tiled(a.ring, a.logw, km) + (size_t(a.wp) << a.logw)] = xm[e];
         }
@@ -229,7 +253,8 @@ __global__ void __launch_bounds__(fft_cfg<T, LOGM>::THREADS, lowlat_min_ctas<T, 
     __syncthreads();
     cta_fft<T, LOGM, +1>::run(v, sm, tw, t);
 
-    // 6.-8. scale, keep samples [B, 2B), add the levels in level order, store positions [pos, end)
+    // 6.-8. scale, keep samples [B, 2B), add the levels in level order, blend with the B side inside a crossfade, store positions
+    // [pos, end)
     if (live) {
         T const scale = T(1) / T(2 * M);
         T* const o    = a.out + row * a.out_stride;
@@ -246,6 +271,11 @@ __global__ void __launch_bounds__(fft_cfg<T, LOGM>::THREADS, lowlat_min_ctas<T, 
                     y.y += l.y;
                 }
             }
+            if (XF && a.fade_y != nullptr) {
+                C const yb = reinterpret_cast<C const*>(a.fade_y + row * M)[j];
+                y.x        = lowlat_blend(y.x, yb.x, a.fade.t0 + 2 * j, a.fade);
+                y.y        = lowlat_blend(y.y, yb.y, a.fade.t0 + 2 * j + 1, a.fade);
+            }
             if (a.vec) { dst[j] = y; }
             else {
                 if (2 * j >= a.pos && 2 * j < a.end) { o[2 * j - a.pos] = y.x; }
@@ -255,23 +285,34 @@ __global__ void __launch_bounds__(fft_cfg<T, LOGM>::THREADS, lowlat_min_ctas<T, 
     }
 }
 
+// head + levels (level order) at block position i of channel ch
+template<typename T>
+__device__ __forceinline__ T lowlat_sum(T const* head, size_t head_stride, lowlat_levels<T> const& levels, size_t ch, int i)
+{
+    T y = head[ch * head_stride + i];
+#pragma unroll
+    for (int l = 0; l < k_lowlat_max_levels; ++l) {
+        if (l < levels.count) { y += levels.plane[l][ch * levels.stride[l] + i]; }
+    }
+    return y;
+}
+
 // the unfused form's tail over block positions [0, end): with an input ring, the block (`in` from position 0) into it; for positions
-// [first, end), out = head + levels (level order), `out` pointing at position `first`. grid (ceil(end/256), C)
+// [first, end), out = head + levels (level order), `out` pointing at position `first`; with head_b, the B side's head_b + levels_b is
+// blended in by `fade`. grid (ceil(end/256), C)
 template<typename T>
 __global__ void __launch_bounds__(256) lowlat_combine_kernel(T const* __restrict__ head, size_t head_stride, int first, int end, T const* in,
                                                              size_t in_stride, T* out, size_t out_stride, T* __restrict__ in_ring,
-                                                             size_t ring_stride, lowlat_levels<T> levels)
+                                                             size_t ring_stride, lowlat_levels<T> levels, T const* __restrict__ head_b,
+                                                             lowlat_levels<T> levels_b, lowlat_fade fade)
 {
     size_t const ch = blockIdx.y;
     int const i     = blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= end) { return; }
     if (in_ring != nullptr) { in_ring[ch * ring_stride + i] = in[ch * in_stride + i]; }  // read before the store below: in == out is allowed
     if (i < first) { return; }
-    T y = head[ch * head_stride + i];
-#pragma unroll
-    for (int l = 0; l < k_lowlat_max_levels; ++l) {
-        if (l < levels.count) { y += levels.plane[l][ch * levels.stride[l] + i]; }
-    }
+    T y = lowlat_sum(head, head_stride, levels, ch, i);
+    if (head_b != nullptr) { y = lowlat_blend(y, lowlat_sum(head_b, head_stride, levels_b, ch, i), fade.t0 + unsigned(i), fade); }
     out[ch * out_stride + (i - first)] = y;
 }
 
