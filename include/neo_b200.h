@@ -270,8 +270,30 @@ NEO_B200_API int neo_b200_conv_set_filter_csr(neo_b200_conv* conv, void const* v
                                               uint64_t const* filter_base);
 /* same, starting from time-domain impulse responses [filters][taps] (uniform_partition fused in, on the device) */
 NEO_B200_API int neo_b200_conv_set_impulse(neo_b200_conv* conv, void const* ir, size_t taps, int memspace);
-/* zero window / FDL / write position, keep the filter */
+/* zero window / FDL / write position, keep the filter; cancels a pending or running crossfade and drops the staged filter (the current
+ * filter is A until the fade has ended, B after) */
 NEO_B200_API int neo_b200_conv_reset(neo_b200_conv* conv);
+/* switch to a new filter mid-stream with a sample-accurate linear crossfade, keeping the delay line (DESIGN §4.6b).
+ * stage_filter / stage_impulse build a second filter set B next to the current set A, on the handle's stream behind any enqueued work,
+ * and return when B is ready. They change no output and touch no delay line, half-window, write position or sample count. H and ir have
+ * the set_filter / set_impulse layouts; ir needs block <= taps and num_partitions(taps, block) <= P, a shorter response is zero-padded
+ * to P partitions. Staging again before a crossfade replaces B. Device bytes grow by the spare set and a [outputs][max_blocks*B] scratch
+ * at the first stage. */
+NEO_B200_API int neo_b200_conv_stage_filter(neo_b200_conv* conv, void const* H, int memspace);
+NEO_B200_API int neo_b200_conv_stage_impulse(neo_b200_conv* conv, void const* ir, size_t taps, int memspace);
+/* starts the switch to the staged set at start = (samples per channel delivered since the last reset / set_filter / set_impulse) + delay,
+ * returned in *start (may be NULL). Every channel's output at sample t is y_A(t) for t < start, y_A(t) + g (y_B(t) - y_A(t)) with
+ * g = (t - start) / fade (computed in double, rounded to the handle's type) for start <= t < start + fade, and y_B(t) from start + fade on
+ * (fade = 0: a hard switch); y_B is the output of B over the whole stream. `delay` places the switch at any sample of a later call, also
+ * inside a frame-mode call. Once a call has delivered sample start + fade - 1, B is the current filter and A the spare. A call inside
+ * [start, start + fade) runs the MAC and the inverse transform once per filter; every other call runs exactly as without a crossfade.
+ * Bits: samples before start are those of the handle without the crossfade, samples from start + fade on those of a handle given B at
+ * its last reset and fed the same calls; HOST (pinned or pageable) and DEVICE calls agree. Errors: NEO_B200_ERR_INVALID with nothing
+ * staged, before any filter, with a crossfade pending or running (stage_* and crossfade) or a forward_range call in progress;
+ * NEO_B200_ERR_UNSUPPORTED on overlap-add (UPOLA) handles, whose carried tail depends on the filter, on partition-sharded handles and on
+ * filters from set_filter_csr. neo_b200_conv_forward / _forward_range / _inverse / _process_window are rejected (INVALID) while a
+ * crossfade is pending or running: they produce partial spectra or windows, not an output to blend. */
+NEO_B200_API int neo_b200_conv_crossfade(neo_b200_conv* conv, size_t delay, size_t fade, size_t* start);
 
 /* `convolver(block)` (uniform_partitioned_convolver.hpp:48-65) for every channel of the bank, `blocks` consecutive
  * blocks per call: in [inputs][blocks*B] -> out [outputs][blocks*B] reals; in == out allowed for DIAGONAL (the

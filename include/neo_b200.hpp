@@ -509,7 +509,24 @@ struct convolver_bank
         detail::check(neo_b200_conv_process(_conv, in, out, blocks, memspace));
     }
 
+    /// a second filter next to the current one, in filter()'s layout (stage_filter) or as impulse responses [outputs][(inputs)][taps]
+    /// (stage_impulse, zero-padded when shorter); no output or state changes. `crossfade(fade, delay)` then fades to it linearly over
+    /// `fade` samples from `delay` samples after the last one delivered, keeping the delay line, and returns the fade's first sample
+    /// (neo_b200_conv_stage_filter / _stage_impulse / _crossfade; overlap-save banks)
+    auto stage_filter(complex_type const* h, int memspace = NEO_B200_HOST) -> void { detail::check(neo_b200_conv_stage_filter(_conv, h, memspace)); }
+    auto stage_impulse(Float const* ir, size_type taps, int memspace = NEO_B200_HOST) -> void
+    {
+        detail::check(neo_b200_conv_stage_impulse(_conv, ir, taps, memspace));
+    }
+    auto crossfade(size_type fade, size_type delay = 0) -> size_type
+    {
+        size_type start = 0;
+        detail::check(neo_b200_conv_crossfade(_conv, delay, fade, &start));
+        return start;
+    }
+
     [[nodiscard]] auto block_size() const noexcept -> size_type { return _cfg.block; }
+    [[nodiscard]] auto partitions() const noexcept -> size_type { return _cfg.partitions; }
     [[nodiscard]] auto device_bytes() const noexcept -> size_type { return neo_b200_conv_device_bytes(_conv); }
     [[nodiscard]] auto handle() const noexcept -> neo_b200_conv* { return _conv; }
 
@@ -686,6 +703,31 @@ struct uniform_partitioned_convolver
             ptr = _copy.data();
         }
         _bank.filter(ptr, 1, 1, parts, bins, NEO_B200_DIAGONAL);
+    }
+
+    /// switches to `h` (the H[P][B+1] view filter() takes, same P and B) with a linear crossfade of `fade` samples from the next sample
+    /// on, keeping the delay line; returns the index of the fade's first sample, counted from the last filter() call. Overlap-save
+    /// only: an overlap-add convolver's carried tail belongs to its filter. Throws while an earlier crossfade has not ended.
+    template<typename Mat>
+    auto crossfade_to(Mat h, std::size_t fade) -> std::size_t
+    {
+        static_assert(Kind == NEO_B200_UPOLS, "crossfade_to: overlap-save convolvers only (upols_convolver)");
+        static_assert(std::is_same_v<detail::element_of<Mat>, Complex>);
+        auto const parts = static_cast<std::size_t>(h.extent(0));
+        auto const bins  = static_cast<std::size_t>(h.extent(1));
+        if (_bank.handle() == nullptr) { throw std::invalid_argument{"neo::b200::uniform_partitioned_convolver: filter() has not been called"}; }
+        if (parts != _bank.partitions() || bins != _bank.block_size() + 1) {
+            throw std::invalid_argument{"neo::b200::uniform_partitioned_convolver: crossfade_to() needs the shape filter() was given"};
+        }
+        _copy.resize(parts * bins);
+        for (std::size_t p = 0; p < parts; ++p) {
+            for (std::size_t k = 0; k < bins; ++k) {
+                auto const v        = h(p, k);
+                _copy[p * bins + k] = std::complex<real_type>{v.real(), v.imag()};
+            }
+        }
+        _bank.stage_filter(_copy.data());
+        return _bank.crossfade(fade);
     }
 
     /// the CSR containers of the last sparse filter() call (row_container, column_container: csr_matrix.hpp:46-48) and what the

@@ -144,6 +144,9 @@ SIGNATURES = {
     "neo_b200_compressed_fdl_row": (_i, [_vp, _sz, _vp, _i]),
     "neo_b200_compressed_fdl_raw": (_i, [_vp, _sz, _vp]),
     "neo_b200_conv_set_impulse": (_i, [_vp, _vp, _sz, _i]),
+    "neo_b200_conv_stage_filter": (_i, [_vp, _vp, _i]),
+    "neo_b200_conv_stage_impulse": (_i, [_vp, _vp, _sz, _i]),
+    "neo_b200_conv_crossfade": (_i, [_vp, _sz, _sz, C.POINTER(_sz)]),
     "neo_b200_conv_reset": (_i, [_vp]),
     "neo_b200_conv_process": (_i, [_vp, _vp, _vp, _sz, _i]),
     "neo_b200_conv_forward": (_i, [_vp, _vp, _sz, _i]),
@@ -600,7 +603,8 @@ class Convolver:
     """A bank of neo::convolution::upols_convolver / upola_convolver instances
     (convolution/uniform_partitioned_convolver.hpp:14-65): `filter(H)` then call on blocks.
 
-    H: DIAGONAL [C][P][B+1] (channel c has its own filter), MATRIX [O][I][P][B+1].
+    H: DIAGONAL [C][P][B+1] (channel c has its own filter), MATRIX [O][I][P][B+1]. `stage_filter(H)` / `stage_impulse(ir)` then
+    `crossfade(fade, delay)` switch to a new response mid-stream with a linear crossfade, keeping the delay line (overlap-save).
     """
 
     def __init__(self, kind: int = UPOLS, dtype="float32", topology: int = DIAGONAL, max_blocks: int = 1,
@@ -674,6 +678,44 @@ class Convolver:
         taps = int(ir.shape[-1])
         self._create(outputs, inputs, block, num_partitions(taps, block))
         _check(library().neo_b200_conv_set_impulse(self._h, _ptr(ir), taps, _space(ir)))
+
+    def stage_filter(self, H) -> None:
+        """H of this handle's shape ([C][P][B+1] diagonal, [O][I][P][B+1] matrix), prepared next to the current filter for
+        `crossfade`: no output, delay line or sample count changes (neo_b200_conv_stage_filter)."""
+        if self.cfg is None:
+            raise RuntimeError("no filter set")
+        lead = (int(self.cfg.outputs),) if self.topology == DIAGONAL else (int(self.cfg.outputs), int(self.cfg.inputs))
+        shape = lead + (int(self.cfg.partitions), int(self.cfg.block) + 1)
+        if H.ndim != len(shape) or tuple(int(n) for n in H.shape) != shape:
+            raise ValueError(f"filter must have the shape {list(shape)}")
+        if _dtype_name(H) != ("complex64" if self.real == "float32" else "complex128"):
+            raise ValueError("filter dtype does not match the convolver")
+        _check(library().neo_b200_conv_stage_filter(self._h, _ptr(H), _space(H)))
+
+    def stage_impulse(self, ir) -> None:
+        """stage_filter(uniform_partition(ir, B)) for ir [C][taps] / [O][I][taps], B <= taps, num_partitions(taps, B) <= P; a shorter
+        response is zero-padded to the handle's P partitions."""
+        if self.cfg is None:
+            raise RuntimeError("no filter set")
+        lead = (int(self.cfg.outputs),) if self.topology == DIAGONAL else (int(self.cfg.outputs), int(self.cfg.inputs))
+        if ir.ndim != len(lead) + 1 or tuple(int(n) for n in ir.shape[:-1]) != lead or _dtype_name(ir) != self.real:
+            raise ValueError("impulse response shape/dtype mismatch")
+        taps, block = int(ir.shape[-1]), int(self.cfg.block)
+        if taps < block or num_partitions(taps, block) > self.cfg.partitions:
+            raise ValueError(f"impulse response of {taps} taps does not fit {self.cfg.partitions} partitions of {block}")
+        _check(library().neo_b200_conv_stage_impulse(self._h, _ptr(ir), taps, _space(ir)))
+
+    def crossfade(self, fade: int, delay: int = 0) -> int:
+        """Switch to the staged filter with a linear fade of `fade` samples (0: hard switch) that starts `delay` samples after the
+        last sample delivered so far, inside any later call. Returns `start`, the absolute index (samples since the last reset /
+        filter / impulse) of the fade's first sample (neo_b200_conv_crossfade)."""
+        if self.cfg is None:
+            raise RuntimeError("no filter set")
+        if int(fade) < 0 or int(delay) < 0:
+            raise ValueError("fade and delay must be >= 0")
+        start = _sz(0)
+        _check(library().neo_b200_conv_crossfade(self._h, int(delay), int(fade), C.byref(start)))
+        return int(start.value)
 
     def set_stream(self, stream) -> None:
         self._stream = _stream_ptr(stream)

@@ -52,6 +52,17 @@ __global__ void digitrev_perm_kernel(unsigned radix, unsigned digits, unsigned s
 
 namespace {
 
+// an engine runs with the spare filter for the lifetime of this guard (staging and the B side of a crossfade)
+struct use_spare
+{
+    device_buffer& a;
+    device_buffer& b;
+    use_spare(device_buffer& filter, device_buffer& spare) : a(filter), b(spare) { a.swap(b); }
+    ~use_spare() { a.swap(b); }
+    use_spare(use_spare const&)            = delete;
+    use_spare& operator=(use_spare const&) = delete;
+};
+
 template<typename T>
 struct conv_engine
 {
@@ -94,6 +105,11 @@ struct conv_engine
     cx<T>* acc_w() const { return (acc_cur != 0 ? acc_alt : acc).template as<cx<T>>(); }
     void* acc_r() const { return in_call ? static_cast<void*>(acc_w()) : (acc_last != 0 ? acc_alt : acc).ptr; }
     int prev_flip{0};  // prev[prev_flip] holds the last block of the previous call
+    size_t samples{0};  // samples per channel the delay line has advanced by since clear_state
+    // crossfade (neo_b200_conv_stage_* / _crossfade), allocated by the first stage: the spare filter set (`filter`'s twin in the direct
+    // form, `filter2`'s in frame mode) and the B side's outputs of a call inside the fade, [outputs][max_blocks B] reals
+    device_buffer spare_filter, fade_y;
+    device_buffer& live_filter() { return frame > 0 ? filter2 : filter; }
 
     // second partition level along block time (conv_frame.cuh). frame == 0: direct form. In frame mode `fdl` is the two-frame
     // level-1 spectra buffer x1 (2T plain rows of B per channel, not tiled) and `filter` only lives while a filter is prepared.
@@ -200,7 +216,7 @@ struct conv_engine
     size_t device_bytes() const
     {
         return sp_meta.bytes + sp_vals.bytes + sp_base.bytes + filter.bytes + fdl.bytes + prev[0].bytes + prev[1].bytes + tail.bytes + acc.bytes + acc_alt.bytes + ola_y.bytes + stage_in.bytes
-             + stage_out.bytes + stage_filter.bytes + fdl2.bytes + filter2.bytes + acc2.bytes + nyq_acc.bytes;
+             + stage_out.bytes + stage_filter.bytes + fdl2.bytes + filter2.bytes + acc2.bytes + nyq_acc.bytes + spare_filter.bytes + fade_y.bytes;
     }
 
     int init(neo_b200_conv_config const& c, cudaStream_t stream)
@@ -300,6 +316,7 @@ struct conv_engine
         write_pos  = 0;
         write_pos2 = 0;
         x1_half    = 0;
+        samples    = 0;
         in_call    = false;  // a reset in the middle of a grouped call abandons it
         range_next = range_blocks = 0;
         acc_cur = acc_last = 0;
@@ -497,6 +514,16 @@ struct conv_engine
             }
         }
         return build_filter(stream);
+    }
+
+    // builds H / ir into the spare filter set through load_filter / load_impulse (neo_b200_conv_stage_*): the current filter, the delay
+    // line, the half-window and the ring position stay as they are. The spare set and fade_y are allocated once and reused.
+    int stage(void const* h, void const* ir, size_t taps, int memspace, cudaStream_t stream)
+    {
+        NEO_TRY(spare_filter.reserve(live_filter().bytes));
+        NEO_TRY(fade_y.reserve(cfg.outputs * cfg.max_blocks * size_t(m) * sizeof(T)));
+        use_spare const use(live_filter(), spare_filter);
+        return ir != nullptr ? load_impulse(ir, taps, memspace, stream) : load_filter(h, memspace, stream);
     }
 
     // the wide kernels move the real rows with 128-bit accesses
@@ -738,6 +765,7 @@ struct conv_engine
         }
         prev_flip ^= 1;  // the r2c kernels saved this call's last block into the other half-window buffer
         in_call = false;
+        samples += blocks * size_t(m);
         if (acc_alt.ptr != nullptr) {
             acc_last = acc_cur;
             acc_cur ^= 1;
@@ -816,6 +844,47 @@ struct conv_engine
     {
         cx<T> const* one[1] = {spectra};
         return inverse_sum(one, 1, out, out_stride, first, count, blocks, stream);
+    }
+
+    // overlap-save c2r of spectra [count][blocks][B] into out [count][out_stride] with the kernel the caller picks (wide or cta_fft);
+    // with `fade`, each kept sample is blended with the same place of yb (conv_c2r_fade_io)
+    int inverse_rows(cx<T> const* spectra, T* out, size_t out_stride, size_t count, size_t blocks, bool wide, T const* yb, conv_fade const* fade,
+                     cudaStream_t stream)
+    {
+        int status = NEO_B200_ERR_UNSUPPORTED;
+        NEO_TRY(mark_begin(2, stream));
+        NEO_DISPATCH_LOGM(T, logb, {
+            if constexpr (LOGM >= 1 && LOGM <= max_cta_logm<T>()) {
+                if (fade == nullptr) {
+                    conv_c2r_io<T, LOGM> io{spectra, int(blocks), out, out_stride, T(1) / T(2 * m), 0};
+                    status = run_c2r<LOGM>(io, wide, count * blocks, stream);
+                } else {
+                    conv_c2r_fade_io<T, LOGM> io{spectra, int(blocks), out, out_stride, T(1) / T(2 * m), yb, *fade};
+                    status = run_c2r<LOGM>(io, wide, count * blocks, stream);
+                }
+            }
+        });
+        if (status != NEO_B200_OK) { return status; }
+        return mark_end(2, stream);
+    }
+
+    // outputs [out0, out0 + nout) of a call with samples on both sides of a crossfade's start .. end, after forward_r2c: the MAC under
+    // the spare filter B and its inverse transform into fade_y, then the MAC under A and its inverse transform blended with fade_y at the
+    // store. The second MAC rewrites what the first wrote besides the spectra (frame mode's ring slot and Nyquist accumulators) with the
+    // same bits. The B side takes the c2r kernel the A side takes for `out` (wide or cta_fft: wide_rows_ok looks at the caller's
+    // pointer), so its samples are the bits a handle running B would store there.
+    int fade_step(size_t blocks, size_t out0, size_t nout, T* out, size_t out_stride, conv_fade const& fade, cudaStream_t stream)
+    {
+        bool const wide            = wide_rows_ok(out, out_stride);
+        cx<T> const* const spectra = acc.template as<cx<T>>() + out0 * blocks * size_t(m);
+        T* const yb                = fade_y.template as<T>() + out0 * out_stride;
+        {
+            use_spare const use_b(live_filter(), spare_filter);
+            NEO_TRY(forward_mac(blocks, out0, nout, stream));
+        }
+        NEO_TRY(inverse_rows(spectra, yb, out_stride, nout, blocks, wide, nullptr, nullptr, stream));
+        NEO_TRY(forward_mac(blocks, out0, nout, stream));
+        return inverse_rows(spectra, out, out_stride, nout, blocks, wide, yb, &fade, stream);
     }
 
     // the same for the sum of `nsrc` partial spectra buffers (partition shards of a multi-device bank; peer-mapped pointers are
@@ -921,6 +990,10 @@ struct neo_b200_conv
     // speed and the copies overlap the kernels whatever memory the caller hands over
     pinned_buffer pin_in[2], pin_out[2];
     cudaEvent_t ev_h2d[2]{}, ev_d2h[2]{};
+    // crossfade (neo_b200_conv_stage_* / _crossfade): the engine's spare filter holds B once `staged`; while `fading`, samples
+    // [fade_start, fade_end) blend A into B, and B becomes the current filter once a call has delivered sample fade_end - 1
+    bool staged{false}, fading{false};
+    size_t fade_start{0}, fade_end{0};
 
     int ensure_pipeline(size_t groups)
     {
@@ -997,6 +1070,7 @@ int neo_b200_conv_set_filter(neo_b200_conv* conv, void const* H, int memspace)
 {
     if (conv == nullptr || H == nullptr) { return fail(NEO_B200_ERR_INVALID, "null argument"); }
     NEO_CUDA_TRY(cudaSetDevice(conv->device));
+    conv->staged = conv->fading = false;
     NEO_TRY(NEO_CONV_ENGINE(conv, set_filter(H, memspace, conv->stream.stream)));
     NEO_CUDA_TRY(cudaStreamSynchronize(conv->stream.stream));
     return NEO_B200_OK;
@@ -1008,6 +1082,7 @@ int neo_b200_conv_set_filter_csr(neo_b200_conv* conv, void const* values, uint64
         return fail(NEO_B200_ERR_INVALID, "null argument");
     }
     NEO_CUDA_TRY(cudaSetDevice(conv->device));
+    conv->staged = conv->fading = false;
     if (conv->cfg.dtype == NEO_B200_F32) {
         NEO_TRY(conv->f32.set_filter_csr(static_cast<float2 const*>(values), cols, row_ptr, filter_base, conv->stream.stream));
     } else {
@@ -1027,6 +1102,7 @@ int neo_b200_conv_set_impulse(neo_b200_conv* conv, void const* ir, size_t taps, 
                     neo_b200_num_partitions(taps, conv->cfg.block), conv->cfg.partitions);
     }
     NEO_CUDA_TRY(cudaSetDevice(conv->device));
+    conv->staged = conv->fading = false;
     NEO_TRY(NEO_CONV_ENGINE(conv, set_impulse(ir, taps, memspace, conv->stream.stream)));
     NEO_CUDA_TRY(cudaStreamSynchronize(conv->stream.stream));
     return NEO_B200_OK;
@@ -1036,7 +1112,97 @@ int neo_b200_conv_reset(neo_b200_conv* conv)
 {
     if (conv == nullptr) { return fail(NEO_B200_ERR_INVALID, "null argument"); }
     NEO_CUDA_TRY(cudaSetDevice(conv->device));
+    conv->staged = conv->fading = false;  // the current filter stays: A while the fade has not ended, B after
     return NEO_CONV_ENGINE(conv, clear_state(conv->stream.stream));
+}
+
+// staging and crossfades need a full output to blend and a filter that does not shape the carried state
+static int conv_fade_check(neo_b200_conv* conv)
+{
+    if (conv->cfg.kind == NEO_B200_UPOLA) {
+        return fail(NEO_B200_ERR_UNSUPPORTED, "crossfade: overlap-add handles carry a tail that depends on the filter, so the new filter's "
+                                              "output has no tail at the fade's start; use an overlap-save (UPOLS) handle");
+    }
+    if (conv->sharded) { return fail(NEO_B200_ERR_UNSUPPORTED, "crossfade: partition-sharded handles produce partial spectra, not outputs"); }
+    if (conv->cfg.dtype == NEO_B200_F32 ? conv->f32.sparse : conv->f64.sparse) {
+        return fail(NEO_B200_ERR_UNSUPPORTED, "crossfade: the filter came from set_filter_csr; sparse filters have no spare set");
+    }
+    if (conv->fading) { return fail(NEO_B200_ERR_INVALID, "a crossfade is pending or running"); }
+    return NEO_B200_OK;
+}
+
+extern "C++" template<typename T>
+int conv_stage_impl(neo_b200_conv* conv, conv_engine<T>& e, void const* H, void const* ir, size_t taps, int memspace)
+{
+    cudaStream_t const s = conv->stream.stream;
+    conv->staged         = false;
+    // on the handle's stream: behind every enqueued call, which may still read the spare set (the A side of a fade that has just ended)
+    NEO_TRY(e.stage(H, ir, taps, memspace, s));
+    NEO_CUDA_TRY(cudaStreamSynchronize(s));
+    conv->staged = true;
+    return NEO_B200_OK;
+}
+
+int neo_b200_conv_stage_filter(neo_b200_conv* conv, void const* H, int memspace)
+{
+    if (conv == nullptr || H == nullptr) { return fail(NEO_B200_ERR_INVALID, "null argument"); }
+    if (!(conv->cfg.dtype == NEO_B200_F32 ? conv->f32.has_filter : conv->f64.has_filter)) {
+        return fail(NEO_B200_ERR_INVALID, "no filter set: stage needs a current filter to fade from");
+    }
+    NEO_TRY(conv_fade_check(conv));
+    NEO_CUDA_TRY(cudaSetDevice(conv->device));
+    if (conv->cfg.dtype == NEO_B200_F32) { return conv_stage_impl<float>(conv, conv->f32, H, nullptr, 0, memspace); }
+    return conv_stage_impl<double>(conv, conv->f64, H, nullptr, 0, memspace);
+}
+
+int neo_b200_conv_stage_impulse(neo_b200_conv* conv, void const* ir, size_t taps, int memspace)
+{
+    if (conv == nullptr || ir == nullptr) { return fail(NEO_B200_ERR_INVALID, "null argument"); }
+    if (!(conv->cfg.dtype == NEO_B200_F32 ? conv->f32.has_filter : conv->f64.has_filter)) {
+        return fail(NEO_B200_ERR_INVALID, "no filter set: stage needs a current filter to fade from");
+    }
+    NEO_TRY(conv_fade_check(conv));
+    if (taps < conv->cfg.block) { return fail(NEO_B200_ERR_INVALID, "impulse response shorter than one block"); }
+    if (neo_b200_num_partitions(taps, conv->cfg.block) > conv->cfg.partitions) {
+        return fail(NEO_B200_ERR_INVALID, "taps=%zu gives %zu partitions, the handle holds %zu", taps, neo_b200_num_partitions(taps, conv->cfg.block),
+                    conv->cfg.partitions);
+    }
+    NEO_CUDA_TRY(cudaSetDevice(conv->device));
+    if (conv->cfg.dtype == NEO_B200_F32) { return conv_stage_impl<float>(conv, conv->f32, nullptr, ir, taps, memspace); }
+    return conv_stage_impl<double>(conv, conv->f64, nullptr, ir, taps, memspace);
+}
+
+// samples per channel delivered since the last reset / set_filter / set_impulse
+static size_t conv_position(neo_b200_conv const* conv) { return conv->cfg.dtype == NEO_B200_F32 ? conv->f32.samples : conv->f64.samples; }
+
+// B becomes the current filter once a call has delivered the fade's last sample, and A the spare: the two buffers trade places
+static void conv_finish_fade(neo_b200_conv* conv)
+{
+    if (!conv->fading || conv_position(conv) < conv->fade_end) { return; }
+    if (conv->cfg.dtype == NEO_B200_F32) { conv->f32.live_filter().swap(conv->f32.spare_filter); }
+    else { conv->f64.live_filter().swap(conv->f64.spare_filter); }
+    conv->fading = false;
+    conv->staged = false;
+}
+
+int neo_b200_conv_crossfade(neo_b200_conv* conv, size_t delay, size_t fade, size_t* start)
+{
+    if (conv == nullptr) { return fail(NEO_B200_ERR_INVALID, "null argument"); }
+    NEO_TRY(conv_fade_check(conv));
+    if (!conv->staged) { return fail(NEO_B200_ERR_INVALID, "nothing staged: call neo_b200_conv_stage_filter / _stage_impulse first"); }
+    if (conv->cfg.dtype == NEO_B200_F32 ? conv->f32.in_call : conv->f64.in_call) {
+        return fail(NEO_B200_ERR_INVALID, "a forward_range call is in progress: pass final != 0 with its last channel range (or reset) first");
+    }
+    size_t const pos = conv_position(conv);
+    if (delay > SIZE_MAX - pos || fade > SIZE_MAX - pos - delay) {
+        return fail(NEO_B200_ERR_INVALID, "delay %zu + fade %zu overflow the stream position", delay, fade);
+    }
+    conv->fading     = true;
+    conv->fade_start = pos + delay;
+    conv->fade_end   = pos + delay + fade;
+    if (start != nullptr) { *start = conv->fade_start; }
+    conv_finish_fade(conv);  // fade = 0 at the next sample: B is current for the next call
+    return NEO_B200_OK;
 }
 
 // true when the CUDA runtime knows the pointer as page-locked host memory (cudaMallocHost / cudaHostRegister / torch pin_memory)
@@ -1078,6 +1244,16 @@ int conv_process_impl(neo_b200_conv* conv, conv_engine<T>& e, void const* in, vo
     cudaStream_t const s = conv->stream.stream;
     size_t const stride  = blocks * e.m;
     size_t const plane   = conv->cfg.outputs * blocks * size_t(e.m);
+    // a call with samples on both sides of a crossfade's start .. end runs both filters (conv_engine::fade_step); every other call runs
+    // the current filter exactly as it would without a crossfade
+    bool const both = conv->fading && e.samples < conv->fade_end && e.samples + stride > conv->fade_start;
+    conv_fade const fade{e.samples, conv->fade_start, conv->fade_end - conv->fade_start};
+    if (memspace == NEO_B200_DEVICE && both) {
+        NEO_TRY(e.forward_r2c(static_cast<T const*>(in), stride, blocks, 0, conv->cfg.inputs, s));
+        NEO_TRY(e.fade_step(blocks, 0, conv->cfg.outputs, static_cast<T*>(out), stride, fade, s));
+        e.advance(blocks);
+        return NEO_B200_OK;
+    }
     if (memspace == NEO_B200_DEVICE) {
         NEO_TRY(e.forward(static_cast<T const*>(in), stride, blocks, s));
         NEO_TRY(e.inverse(e.acc.template as<cx<T>>(), plane, 1, static_cast<T*>(out), stride, 0, conv->cfg.outputs, blocks, s));
@@ -1106,8 +1282,14 @@ int conv_process_impl(neo_b200_conv* conv, conv_engine<T>& e, void const* in, vo
     }
     if (groups == 1) {
         NEO_CUDA_TRY(cudaMemcpyAsync(din, in, conv->cfg.inputs * stride * sizeof(T), cudaMemcpyHostToDevice, s));
-        NEO_TRY(e.forward(din, stride, blocks, s));
-        NEO_TRY(e.inverse(e.acc.template as<cx<T>>(), plane, 1, dout, stride, 0, chans, blocks, s));
+        if (both) {
+            NEO_TRY(e.forward_r2c(din, stride, blocks, 0, conv->cfg.inputs, s));
+            NEO_TRY(e.fade_step(blocks, 0, chans, dout, stride, fade, s));
+            e.advance(blocks);
+        } else {
+            NEO_TRY(e.forward(din, stride, blocks, s));
+            NEO_TRY(e.inverse(e.acc.template as<cx<T>>(), plane, 1, dout, stride, 0, chans, blocks, s));
+        }
         NEO_CUDA_TRY(cudaMemcpyAsync(out, dout, chans * stride * sizeof(T), cudaMemcpyDeviceToHost, s));
     } else {
         NEO_TRY(conv->ensure_pipeline(groups));
@@ -1150,9 +1332,13 @@ int conv_process_impl(neo_b200_conv* conv, conv_engine<T>& e, void const* in, vo
             NEO_CUDA_TRY(cudaEventRecord(conv->ev_in[g], conv->s_in));
             NEO_CUDA_TRY(cudaStreamWaitEvent(s, conv->ev_in[g], 0));
             NEO_TRY(e.forward_r2c(din + c0 * stride, stride, blocks, c0, n, s));
-            NEO_TRY(e.forward_mac(blocks, c0, n, s));
-            NEO_TRY(e.inverse(e.acc.template as<cx<T>>() + c0 * blocks * size_t(e.m), plane, 1, dout + c0 * stride, stride, c0, n,
-                              blocks, s));
+            if (both) {
+                NEO_TRY(e.fade_step(blocks, c0, n, dout + c0 * stride, stride, fade, s));
+            } else {
+                NEO_TRY(e.forward_mac(blocks, c0, n, s));
+                NEO_TRY(e.inverse(e.acc.template as<cx<T>>() + c0 * blocks * size_t(e.m), plane, 1, dout + c0 * stride, stride, c0, n,
+                                  blocks, s));
+            }
             NEO_CUDA_TRY(cudaEventRecord(conv->ev_done[g], s));
             NEO_CUDA_TRY(cudaStreamWaitEvent(conv->s_out, conv->ev_done[g], 0));
             if (staged && g >= 2) { NEO_TRY(drain(g - 2)); }  // frees pin_out[g & 1] for this group
@@ -1195,8 +1381,20 @@ int neo_b200_conv_process(neo_b200_conv* conv, void const* in, void* out, size_t
     if (in == nullptr || out == nullptr) { return fail(NEO_B200_ERR_INVALID, "null buffer"); }
     if (conv->sharded) { return fail(NEO_B200_ERR_INVALID, "partition-sharded handle: use conv_forward / conv_inverse around the reduction"); }
     if (in == out && conv->cfg.topology != NEO_B200_DIAGONAL) { return fail(NEO_B200_ERR_INVALID, "in-place needs the diagonal topology"); }
-    if (conv->cfg.dtype == NEO_B200_F32) { return conv_process_impl<float>(conv, conv->f32, in, out, blocks, memspace); }
-    return conv_process_impl<double>(conv, conv->f64, in, out, blocks, memspace);
+    NEO_TRY(conv->cfg.dtype == NEO_B200_F32 ? conv_process_impl<float>(conv, conv->f32, in, out, blocks, memspace)
+                                            : conv_process_impl<double>(conv, conv->f64, in, out, blocks, memspace));
+    conv_finish_fade(conv);
+    return NEO_B200_OK;
+}
+
+// the split and windowed forms produce partial spectra or windows: there is no whole output for a crossfade to blend
+static int conv_no_fade(neo_b200_conv* conv, char const* what)
+{
+    if (conv != nullptr && conv->fading) {
+        return fail(NEO_B200_ERR_INVALID, "%s while a crossfade is pending or running: it produces no whole output to blend (use neo_b200_conv_process, "
+                                          "or reset)", what);
+    }
+    return NEO_B200_OK;
 }
 
 extern "C++" template<typename T>
@@ -1215,6 +1413,7 @@ int conv_forward_impl(neo_b200_conv* conv, conv_engine<T>& e, void const* in, si
 
 int neo_b200_conv_forward(neo_b200_conv* conv, void const* in, size_t blocks, int memspace)
 {
+    NEO_TRY(conv_no_fade(conv, "forward"));
     NEO_TRY(conv_check_call(conv, blocks));
     if (in == nullptr) { return fail(NEO_B200_ERR_INVALID, "null buffer"); }
     if (conv->cfg.dtype == NEO_B200_F32) { return conv_forward_impl<float>(conv, conv->f32, in, blocks, memspace); }
@@ -1256,6 +1455,7 @@ int conv_forward_range_impl(neo_b200_conv* conv, conv_engine<T>& e, void const* 
 
 int neo_b200_conv_forward_range(neo_b200_conv* conv, void const* in, size_t blocks, size_t first, size_t count, int final)
 {
+    NEO_TRY(conv_no_fade(conv, "forward_range"));
     NEO_TRY(conv_check_call(conv, blocks, false));
     if (in == nullptr) { return fail(NEO_B200_ERR_INVALID, "null buffer"); }
     if (conv->cfg.topology != NEO_B200_DIAGONAL) { return fail(NEO_B200_ERR_INVALID, "forward_range needs the diagonal topology"); }
@@ -1293,6 +1493,7 @@ int conv_inverse_impl(neo_b200_conv* conv, conv_engine<T>& e, void const* spectr
 
 int neo_b200_conv_inverse(neo_b200_conv* conv, void const* spectra_device, void* out, size_t first, size_t count, size_t blocks, int memspace)
 {
+    NEO_TRY(conv_no_fade(conv, "inverse"));
     NEO_TRY(conv_check_call(conv, blocks, false));
     if (spectra_device == nullptr || out == nullptr) { return fail(NEO_B200_ERR_INVALID, "null buffer"); }
     if (first + count > conv->cfg.outputs) { return fail(NEO_B200_ERR_INVALID, "output range [%zu, %zu) outside the bank", first, first + count); }
@@ -1325,6 +1526,7 @@ int conv_window_impl(neo_b200_conv* conv, conv_engine<T>& e, void const* window,
 
 int neo_b200_conv_process_window(neo_b200_conv* conv, void const* window, void* y, int commit, int memspace)
 {
+    NEO_TRY(conv_no_fade(conv, "process_window"));
     NEO_TRY(conv_check_call(conv, 1));
     if (window == nullptr || y == nullptr) { return fail(NEO_B200_ERR_INVALID, "null buffer"); }
     if (conv->cfg.kind != NEO_B200_UPOLA || conv->cfg.topology != NEO_B200_DIAGONAL || conv->cfg.frame_blocks != 0 || conv->sharded) {
@@ -1798,17 +2000,6 @@ struct lowlat_state
     }
 };
 
-// an engine runs with the spare filter for the lifetime of this guard
-struct lowlat_use_spare
-{
-    device_buffer& a;
-    device_buffer& b;
-    lowlat_use_spare(device_buffer& filter, device_buffer& spare) : a(filter), b(spare) { a.swap(b); }
-    ~lowlat_use_spare() { a.swap(b); }
-    lowlat_use_spare(lowlat_use_spare const&)            = delete;
-    lowlat_use_spare& operator=(lowlat_use_spare const&) = delete;
-};
-
 }  // namespace
 }  // namespace neo_b200
 
@@ -1965,7 +2156,7 @@ int lowlat_segment(neo_b200_lowlat* h, T const* in, size_t in_stride, T* out, si
     size_t const C = h->cfg.channels, B = h->cfg.block, tb = h->block_pos;
     bool const completes = end == B;
     bool const both      = h->fading && tb * B + pos < h->fade_end && tb * B + end > h->fade_start;
-    lowlat_fade const fade{tb * B, h->fade_start, h->fade_end - h->fade_start};
+    conv_fade const fade{tb * B, h->fade_start, h->fade_end - h->fade_start};
 
     // the partial output of level i for block tb comes from its frame tb / T_i - 2; the first segment of the block waits for it
     lowlat_levels<T> lv{}, lvb{};
@@ -2021,7 +2212,7 @@ int lowlat_segment(neo_b200_lowlat* h, T const* in, size_t in_stride, T* out, si
         if (both) {  // one insert, the B side's MAC and inverse transform into fade_y, then the A side's MAC as forward() runs it
             NEO_TRY(e.forward_r2c(blk, blk_stride, 1, 0, C, st));
             {
-                lowlat_use_spare const use_b(e.filter, s.spare_head);
+                use_spare const use_b(e.filter, s.spare_head);
                 NEO_TRY(e.forward_mac(1, 0, C, st));
             }
             NEO_TRY(e.inverse(e.acc_w(), 0, 1, s.fade_y.template as<T>(), B, 0, C, 1, st));
@@ -2045,7 +2236,7 @@ int lowlat_segment(neo_b200_lowlat* h, T const* in, size_t in_stride, T* out, si
         NEO_TRY(check_launch("lowlat_window_kernel"));
         NEO_TRY(e.window_step(s.window.template as<T>(), s.window_y.template as<T>(), false, st));
         if (both) {
-            lowlat_use_spare const use_b(e.filter, s.spare_head);
+            use_spare const use_b(e.filter, s.spare_head);
             NEO_TRY(e.window_step(s.window.template as<T>(), s.fade_y.template as<T>(), false, st));
         }
         dim3 const grid(unsigned((end + 255) / 256), unsigned(C));
@@ -2104,7 +2295,7 @@ int lowlat_segment(neo_b200_lowlat* h, T const* in, size_t in_stride, T* out, si
                 NEO_TRY(e.inverse(e.acc_w(), 0, 1, s.plane[i].template as<T>() + slot, 2 * ti * B, 0, C, ti, ls));
             }
             {
-                lowlat_use_spare const use_b(e.filter2, s.spare_level[i]);
+                use_spare const use_b(e.filter2, s.spare_level[i]);
                 NEO_TRY(e.forward_mac(ti, 0, C, ls));
             }
             NEO_TRY(e.inverse(e.acc_w(), 0, 1, s.plane_b[i].template as<T>() + slot, 2 * ti * B, 0, C, ti, ls));
@@ -2234,11 +2425,11 @@ int lowlat_stage_impl(neo_b200_lowlat* h, void const* H, void const* ir, size_t 
     }
     h->staged = false;
     {
-        lowlat_use_spare const use(s.head.filter, s.spare_head);
+        use_spare const use(s.head.filter, s.spare_head);
         NEO_TRY(ir != nullptr ? s.head.load_impulse(ir, taps, memspace, ss) : s.head.load_filter(H, memspace, ss));
     }
     for (size_t i = 0; i < h->levels; ++i) {
-        lowlat_use_spare const use(s.level[i].filter2, s.spare_level[i]);
+        use_spare const use(s.level[i].filter2, s.spare_level[i]);
         NEO_TRY(ir != nullptr ? s.level[i].load_impulse(ir, taps, memspace, ss) : s.level[i].load_filter(H, memspace, ss));
     }
     NEO_CUDA_TRY(cudaStreamSynchronize(ss));

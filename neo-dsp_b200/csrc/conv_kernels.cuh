@@ -683,6 +683,80 @@ struct conv_c2r_io
     }
 };
 
+// ---- crossfade between two filters (neo_b200_conv_crossfade, neo_b200_lowlat_crossfade): out = y_A before `start`,
+// y_A + g (y_B - y_A) with g = (t - start) / len inside, y_B after. One formula for both convolvers.
+struct conv_fade
+{
+    unsigned long long t0;          // absolute sample index of block position 0 (of the row's first block)
+    unsigned long long start, len;  // the fade covers samples [start, start + len)
+};
+
+template<typename T>
+__device__ __forceinline__ T conv_blend(T ya, T yb, unsigned long long t, conv_fade const& f)
+{
+    if (t < f.start) { return ya; }
+    if (t - f.start >= f.len) { return yb; }
+    T const g = T(double(t - f.start) / double(f.len));
+    return ya + g * (yb - ya);
+}
+
+// the A side of a bank call inside a crossfade: conv_c2r_io's overlap-save store (no overlap-add: its tail depends on the filter), each
+// kept sample blended with the B side's output at the same place of `yb` ([count][out_stride] reals, laid out as `out`). Sample j of
+// block tau of a row is absolute sample fade.t0 + tau B + j.
+template<typename T, int LOGM>
+struct conv_c2r_fade_io
+{
+    using C = cx<T>;
+    C const* acc;  // [count][blocks][B]
+    int blocks;
+    T* out;
+    size_t out_stride;
+    T scale;
+    T const* yb;
+    conv_fade fade;
+    // the wide c2r at 6 resident CTAs (80 registers) would spill the blend; a fade call runs it at 5 (96), same arithmetic
+    static constexpr int wide_max_minb = 5;
+
+    struct row_state
+    {
+        C const* src;
+        C* dst;
+        C const* yb;
+        unsigned long long t;  // absolute index of the block's first sample
+    };
+    __device__ __forceinline__ row_state open(size_t b) const
+    {
+        constexpr size_t B = size_t(1) << LOGM;
+        size_t const ch    = b / blocks;
+        size_t const tau   = b - ch * blocks;
+        size_t const off   = ch * out_stride + tau * B;
+        return {acc + (ch * blocks + tau) * B, reinterpret_cast<C*>(out + off), reinterpret_cast<C const*>(yb + off), fade.t0 + tau * B};
+    }
+    __device__ __forceinline__ C load(row_state const& r, int k) const { return r.src[k]; }
+    __device__ __forceinline__ C load_edges(row_state const& r) const { return load(r, 0); }
+    __device__ __forceinline__ void store(row_state const& r, int j, C z) const
+    {
+        constexpr int H = (1 << LOGM) / 2;
+        if (j >= H) {
+            C const b                  = r.yb[j - H];
+            unsigned long long const t = r.t + 2ULL * unsigned(j - H);
+            r.dst[j - H]               = mk<T>(conv_blend(z.x * scale, b.x, t, fade), conv_blend(z.y * scale, b.y, t + 1, fade));
+        }
+    }
+    // the wide kernel's 128-bit stores; the four samples of a float4 are blended one by one
+    template<bool HI>
+    __device__ __forceinline__ void store_pair(row_state const& r, int j, C z0, C z1) const
+    {
+        static_assert(sizeof(T) == 4, "float rows");
+        if constexpr (HI) {
+            float4 const b             = *reinterpret_cast<float4 const*>(r.yb + j);
+            unsigned long long const t = r.t + 2ULL * unsigned(j);
+            *reinterpret_cast<float4*>(r.dst + j) = make_float4(conv_blend(z0.x * scale, b.x, t, fade), conv_blend(z0.y * scale, b.y, t + 1, fade),
+                                                                conv_blend(z1.x * scale, b.z, t + 2, fade), conv_blend(z1.y * scale, b.w, t + 3, fade));
+        }
+    }
+};
+
 // ---- inverse side of a partition-sharded bank whose shards sit in peer-mapped memory: the cross-device reduction of the partial
 // spectra is fused into the loads of the c2r kernel. src[j] is the partial-spectra buffer of partition shard j (this device's own
 // buffer or a peer's, read over NVLink through the mapped pointer), all with the same [count][blocks][B] layout; they are summed in

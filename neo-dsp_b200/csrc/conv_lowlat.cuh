@@ -39,22 +39,6 @@ struct lowlat_levels
     size_t stride[k_lowlat_max_levels];    // reals between channels of a plane
 };
 
-// a crossfade (neo_b200_lowlat_crossfade): out = y_A before `start`, y_A + g (y_B - y_A) with g = (t - start) / len inside, y_B after
-struct lowlat_fade
-{
-    unsigned long long t0;          // absolute sample index of block position 0
-    unsigned long long start, len;  // the fade covers samples [start, start + len)
-};
-
-template<typename T>
-__device__ __forceinline__ T lowlat_blend(T ya, T yb, unsigned long long t, lowlat_fade const& f)
-{
-    if (t < f.start) { return ya; }
-    if (t - f.start >= f.len) { return yb; }
-    T const g = T(double(t - f.start) / double(f.len));
-    return ya + g * (yb - ya);
-}
-
 template<typename T>
 struct lowlat_head_args
 {
@@ -76,7 +60,7 @@ struct lowlat_head_args
     int vec;       // pos == 0, end == B and every row of `in` / `out` starts on a complex pair: 8- / 16-byte accesses
     int commit;    // 0: outputs only (the B side of a crossfade): no half-window, delay-line, input-ring or pending writes
     T const* fade_y;  // [C][B] the B side's outputs of this segment by block position, blended in by `fade`; nullptr: no crossfade
-    lowlat_fade fade;
+    conv_fade fade;
 };
 
 // sample j of the new half-window of a segment: pending, then `in`, then zeros
@@ -273,8 +257,8 @@ __global__ void __launch_bounds__(fft_cfg<T, LOGM>::THREADS, lowlat_min_ctas<T, 
             }
             if (XF && a.fade_y != nullptr) {
                 C const yb = reinterpret_cast<C const*>(a.fade_y + row * M)[j];
-                y.x        = lowlat_blend(y.x, yb.x, a.fade.t0 + 2 * j, a.fade);
-                y.y        = lowlat_blend(y.y, yb.y, a.fade.t0 + 2 * j + 1, a.fade);
+                y.x        = conv_blend(y.x, yb.x, a.fade.t0 + 2 * j, a.fade);
+                y.y        = conv_blend(y.y, yb.y, a.fade.t0 + 2 * j + 1, a.fade);
             }
             if (a.vec) { dst[j] = y; }
             else {
@@ -304,7 +288,7 @@ template<typename T>
 __global__ void __launch_bounds__(256) lowlat_combine_kernel(T const* __restrict__ head, size_t head_stride, int first, int end, T const* in,
                                                              size_t in_stride, T* out, size_t out_stride, T* __restrict__ in_ring,
                                                              size_t ring_stride, lowlat_levels<T> levels, T const* __restrict__ head_b,
-                                                             lowlat_levels<T> levels_b, lowlat_fade fade)
+                                                             lowlat_levels<T> levels_b, conv_fade fade)
 {
     size_t const ch = blockIdx.y;
     int const i     = blockIdx.x * blockDim.x + threadIdx.x;
@@ -312,7 +296,7 @@ __global__ void __launch_bounds__(256) lowlat_combine_kernel(T const* __restrict
     if (in_ring != nullptr) { in_ring[ch * ring_stride + i] = in[ch * in_stride + i]; }  // read before the store below: in == out is allowed
     if (i < first) { return; }
     T y = lowlat_sum(head, head_stride, levels, ch, i);
-    if (head_b != nullptr) { y = lowlat_blend(y, lowlat_sum(head_b, head_stride, levels_b, ch, i), fade.t0 + unsigned(i), fade); }
+    if (head_b != nullptr) { y = conv_blend(y, lowlat_sum(head_b, head_stride, levels_b, ch, i), fade.t0 + unsigned(i), fade); }
     out[ch * out_stride + (i - first)] = y;
 }
 

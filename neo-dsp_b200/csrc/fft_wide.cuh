@@ -23,6 +23,7 @@
 
 #include "fft_kernels.cuh"
 
+#include <algorithm>
 #include <type_traits>
 
 namespace neo_b200 {
@@ -1116,6 +1117,19 @@ int launch_r2c_wide_io(IO const& io, float2 const* ta, float2 const* tb, float2 
     return go(r2c_wide_io_kernel<LOGM, LOGR1, LOGR2, G, IO, 4>);
 }
 
+// the most resident CTAs a c2r policy may be compiled for: IO::wide_max_minb where a policy sets it (a policy whose store needs more
+// registers than 80 without spilling), else 6; a larger request runs at that bound
+template<class IO, class = void>
+struct wide_max_minb
+{
+    static constexpr int value = 6;
+};
+template<class IO>
+struct wide_max_minb<IO, std::void_t<decltype(IO::wide_max_minb)>>
+{
+    static constexpr int value = IO::wide_max_minb;
+};
+
 template<int LOGM, int LOGR1, int LOGR2, class IO>
 int launch_c2r_wide_io(IO const& io, float2 const* ta, float2 const* tb, float2 const* rtw, size_t batch, cudaStream_t stream, int minb = 4)
 {
@@ -1127,8 +1141,11 @@ int launch_c2r_wide_io(IO const& io, float2 const* ta, float2 const* tb, float2 
         kernel<<<unsigned((batch + G - 1) / G), 32 * G, G * cfg::SMEM, stream>>>(io, ta, tb, rtw, batch);
         return check_launch("c2r_wide_io_kernel");
     };
+    if constexpr (wide_max_minb<IO>::value < 6) { minb = std::min(minb, wide_max_minb<IO>::value); }
     if (minb == 5) { return go(c2r_wide_io_kernel<LOGM, LOGR1, LOGR2, G, IO, 5>); }
-    if (minb == 6) { return go(c2r_wide_io_kernel<LOGM, LOGR1, LOGR2, G, IO, 6>); }
+    if constexpr (wide_max_minb<IO>::value >= 6) {
+        if (minb == 6) { return go(c2r_wide_io_kernel<LOGM, LOGR1, LOGR2, G, IO, 6>); }
+    }
     return go(c2r_wide_io_kernel<LOGM, LOGR1, LOGR2, G, IO, 4>);
 }
 
