@@ -52,15 +52,25 @@ __global__ void digitrev_perm_kernel(unsigned radix, unsigned digits, unsigned s
 
 namespace {
 
-// an engine runs with the spare filter for the lifetime of this guard (staging and the B side of a crossfade)
-struct use_spare
+// a crossfade's window (neo_b200_conv_* and neo_b200_lowlat_*): the engines' spare filters hold B once `staged`; while `fading`,
+// samples [start, end) blend A into B, and B becomes the current filter once every sample before `end` has been delivered
+struct fade_window
 {
-    device_buffer& a;
-    device_buffer& b;
-    use_spare(device_buffer& filter, device_buffer& spare) : a(filter), b(spare) { a.swap(b); }
-    ~use_spare() { a.swap(b); }
-    use_spare(use_spare const&)            = delete;
-    use_spare& operator=(use_spare const&) = delete;
+    bool staged{false}, fading{false};
+    size_t start{0}, end{0};
+
+    // a call covering samples [lo, hi) runs both filters; every other call runs the current filter exactly as without a crossfade
+    bool overlaps(size_t lo, size_t hi) const { return fading && lo < end && hi > start; }
+    bool over(size_t pos) const { return fading && pos >= end; }
+    void cancel() { staged = fading = false; }
+    conv_fade from(size_t t0) const { return {t0, start, end - start}; }  // for a call whose first sample is t0
+    // true once, when a call has delivered the fade's last sample: the caller trades the current and the spare buffers
+    bool finish(size_t pos)
+    {
+        if (!over(pos)) { return false; }
+        cancel();
+        return true;
+    }
 };
 
 template<typename T>
@@ -106,10 +116,24 @@ struct conv_engine
     void* acc_r() const { return in_call ? static_cast<void*>(acc_w()) : (acc_last != 0 ? acc_alt : acc).ptr; }
     int prev_flip{0};  // prev[prev_flip] holds the last block of the previous call
     size_t samples{0};  // samples per channel the delay line has advanced by since clear_state
-    // crossfade (neo_b200_conv_stage_* / _crossfade), allocated by the first stage: the spare filter set (`filter`'s twin in the direct
-    // form, `filter2`'s in frame mode) and the B side's outputs of a call inside the fade, [outputs][max_blocks B] reals
+    // crossfade (neo_b200_conv_stage_* / _crossfade, neo_b200_lowlat_stage_*), allocated by the first stage: the spare filter set
+    // (`filter`'s twin in the direct form, `filter2`'s in frame mode); a bank's stage also allocates the B side's outputs of a call
+    // inside the fade, [outputs][max_blocks B] reals
     device_buffer spare_filter, fade_y;
     device_buffer& live_filter() { return frame > 0 ? filter2 : filter; }
+    // the staged filter becomes the current one and the current one the spare
+    void swap_spare() { live_filter().swap(spare_filter); }
+
+    // the engine runs with the spare filter for the lifetime of this guard when `on` (staging and the B side of a crossfade)
+    struct use_spare
+    {
+        conv_engine& e;
+        bool on;
+        use_spare(conv_engine& engine, bool spare) : e(engine), on(spare) { if (on) { e.swap_spare(); } }
+        ~use_spare() { if (on) { e.swap_spare(); } }
+        use_spare(use_spare const&)            = delete;
+        use_spare& operator=(use_spare const&) = delete;
+    };
 
     // second partition level along block time (conv_frame.cuh). frame == 0: direct form. In frame mode `fdl` is the two-frame
     // level-1 spectra buffer x1 (2T plain rows of B per channel, not tiled) and `filter` only lives while a filter is prepared.
@@ -339,9 +363,10 @@ struct conv_engine
     // `sparse_filter::filter(partitions, sparsity)` (sparse_filter.hpp:25-28) for every channel of a diagonal bank: the CSR matrices
     // exactly as neo::csr_matrix builds them (csr_matrix.hpp:64-98; rows = partitions, columns = the B+1 bins). Filter f owns entries
     // [filter_base[f], filter_base[f+1]) of values / cols; row_ptr[f * (P+1) + p] is relative to filter_base[f]. Host memory.
-    int set_filter_csr(cx<T> const* values, std::uint64_t const* cols, std::uint64_t const* row_ptr, std::uint64_t const* filter_base,
+    int set_filter_csr(void const* values_host, std::uint64_t const* cols, std::uint64_t const* row_ptr, std::uint64_t const* filter_base,
                        cudaStream_t stream)
     {
+        cx<T> const* const values = static_cast<cx<T> const*>(values_host);
         if (cfg.topology != NEO_B200_DIAGONAL || frame > 0 || cfg.partition_begin != 0 || cfg.partition_end != cfg.partitions) {
             return fail(NEO_B200_ERR_UNSUPPORTED, "sparse filters: diagonal topology, direct form (frame_blocks = 0), unsharded partitions");
         }
@@ -516,13 +541,12 @@ struct conv_engine
         return build_filter(stream);
     }
 
-    // builds H / ir into the spare filter set through load_filter / load_impulse (neo_b200_conv_stage_*): the current filter, the delay
-    // line, the half-window and the ring position stay as they are. The spare set and fade_y are allocated once and reused.
+    // builds H / ir into the spare filter set through load_filter / load_impulse: the current filter, the delay line, the half-window
+    // and the ring position stay as they are. The spare set is allocated once and reused.
     int stage(void const* h, void const* ir, size_t taps, int memspace, cudaStream_t stream)
     {
         NEO_TRY(spare_filter.reserve(live_filter().bytes));
-        NEO_TRY(fade_y.reserve(cfg.outputs * cfg.max_blocks * size_t(m) * sizeof(T)));
-        use_spare const use(live_filter(), spare_filter);
+        use_spare const use(*this, true);
         return ir != nullptr ? load_impulse(ir, taps, memspace, stream) : load_filter(h, memspace, stream);
     }
 
@@ -583,8 +607,9 @@ struct conv_engine
 
     // one chunk of neo::convolution::overlap_add_convolver (overlap_add_convolver.hpp:91-115): transform the windows [channels][2B] as
     // they stand into the newest delay-line row, MAC over all partitions, inverse transform, scale by 1/2B -> y [channels][2B].
-    // commit: the chunk completed a block, the delay line advances (:122-131). Overlap-add, direct form.
-    int window_step(T const* window, T* y, bool commit, cudaStream_t stream)
+    // commit: the chunk completed a block, the delay line advances (:122-131). Overlap-add, direct form. `spare`: the MAC runs the spare
+    // filter (the B side of a crossfade; its step stores the same delay-line row again)
+    int window_step(T const* window, T* y, bool commit, bool spare, cudaStream_t stream)
     {
         int status = NEO_B200_ERR_UNSUPPORTED;
         NEO_DISPATCH_LOGM(T, logb, {
@@ -606,7 +631,7 @@ struct conv_engine
             }
         });
         if (status != NEO_B200_OK) { return status; }
-        NEO_TRY(forward_mac(1, 0, cfg.outputs, stream));
+        NEO_TRY(mac(spare, 1, 0, cfg.outputs, stream));
         NEO_DISPATCH_LOGM(T, logb, {
             if constexpr (LOGM >= 1 && LOGM <= max_cta_logm<T>()) {
                 conv_c2r_io<T, LOGM> io{acc_w(), 1, y, 2 * size_t(m), T(1) / T(2 * m), 1};
@@ -754,6 +779,25 @@ struct conv_engine
         return mark_end(1, stream);
     }
 
+    // forward_mac under the current filter, or under the spare one
+    int mac(bool spare, size_t blocks, size_t out0, size_t nout, cudaStream_t stream)
+    {
+        use_spare const use(*this, spare);
+        return forward_mac(blocks, out0, nout, stream);
+    }
+
+    // outputs [out0, out0 + nout) of the `blocks` blocks just inserted, into out [nout][out_stride]: the MAC under the current filter,
+    // or with `spare` under the staged filter B, then the inverse transform (the optional arguments as inverse's). The two sides of a
+    // crossfade run this once each between one insert and one advance: the second MAC rewrites what the first wrote besides the spectra
+    // (frame mode's ring slot and Nyquist accumulators) with the same bits.
+    int mac_inverse(bool spare, size_t blocks, size_t out0, size_t nout, T* out, size_t out_stride, cudaStream_t stream,
+                    T const* wide_as = nullptr, T const* yb = nullptr, conv_fade const* fade = nullptr)
+    {
+        NEO_TRY(mac(spare, blocks, out0, nout, stream));
+        cx<T> const* const spectra = acc_w() + out0 * blocks * size_t(m);
+        return inverse(&spectra, 1, out, out_stride, out0, nout, blocks, stream, wide_as, yb, fade);
+    }
+
     // the ring position moves once per call, after every channel group has been inserted
     void advance(size_t blocks)
     {
@@ -838,70 +882,29 @@ struct conv_engine
         return check_launch("fdl_mac_tma_kernel");
     }
 
-    // c2r + scale + overlap handling of spectra [count][blocks][B] (S partial planes `plane` apart) into out [count][out_stride]
-    int inverse(cx<T> const* spectra, size_t /*plane*/, int /*nsplits*/, T* out, size_t out_stride, size_t first, size_t count,
-                size_t blocks, cudaStream_t stream)
+    // c2r + scale + overlap handling of spectra [count][blocks][B] into out [count][out_stride]: the sum of `nsrc` spectra buffers
+    // (partition shards of a multi-device bank; peer-mapped pointers are read over NVLink inside the c2r kernel: reduction and inverse
+    // transform are one pass). The c2r kernel (wide or cta_fft) is the one wide_rows_ok allows for the destination, or for `wide_as`:
+    // the B side of a bank's crossfade takes the kernel its A side takes for the caller's `out`, so its samples are the bits a handle
+    // running B would store there. With `fade` (one buffer, overlap-save), each kept sample is blended with the same place of `yb`
+    // (conv_c2r_fade_io).
+    int inverse(cx<T> const* const* srcs, int nsrc, T* out, size_t out_stride, size_t first, size_t count, size_t blocks, cudaStream_t stream,
+                T const* wide_as = nullptr, T const* yb = nullptr, conv_fade const* fade = nullptr)
     {
-        cx<T> const* one[1] = {spectra};
-        return inverse_sum(one, 1, out, out_stride, first, count, blocks, stream);
-    }
-
-    // overlap-save c2r of spectra [count][blocks][B] into out [count][out_stride] with the kernel the caller picks (wide or cta_fft);
-    // with `fade`, each kept sample is blended with the same place of yb (conv_c2r_fade_io)
-    int inverse_rows(cx<T> const* spectra, T* out, size_t out_stride, size_t count, size_t blocks, bool wide, T const* yb, conv_fade const* fade,
-                     cudaStream_t stream)
-    {
-        int status = NEO_B200_ERR_UNSUPPORTED;
-        NEO_TRY(mark_begin(2, stream));
-        NEO_DISPATCH_LOGM(T, logb, {
-            if constexpr (LOGM >= 1 && LOGM <= max_cta_logm<T>()) {
-                if (fade == nullptr) {
-                    conv_c2r_io<T, LOGM> io{spectra, int(blocks), out, out_stride, T(1) / T(2 * m), 0};
-                    status = run_c2r<LOGM>(io, wide, count * blocks, stream);
-                } else {
-                    conv_c2r_fade_io<T, LOGM> io{spectra, int(blocks), out, out_stride, T(1) / T(2 * m), yb, *fade};
-                    status = run_c2r<LOGM>(io, wide, count * blocks, stream);
-                }
-            }
-        });
-        if (status != NEO_B200_OK) { return status; }
-        return mark_end(2, stream);
-    }
-
-    // outputs [out0, out0 + nout) of a call with samples on both sides of a crossfade's start .. end, after forward_r2c: the MAC under
-    // the spare filter B and its inverse transform into fade_y, then the MAC under A and its inverse transform blended with fade_y at the
-    // store. The second MAC rewrites what the first wrote besides the spectra (frame mode's ring slot and Nyquist accumulators) with the
-    // same bits. The B side takes the c2r kernel the A side takes for `out` (wide or cta_fft: wide_rows_ok looks at the caller's
-    // pointer), so its samples are the bits a handle running B would store there.
-    int fade_step(size_t blocks, size_t out0, size_t nout, T* out, size_t out_stride, conv_fade const& fade, cudaStream_t stream)
-    {
-        bool const wide            = wide_rows_ok(out, out_stride);
-        cx<T> const* const spectra = acc.template as<cx<T>>() + out0 * blocks * size_t(m);
-        T* const yb                = fade_y.template as<T>() + out0 * out_stride;
-        {
-            use_spare const use_b(live_filter(), spare_filter);
-            NEO_TRY(forward_mac(blocks, out0, nout, stream));
-        }
-        NEO_TRY(inverse_rows(spectra, yb, out_stride, nout, blocks, wide, nullptr, nullptr, stream));
-        NEO_TRY(forward_mac(blocks, out0, nout, stream));
-        return inverse_rows(spectra, out, out_stride, nout, blocks, wide, yb, &fade, stream);
-    }
-
-    // the same for the sum of `nsrc` partial spectra buffers (partition shards of a multi-device bank; peer-mapped pointers are
-    // read over NVLink inside the c2r kernel: reduction and inverse transform are one pass)
-    int inverse_sum(cx<T> const* const* srcs, int nsrc, T* out, size_t out_stride, size_t first, size_t count, size_t blocks,
-                    cudaStream_t stream)
-    {
-        bool const ola = cfg.kind == NEO_B200_UPOLA;
-        T* const dst   = ola ? ola_y.template as<T>() : out;
-        int status     = NEO_B200_ERR_UNSUPPORTED;
+        bool const ola  = cfg.kind == NEO_B200_UPOLA;
+        T* const dst    = ola ? ola_y.template as<T>() : out;
+        bool const wide = wide_rows_ok(wide_as != nullptr ? wide_as : dst, ola ? 4 : out_stride);
+        int status      = NEO_B200_ERR_UNSUPPORTED;
         if (nsrc < 1 || nsrc > k_bank_max_shards) { return fail(NEO_B200_ERR_INVALID, "bad number of partial spectra %d", nsrc); }
         NEO_TRY(mark_begin(2, stream));
         NEO_DISPATCH_LOGM(T, logb, {
             if constexpr (LOGM >= 1 && LOGM <= max_cta_logm<T>()) {
-                if (nsrc == 1) {
+                if (fade != nullptr) {
+                    conv_c2r_fade_io<T, LOGM> io{srcs[0], int(blocks), out, out_stride, T(1) / T(2 * m), yb, *fade};
+                    status = run_c2r<LOGM>(io, wide, count * blocks, stream);
+                } else if (nsrc == 1) {
                     conv_c2r_io<T, LOGM> io{srcs[0], int(blocks), dst, out_stride, T(1) / T(2 * m), ola ? 1 : 0};
-                    status = run_c2r<LOGM>(io, wide_rows_ok(dst, ola ? 4 : out_stride), count * blocks, stream);
+                    status = run_c2r<LOGM>(io, wide, count * blocks, stream);
                 } else {
                     auto const run = [&](auto io) {
                         for (int j = 0; j < nsrc; ++j) { io.src[j] = srcs[j]; }
@@ -911,7 +914,7 @@ struct conv_engine
                         io.out_stride  = out_stride;
                         io.scale       = T(1) / T(2 * m);
                         io.overlap_add = ola ? 1 : 0;
-                        return run_c2r<LOGM>(io, wide_rows_ok(dst, ola ? 4 : out_stride), count * blocks, stream);
+                        return run_c2r<LOGM>(io, wide, count * blocks, stream);
                     };
                     status = nsrc == 2 ? run(conv_c2r_sum_io<T, LOGM, 2>{}) : run(conv_c2r_sum_io<T, LOGM, 0>{});
                 }
@@ -968,6 +971,17 @@ int validate(neo_b200_conv_config& c)
     return NEO_B200_OK;
 }
 
+// an impulse response of `taps` for a handle of `partitions` partitions of `block`: set_* needs exactly that many (`exact`), stage_* at
+// most that many (the rest is zero). stft would underflow L-B for L < B (fft/stft.hpp:24).
+int check_taps(size_t taps, size_t block, size_t partitions, bool exact)
+{
+    if (taps < block) { return fail(NEO_B200_ERR_INVALID, "impulse response shorter than one block"); }
+    size_t const n = neo_b200_num_partitions(taps, block);
+    if (exact && n != partitions) { return fail(NEO_B200_ERR_INVALID, "taps=%zu gives %zu partitions, handle was created for %zu", taps, n, partitions); }
+    if (n > partitions) { return fail(NEO_B200_ERR_INVALID, "taps=%zu gives %zu partitions, the handle holds %zu", taps, n, partitions); }
+    return NEO_B200_OK;
+}
+
 }  // namespace
 }  // namespace neo_b200
 
@@ -990,10 +1004,7 @@ struct neo_b200_conv
     // speed and the copies overlap the kernels whatever memory the caller hands over
     pinned_buffer pin_in[2], pin_out[2];
     cudaEvent_t ev_h2d[2]{}, ev_d2h[2]{};
-    // crossfade (neo_b200_conv_stage_* / _crossfade): the engine's spare filter holds B once `staged`; while `fading`, samples
-    // [fade_start, fade_end) blend A into B, and B becomes the current filter once a call has delivered sample fade_end - 1
-    bool staged{false}, fading{false};
-    size_t fade_start{0}, fade_end{0};
+    fade_window fade;  // neo_b200_conv_stage_* / _crossfade
 
     int ensure_pipeline(size_t groups)
     {
@@ -1030,9 +1041,15 @@ struct neo_b200_conv
     }
 };
 
-#include "conv_bank.cuh"
+// f(the handle's engine): conv_engine<float> or conv_engine<double> by the configured dtype
+template<typename Conv, typename F>
+decltype(auto) with_engine(Conv* conv, F&& f)
+{
+    if (conv->cfg.dtype == NEO_B200_F32) { return f(conv->f32); }
+    return f(conv->f64);
+}
 
-#define NEO_CONV_ENGINE(conv, CALL) ((conv)->cfg.dtype == NEO_B200_F32 ? (conv)->f32.CALL : (conv)->f64.CALL)
+#include "conv_bank.cuh"
 
 extern "C" {
 
@@ -1053,7 +1070,7 @@ int neo_b200_conv_create(neo_b200_conv** conv, neo_b200_conv_config const* confi
     p->sharded = !(c.partition_begin == 0 && c.partition_end == c.partitions);
     NEO_CUDA_TRY(cudaGetDevice(&p->device));
     NEO_TRY(p->stream.create());
-    NEO_TRY(NEO_CONV_ENGINE(p, init(c, p->stream.stream)));
+    NEO_TRY(with_engine(p.get(), [&](auto& e) { return e.init(c, p->stream.stream); }));
     NEO_CUDA_TRY(cudaStreamSynchronize(p->stream.stream));
     *conv = p.release();
     return NEO_B200_OK;
@@ -1070,8 +1087,8 @@ int neo_b200_conv_set_filter(neo_b200_conv* conv, void const* H, int memspace)
 {
     if (conv == nullptr || H == nullptr) { return fail(NEO_B200_ERR_INVALID, "null argument"); }
     NEO_CUDA_TRY(cudaSetDevice(conv->device));
-    conv->staged = conv->fading = false;
-    NEO_TRY(NEO_CONV_ENGINE(conv, set_filter(H, memspace, conv->stream.stream)));
+    conv->fade.cancel();
+    NEO_TRY(with_engine(conv, [&](auto& e) { return e.set_filter(H, memspace, conv->stream.stream); }));
     NEO_CUDA_TRY(cudaStreamSynchronize(conv->stream.stream));
     return NEO_B200_OK;
 }
@@ -1082,12 +1099,8 @@ int neo_b200_conv_set_filter_csr(neo_b200_conv* conv, void const* values, uint64
         return fail(NEO_B200_ERR_INVALID, "null argument");
     }
     NEO_CUDA_TRY(cudaSetDevice(conv->device));
-    conv->staged = conv->fading = false;
-    if (conv->cfg.dtype == NEO_B200_F32) {
-        NEO_TRY(conv->f32.set_filter_csr(static_cast<float2 const*>(values), cols, row_ptr, filter_base, conv->stream.stream));
-    } else {
-        NEO_TRY(conv->f64.set_filter_csr(static_cast<double2 const*>(values), cols, row_ptr, filter_base, conv->stream.stream));
-    }
+    conv->fade.cancel();
+    NEO_TRY(with_engine(conv, [&](auto& e) { return e.set_filter_csr(values, cols, row_ptr, filter_base, conv->stream.stream); }));
     NEO_CUDA_TRY(cudaStreamSynchronize(conv->stream.stream));
     return NEO_B200_OK;
 }
@@ -1095,15 +1108,10 @@ int neo_b200_conv_set_filter_csr(neo_b200_conv* conv, void const* values, uint64
 int neo_b200_conv_set_impulse(neo_b200_conv* conv, void const* ir, size_t taps, int memspace)
 {
     if (conv == nullptr || ir == nullptr) { return fail(NEO_B200_ERR_INVALID, "null argument"); }
-    // stft would underflow L-B for L < B (fft/stft.hpp:24); the frame count must match the configured partitions
-    if (taps < conv->cfg.block) { return fail(NEO_B200_ERR_INVALID, "impulse response shorter than one block"); }
-    if (neo_b200_num_partitions(taps, conv->cfg.block) != conv->cfg.partitions) {
-        return fail(NEO_B200_ERR_INVALID, "taps=%zu gives %zu partitions, handle was created for %zu", taps,
-                    neo_b200_num_partitions(taps, conv->cfg.block), conv->cfg.partitions);
-    }
+    NEO_TRY(check_taps(taps, conv->cfg.block, conv->cfg.partitions, true));
     NEO_CUDA_TRY(cudaSetDevice(conv->device));
-    conv->staged = conv->fading = false;
-    NEO_TRY(NEO_CONV_ENGINE(conv, set_impulse(ir, taps, memspace, conv->stream.stream)));
+    conv->fade.cancel();
+    NEO_TRY(with_engine(conv, [&](auto& e) { return e.set_impulse(ir, taps, memspace, conv->stream.stream); }));
     NEO_CUDA_TRY(cudaStreamSynchronize(conv->stream.stream));
     return NEO_B200_OK;
 }
@@ -1112,8 +1120,8 @@ int neo_b200_conv_reset(neo_b200_conv* conv)
 {
     if (conv == nullptr) { return fail(NEO_B200_ERR_INVALID, "null argument"); }
     NEO_CUDA_TRY(cudaSetDevice(conv->device));
-    conv->staged = conv->fading = false;  // the current filter stays: A while the fade has not ended, B after
-    return NEO_CONV_ENGINE(conv, clear_state(conv->stream.stream));
+    conv->fade.cancel();  // the current filter stays: A while the fade has not ended, B after
+    return with_engine(conv, [&](auto& e) { return e.clear_state(conv->stream.stream); });
 }
 
 // staging and crossfades need a full output to blend and a filter that does not shape the carried state
@@ -1124,83 +1132,72 @@ static int conv_fade_check(neo_b200_conv* conv)
                                               "output has no tail at the fade's start; use an overlap-save (UPOLS) handle");
     }
     if (conv->sharded) { return fail(NEO_B200_ERR_UNSUPPORTED, "crossfade: partition-sharded handles produce partial spectra, not outputs"); }
-    if (conv->cfg.dtype == NEO_B200_F32 ? conv->f32.sparse : conv->f64.sparse) {
+    if (with_engine(conv, [](auto& e) { return e.sparse; })) {
         return fail(NEO_B200_ERR_UNSUPPORTED, "crossfade: the filter came from set_filter_csr; sparse filters have no spare set");
     }
-    if (conv->fading) { return fail(NEO_B200_ERR_INVALID, "a crossfade is pending or running"); }
+    if (conv->fade.fading) { return fail(NEO_B200_ERR_INVALID, "a crossfade is pending or running"); }
     return NEO_B200_OK;
 }
 
-extern "C++" template<typename T>
-int conv_stage_impl(neo_b200_conv* conv, conv_engine<T>& e, void const* H, void const* ir, size_t taps, int memspace)
+// builds H / ir into the engine's spare filter set (and allocates the B side's outputs once) on the handle's stream: behind every
+// enqueued call, which may still read the spare set (the A side of a fade that has just ended)
+static int conv_stage(neo_b200_conv* conv, void const* H, void const* ir, size_t taps, int memspace)
 {
+    if (!with_engine(conv, [](auto& e) { return e.has_filter; })) {
+        return fail(NEO_B200_ERR_INVALID, "no filter set: stage needs a current filter to fade from");
+    }
+    NEO_TRY(conv_fade_check(conv));
+    if (ir != nullptr) { NEO_TRY(check_taps(taps, conv->cfg.block, conv->cfg.partitions, false)); }
+    NEO_CUDA_TRY(cudaSetDevice(conv->device));
     cudaStream_t const s = conv->stream.stream;
-    conv->staged         = false;
-    // on the handle's stream: behind every enqueued call, which may still read the spare set (the A side of a fade that has just ended)
-    NEO_TRY(e.stage(H, ir, taps, memspace, s));
+    conv->fade.staged    = false;
+    NEO_TRY(with_engine(conv, [&](auto& e) {
+        NEO_TRY(e.fade_y.reserve(conv->cfg.outputs * conv->cfg.max_blocks * conv->cfg.block * elem_size(conv->cfg.dtype)));
+        return e.stage(H, ir, taps, memspace, s);
+    }));
     NEO_CUDA_TRY(cudaStreamSynchronize(s));
-    conv->staged = true;
+    conv->fade.staged = true;
     return NEO_B200_OK;
 }
 
 int neo_b200_conv_stage_filter(neo_b200_conv* conv, void const* H, int memspace)
 {
     if (conv == nullptr || H == nullptr) { return fail(NEO_B200_ERR_INVALID, "null argument"); }
-    if (!(conv->cfg.dtype == NEO_B200_F32 ? conv->f32.has_filter : conv->f64.has_filter)) {
-        return fail(NEO_B200_ERR_INVALID, "no filter set: stage needs a current filter to fade from");
-    }
-    NEO_TRY(conv_fade_check(conv));
-    NEO_CUDA_TRY(cudaSetDevice(conv->device));
-    if (conv->cfg.dtype == NEO_B200_F32) { return conv_stage_impl<float>(conv, conv->f32, H, nullptr, 0, memspace); }
-    return conv_stage_impl<double>(conv, conv->f64, H, nullptr, 0, memspace);
+    return conv_stage(conv, H, nullptr, 0, memspace);
 }
 
 int neo_b200_conv_stage_impulse(neo_b200_conv* conv, void const* ir, size_t taps, int memspace)
 {
     if (conv == nullptr || ir == nullptr) { return fail(NEO_B200_ERR_INVALID, "null argument"); }
-    if (!(conv->cfg.dtype == NEO_B200_F32 ? conv->f32.has_filter : conv->f64.has_filter)) {
-        return fail(NEO_B200_ERR_INVALID, "no filter set: stage needs a current filter to fade from");
-    }
-    NEO_TRY(conv_fade_check(conv));
-    if (taps < conv->cfg.block) { return fail(NEO_B200_ERR_INVALID, "impulse response shorter than one block"); }
-    if (neo_b200_num_partitions(taps, conv->cfg.block) > conv->cfg.partitions) {
-        return fail(NEO_B200_ERR_INVALID, "taps=%zu gives %zu partitions, the handle holds %zu", taps, neo_b200_num_partitions(taps, conv->cfg.block),
-                    conv->cfg.partitions);
-    }
-    NEO_CUDA_TRY(cudaSetDevice(conv->device));
-    if (conv->cfg.dtype == NEO_B200_F32) { return conv_stage_impl<float>(conv, conv->f32, nullptr, ir, taps, memspace); }
-    return conv_stage_impl<double>(conv, conv->f64, nullptr, ir, taps, memspace);
+    return conv_stage(conv, nullptr, ir, taps, memspace);
 }
 
 // samples per channel delivered since the last reset / set_filter / set_impulse
-static size_t conv_position(neo_b200_conv const* conv) { return conv->cfg.dtype == NEO_B200_F32 ? conv->f32.samples : conv->f64.samples; }
+static size_t conv_position(neo_b200_conv const* conv) { return with_engine(conv, [](auto& e) { return e.samples; }); }
 
-// B becomes the current filter once a call has delivered the fade's last sample, and A the spare: the two buffers trade places
 static void conv_finish_fade(neo_b200_conv* conv)
 {
-    if (!conv->fading || conv_position(conv) < conv->fade_end) { return; }
-    if (conv->cfg.dtype == NEO_B200_F32) { conv->f32.live_filter().swap(conv->f32.spare_filter); }
-    else { conv->f64.live_filter().swap(conv->f64.spare_filter); }
-    conv->fading = false;
-    conv->staged = false;
+    with_engine(conv, [&](auto& e) {
+        if (conv->fade.finish(e.samples)) { e.swap_spare(); }
+    });
 }
 
 int neo_b200_conv_crossfade(neo_b200_conv* conv, size_t delay, size_t fade, size_t* start)
 {
     if (conv == nullptr) { return fail(NEO_B200_ERR_INVALID, "null argument"); }
     NEO_TRY(conv_fade_check(conv));
-    if (!conv->staged) { return fail(NEO_B200_ERR_INVALID, "nothing staged: call neo_b200_conv_stage_filter / _stage_impulse first"); }
-    if (conv->cfg.dtype == NEO_B200_F32 ? conv->f32.in_call : conv->f64.in_call) {
+    if (!conv->fade.staged) { return fail(NEO_B200_ERR_INVALID, "nothing staged: call neo_b200_conv_stage_filter / _stage_impulse first"); }
+    if (with_engine(conv, [](auto& e) { return e.in_call; })) {
         return fail(NEO_B200_ERR_INVALID, "a forward_range call is in progress: pass final != 0 with its last channel range (or reset) first");
     }
     size_t const pos = conv_position(conv);
     if (delay > SIZE_MAX - pos || fade > SIZE_MAX - pos - delay) {
         return fail(NEO_B200_ERR_INVALID, "delay %zu + fade %zu overflow the stream position", delay, fade);
     }
-    conv->fading     = true;
-    conv->fade_start = pos + delay;
-    conv->fade_end   = pos + delay + fade;
-    if (start != nullptr) { *start = conv->fade_start; }
+    conv->fade.fading = true;
+    conv->fade.start  = pos + delay;
+    conv->fade.end    = pos + delay + fade;
+    if (start != nullptr) { *start = conv->fade.start; }
     conv_finish_fade(conv);  // fade = 0 at the next sample: B is current for the next call
     return NEO_B200_OK;
 }
@@ -1243,20 +1240,21 @@ int conv_process_impl(neo_b200_conv* conv, conv_engine<T>& e, void const* in, vo
 {
     cudaStream_t const s = conv->stream.stream;
     size_t const stride  = blocks * e.m;
-    size_t const plane   = conv->cfg.outputs * blocks * size_t(e.m);
-    // a call with samples on both sides of a crossfade's start .. end runs both filters (conv_engine::fade_step); every other call runs
-    // the current filter exactly as it would without a crossfade
-    bool const both = conv->fading && e.samples < conv->fade_end && e.samples + stride > conv->fade_start;
-    conv_fade const fade{e.samples, conv->fade_start, conv->fade_end - conv->fade_start};
-    if (memspace == NEO_B200_DEVICE && both) {
-        NEO_TRY(e.forward_r2c(static_cast<T const*>(in), stride, blocks, 0, conv->cfg.inputs, s));
-        NEO_TRY(e.fade_step(blocks, 0, conv->cfg.outputs, static_cast<T*>(out), stride, fade, s));
-        e.advance(blocks);
-        return NEO_B200_OK;
-    }
+    bool const both      = conv->fade.overlaps(e.samples, e.samples + stride);
+    conv_fade const fade = conv->fade.from(e.samples);
+    // channels [c0, c0 + n) of rows x -> y: r2c, then the MAC and inverse transform under the current filter, or for a call inside a
+    // crossfade the B side's into fade_y, then the A side's blended with it at the store. One group is the whole bank: the r2c covers
+    // its inputs and the MAC its outputs (matrix topology).
+    auto const step = [&](T const* x, T* y, size_t c0, size_t nin, size_t nout) -> int {
+        NEO_TRY(e.forward_r2c(x, stride, blocks, c0, nin, s));
+        if (!both) { return e.mac_inverse(false, blocks, c0, nout, y, stride, s); }
+        T* const yb = e.fade_y.template as<T>() + c0 * stride;
+        NEO_TRY(e.mac_inverse(true, blocks, c0, nout, yb, stride, s, y));
+        return e.mac_inverse(false, blocks, c0, nout, y, stride, s, nullptr, yb, &fade);
+    };
     if (memspace == NEO_B200_DEVICE) {
-        NEO_TRY(e.forward(static_cast<T const*>(in), stride, blocks, s));
-        NEO_TRY(e.inverse(e.acc.template as<cx<T>>(), plane, 1, static_cast<T*>(out), stride, 0, conv->cfg.outputs, blocks, s));
+        NEO_TRY(step(static_cast<T const*>(in), static_cast<T*>(out), 0, conv->cfg.inputs, conv->cfg.outputs));
+        e.advance(blocks);
         return NEO_B200_OK;
     }
 
@@ -1282,14 +1280,8 @@ int conv_process_impl(neo_b200_conv* conv, conv_engine<T>& e, void const* in, vo
     }
     if (groups == 1) {
         NEO_CUDA_TRY(cudaMemcpyAsync(din, in, conv->cfg.inputs * stride * sizeof(T), cudaMemcpyHostToDevice, s));
-        if (both) {
-            NEO_TRY(e.forward_r2c(din, stride, blocks, 0, conv->cfg.inputs, s));
-            NEO_TRY(e.fade_step(blocks, 0, chans, dout, stride, fade, s));
-            e.advance(blocks);
-        } else {
-            NEO_TRY(e.forward(din, stride, blocks, s));
-            NEO_TRY(e.inverse(e.acc.template as<cx<T>>(), plane, 1, dout, stride, 0, chans, blocks, s));
-        }
+        NEO_TRY(step(din, dout, 0, conv->cfg.inputs, chans));
+        e.advance(blocks);
         NEO_CUDA_TRY(cudaMemcpyAsync(out, dout, chans * stride * sizeof(T), cudaMemcpyDeviceToHost, s));
     } else {
         NEO_TRY(conv->ensure_pipeline(groups));
@@ -1331,14 +1323,7 @@ int conv_process_impl(neo_b200_conv* conv, conv_engine<T>& e, void const* in, vo
             if (staged) { NEO_CUDA_TRY(cudaEventRecord(conv->ev_h2d[g & 1], conv->s_in)); }
             NEO_CUDA_TRY(cudaEventRecord(conv->ev_in[g], conv->s_in));
             NEO_CUDA_TRY(cudaStreamWaitEvent(s, conv->ev_in[g], 0));
-            NEO_TRY(e.forward_r2c(din + c0 * stride, stride, blocks, c0, n, s));
-            if (both) {
-                NEO_TRY(e.fade_step(blocks, c0, n, dout + c0 * stride, stride, fade, s));
-            } else {
-                NEO_TRY(e.forward_mac(blocks, c0, n, s));
-                NEO_TRY(e.inverse(e.acc.template as<cx<T>>() + c0 * blocks * size_t(e.m), plane, 1, dout + c0 * stride, stride, c0, n,
-                                  blocks, s));
-            }
+            NEO_TRY(step(din + c0 * stride, dout + c0 * stride, c0, n, n));
             NEO_CUDA_TRY(cudaEventRecord(conv->ev_done[g], s));
             NEO_CUDA_TRY(cudaStreamWaitEvent(conv->s_out, conv->ev_done[g], 0));
             if (staged && g >= 2) { NEO_TRY(drain(g - 2)); }  // frees pin_out[g & 1] for this group
@@ -1359,10 +1344,8 @@ int conv_process_impl(neo_b200_conv* conv, conv_engine<T>& e, void const* in, vo
 static int conv_check_call(neo_b200_conv* conv, size_t blocks, bool whole_bank = true)
 {
     if (conv == nullptr) { return fail(NEO_B200_ERR_INVALID, "null argument"); }
-    bool const ready = conv->cfg.dtype == NEO_B200_F32 ? conv->f32.has_filter : conv->f64.has_filter;
-    if (!ready) { return fail(NEO_B200_ERR_INVALID, "no filter set"); }
-    bool const in_call = conv->cfg.dtype == NEO_B200_F32 ? conv->f32.in_call : conv->f64.in_call;
-    if (whole_bank && in_call) {
+    if (!with_engine(conv, [](auto& e) { return e.has_filter; })) { return fail(NEO_B200_ERR_INVALID, "no filter set"); }
+    if (whole_bank && with_engine(conv, [](auto& e) { return e.in_call; })) {
         return fail(NEO_B200_ERR_INVALID, "a forward_range call is in progress: pass final != 0 with its last channel range (or reset) first");
     }
     if (blocks == 0 || blocks > conv->cfg.max_blocks) {
@@ -1381,8 +1364,7 @@ int neo_b200_conv_process(neo_b200_conv* conv, void const* in, void* out, size_t
     if (in == nullptr || out == nullptr) { return fail(NEO_B200_ERR_INVALID, "null buffer"); }
     if (conv->sharded) { return fail(NEO_B200_ERR_INVALID, "partition-sharded handle: use conv_forward / conv_inverse around the reduction"); }
     if (in == out && conv->cfg.topology != NEO_B200_DIAGONAL) { return fail(NEO_B200_ERR_INVALID, "in-place needs the diagonal topology"); }
-    NEO_TRY(conv->cfg.dtype == NEO_B200_F32 ? conv_process_impl<float>(conv, conv->f32, in, out, blocks, memspace)
-                                            : conv_process_impl<double>(conv, conv->f64, in, out, blocks, memspace));
+    NEO_TRY(with_engine(conv, [&](auto& e) { return conv_process_impl(conv, e, in, out, blocks, memspace); }));
     conv_finish_fade(conv);
     return NEO_B200_OK;
 }
@@ -1390,7 +1372,7 @@ int neo_b200_conv_process(neo_b200_conv* conv, void const* in, void* out, size_t
 // the split and windowed forms produce partial spectra or windows: there is no whole output for a crossfade to blend
 static int conv_no_fade(neo_b200_conv* conv, char const* what)
 {
-    if (conv != nullptr && conv->fading) {
+    if (conv != nullptr && conv->fade.fading) {
         return fail(NEO_B200_ERR_INVALID, "%s while a crossfade is pending or running: it produces no whole output to blend (use neo_b200_conv_process, "
                                           "or reset)", what);
     }
@@ -1416,8 +1398,7 @@ int neo_b200_conv_forward(neo_b200_conv* conv, void const* in, size_t blocks, in
     NEO_TRY(conv_no_fade(conv, "forward"));
     NEO_TRY(conv_check_call(conv, blocks));
     if (in == nullptr) { return fail(NEO_B200_ERR_INVALID, "null buffer"); }
-    if (conv->cfg.dtype == NEO_B200_F32) { return conv_forward_impl<float>(conv, conv->f32, in, blocks, memspace); }
-    return conv_forward_impl<double>(conv, conv->f64, in, blocks, memspace);
+    return with_engine(conv, [&](auto& e) { return conv_forward_impl(conv, e, in, blocks, memspace); });
 }
 
 extern "C++" template<typename T>
@@ -1460,14 +1441,13 @@ int neo_b200_conv_forward_range(neo_b200_conv* conv, void const* in, size_t bloc
     if (in == nullptr) { return fail(NEO_B200_ERR_INVALID, "null buffer"); }
     if (conv->cfg.topology != NEO_B200_DIAGONAL) { return fail(NEO_B200_ERR_INVALID, "forward_range needs the diagonal topology"); }
     if (count == 0 || first + count > conv->cfg.outputs) { return fail(NEO_B200_ERR_INVALID, "bad channel range"); }
-    if (conv->cfg.dtype == NEO_B200_F32) { return conv_forward_range_impl<float>(conv, conv->f32, in, blocks, first, count, final); }
-    return conv_forward_range_impl<double>(conv, conv->f64, in, blocks, first, count, final);
+    return with_engine(conv, [&](auto& e) { return conv_forward_range_impl(conv, e, in, blocks, first, count, final); });
 }
 
 int neo_b200_conv_spectra(neo_b200_conv* conv, void** device_ptr, size_t* bytes_per_output_block)
 {
     if (conv == nullptr || device_ptr == nullptr) { return fail(NEO_B200_ERR_INVALID, "null argument"); }
-    *device_ptr = conv->cfg.dtype == NEO_B200_F32 ? conv->f32.acc_r() : conv->f64.acc_r();
+    *device_ptr = with_engine(conv, [](auto& e) { return e.acc_r(); });
     if (bytes_per_output_block != nullptr) { *bytes_per_output_block = conv->cfg.block * 2 * elem_size(conv->cfg.dtype); }
     return NEO_B200_OK;
 }
@@ -1483,7 +1463,8 @@ int conv_inverse_impl(neo_b200_conv* conv, conv_engine<T>& e, void const* spectr
         NEO_TRY(e.stage_out.reserve(count * stride * sizeof(T)));
         dout = e.stage_out.template as<T>();
     }
-    NEO_TRY(e.inverse(static_cast<cx<T> const*>(spectra), 0, 1, dout, stride, first, count, blocks, s));
+    cx<T> const* const src = static_cast<cx<T> const*>(spectra);
+    NEO_TRY(e.inverse(&src, 1, dout, stride, first, count, blocks, s));
     if (memspace == NEO_B200_HOST) {
         NEO_CUDA_TRY(cudaMemcpyAsync(out, dout, count * stride * sizeof(T), cudaMemcpyDeviceToHost, s));
         NEO_CUDA_TRY(cudaStreamSynchronize(s));
@@ -1498,8 +1479,7 @@ int neo_b200_conv_inverse(neo_b200_conv* conv, void const* spectra_device, void*
     if (spectra_device == nullptr || out == nullptr) { return fail(NEO_B200_ERR_INVALID, "null buffer"); }
     if (first + count > conv->cfg.outputs) { return fail(NEO_B200_ERR_INVALID, "output range [%zu, %zu) outside the bank", first, first + count); }
     if (count == 0) { return NEO_B200_OK; }
-    if (conv->cfg.dtype == NEO_B200_F32) { return conv_inverse_impl<float>(conv, conv->f32, spectra_device, out, first, count, blocks, memspace); }
-    return conv_inverse_impl<double>(conv, conv->f64, spectra_device, out, first, count, blocks, memspace);
+    return with_engine(conv, [&](auto& e) { return conv_inverse_impl(conv, e, spectra_device, out, first, count, blocks, memspace); });
 }
 
 extern "C++" template<typename T>
@@ -1516,7 +1496,7 @@ int conv_window_impl(neo_b200_conv* conv, conv_engine<T>& e, void const* window,
         win = e.stage_in.template as<T>();
         out = e.stage_out.template as<T>();
     }
-    NEO_TRY(e.window_step(win, out, commit != 0, s));
+    NEO_TRY(e.window_step(win, out, commit != 0, false, s));
     if (memspace == NEO_B200_HOST) {
         NEO_CUDA_TRY(cudaMemcpyAsync(y, out, bytes, cudaMemcpyDeviceToHost, s));
         NEO_CUDA_TRY(cudaStreamSynchronize(s));
@@ -1532,8 +1512,7 @@ int neo_b200_conv_process_window(neo_b200_conv* conv, void const* window, void* 
     if (conv->cfg.kind != NEO_B200_UPOLA || conv->cfg.topology != NEO_B200_DIAGONAL || conv->cfg.frame_blocks != 0 || conv->sharded) {
         return fail(NEO_B200_ERR_INVALID, "process_window needs an unsharded overlap-add diagonal bank in the direct form");
     }
-    if (conv->cfg.dtype == NEO_B200_F32) { return conv_window_impl<float>(conv, conv->f32, window, y, commit, memspace); }
-    return conv_window_impl<double>(conv, conv->f64, window, y, commit, memspace);
+    return with_engine(conv, [&](auto& e) { return conv_window_impl(conv, e, window, y, commit, memspace); });
 }
 
 int neo_b200_conv_tail(neo_b200_conv* conv, void* tail, int memspace)
@@ -1541,7 +1520,7 @@ int neo_b200_conv_tail(neo_b200_conv* conv, void* tail, int memspace)
     if (conv == nullptr || tail == nullptr) { return fail(NEO_B200_ERR_INVALID, "null argument"); }
     if (conv->cfg.kind != NEO_B200_UPOLA) { return fail(NEO_B200_ERR_INVALID, "only overlap-add handles keep a tail"); }
     NEO_CUDA_TRY(cudaSetDevice(conv->device));
-    device_buffer const& buf = conv->cfg.dtype == NEO_B200_F32 ? conv->f32.tail : conv->f64.tail;
+    device_buffer const& buf = with_engine(conv, [](auto& e) -> device_buffer const& { return e.tail; });
     NEO_CUDA_TRY(cudaMemcpyAsync(tail, buf.ptr, buf.bytes, memspace == NEO_B200_HOST ? cudaMemcpyDeviceToHost : cudaMemcpyDeviceToDevice,
                                  conv->stream.stream));
     NEO_CUDA_TRY(cudaStreamSynchronize(conv->stream.stream));
@@ -1572,13 +1551,13 @@ int neo_b200_conv_profile_enable(neo_b200_conv* conv, int enable)
 int neo_b200_conv_profile_read(neo_b200_conv* conv, double* phase_ms, uint64_t* mac_launches)
 {
     if (conv == nullptr || phase_ms == nullptr || mac_launches == nullptr) { return fail(NEO_B200_ERR_INVALID, "null argument"); }
-    return NEO_CONV_ENGINE(conv, read_profile(phase_ms, mac_launches, conv->stream.stream));
+    return with_engine(conv, [&](auto& e) { return e.read_profile(phase_ms, mac_launches, conv->stream.stream); });
 }
 
 size_t neo_b200_conv_device_bytes(neo_b200_conv const* conv)
 {
     if (conv == nullptr) { return 0; }
-    return conv->cfg.dtype == NEO_B200_F32 ? conv->f32.device_bytes() : conv->f64.device_bytes();
+    return with_engine(conv, [](auto& e) { return e.device_bytes(); });
 }
 
 // ---- filter preparation -------------------------------------------------------------------------------------------------------
@@ -1977,24 +1956,24 @@ struct lowlat_state
     device_buffer head_y, stage_in, stage_out; // unfused head output; HOST staging
     device_buffer pending;                     // [C][B] the current block's samples delivered so far (sample-granular calls)
     device_buffer window, window_y;            // unfused head: [C][2B] a segment's window and its inverse transform
-    // the spare filter set (neo_b200_lowlat_stage_*), allocated by the first stage: the head's filter, each level's filter2, each level's
-    // B-side planes [C][2 T_i][B], and the head's B-side outputs of a segment inside a crossfade ([C][B] fused, [C][2B] unfused)
-    device_buffer spare_head, spare_level[k_lowlat_max_levels], plane_b[k_lowlat_max_levels], fade_y;
+    // crossfade (neo_b200_lowlat_stage_*), allocated by the first stage besides the engines' spare filters: each level's B-side planes
+    // [C][2 T_i][B], and the head's B-side outputs of a segment inside a crossfade ([C][B] fused, [C][2B] unfused)
+    device_buffer plane_b[k_lowlat_max_levels], fade_y;
 
     size_t device_bytes(size_t levels) const
     {
         size_t n = head.device_bytes() + in_ring.bytes + head_y.bytes + stage_in.bytes + stage_out.bytes + pending.bytes + window.bytes
-                 + window_y.bytes + spare_head.bytes + fade_y.bytes;
-        for (size_t i = 0; i < levels; ++i) { n += level[i].device_bytes() + plane[i].bytes + spare_level[i].bytes + plane_b[i].bytes; }
+                 + window_y.bytes + fade_y.bytes;
+        for (size_t i = 0; i < levels; ++i) { n += level[i].device_bytes() + plane[i].bytes + plane_b[i].bytes; }
         return n;
     }
 
     // the staged set becomes the current one, and the current one the spare
     void swap_sets(size_t levels)
     {
-        head.filter.swap(spare_head);
+        head.swap_spare();
         for (size_t i = 0; i < levels; ++i) {
-            level[i].filter2.swap(spare_level[i]);
+            level[i].swap_spare();
             plane[i].swap(plane_b[i]);
         }
     }
@@ -2020,11 +1999,7 @@ struct neo_b200_lowlat
     bool has_filter{false};
     size_t block_pos{0};    // blocks since the last reset
     size_t sample_pos{0};   // samples of block block_pos delivered so far (in the pending buffer); 0 after whole-block calls
-    // crossfade (neo_b200_lowlat_stage_* / _crossfade): the spare set holds B; while `fading`, samples [fade_start, fade_end) blend A into
-    // B and B becomes the current set once every sample before fade_end has been delivered
-    bool staged{false};
-    bool fading{false};
-    size_t fade_start{0}, fade_end{0};
+    fade_window fade;  // neo_b200_lowlat_stage_* / _crossfade
     cudaStream_t stage_stream{nullptr};                // lowest priority: staging runs behind the stream's work
     cudaEvent_t stage_after[k_lowlat_max_levels + 1]{};  // staging waits for the head's stream and each side stream
     lowlat_state<float> f32;
@@ -2061,20 +2036,20 @@ struct neo_b200_lowlat
     }
 };
 
+// f(the handle's state): lowlat_state<float> or lowlat_state<double> by the configured dtype
+template<typename H, typename F>
+decltype(auto) with_state(H* h, F&& f)
+{
+    if (h->cfg.dtype == NEO_B200_F32) { return f(h->f32); }
+    return f(h->f64);
+}
+
 namespace neo_b200 {
 namespace {
 
 template<typename T>
-lowlat_state<T>& lowlat_of(neo_b200_lowlat* h);
-template<>
-lowlat_state<float>& lowlat_of<float>(neo_b200_lowlat* h) { return h->f32; }
-template<>
-lowlat_state<double>& lowlat_of<double>(neo_b200_lowlat* h) { return h->f64; }
-
-template<typename T>
-int lowlat_init(neo_b200_lowlat* h)
+int lowlat_init(neo_b200_lowlat* h, lowlat_state<T>& s)
 {
-    lowlat_state<T>& s   = lowlat_of<T>(h);
     cudaStream_t const st = h->stream.stream;
     size_t const C = h->cfg.channels, B = h->cfg.block;
     neo_b200_conv_config hc{NEO_B200_UPOLS, h->cfg.dtype, NEO_B200_DIAGONAL, C, C, B, h->cfg.partitions, 1, 0, h->ranges[0][1], 0, 0};
@@ -2099,9 +2074,8 @@ int lowlat_init(neo_b200_lowlat* h)
 
 // zero every piece of stream state and drop a staged set or a pending / running crossfade; the caller has synchronised the side streams
 template<typename T>
-int lowlat_clear(neo_b200_lowlat* h)
+int lowlat_clear(neo_b200_lowlat* h, lowlat_state<T>& s)
 {
-    lowlat_state<T>& s   = lowlat_of<T>(h);
     cudaStream_t const st = h->stream.stream;
     NEO_TRY(s.head.clear_state(st));
     for (size_t i = 0; i < h->levels; ++i) {
@@ -2111,8 +2085,7 @@ int lowlat_clear(neo_b200_lowlat* h)
     NEO_CUDA_TRY(cudaMemsetAsync(s.in_ring.ptr, 0, s.in_ring.bytes, st));
     h->block_pos  = 0;
     h->sample_pos = 0;  // the pending samples are discarded
-    h->staged     = false;
-    h->fading     = false;
+    h->fade.cancel();
     NEO_CUDA_TRY(cudaStreamSynchronize(st));
     return NEO_B200_OK;
 }
@@ -2134,14 +2107,10 @@ bool lowlat_pairs(T const* p, size_t stride)
     return reinterpret_cast<std::uintptr_t>(p) % (2 * sizeof(T)) == 0 && stride % 2 == 0;
 }
 
-// the staged set becomes the current one once every sample before the end of the fade has been delivered
 template<typename T>
-void lowlat_finish_fade(neo_b200_lowlat* h)
+void lowlat_finish_fade(neo_b200_lowlat* h, lowlat_state<T>& s)
 {
-    if (!h->fading || h->position() < h->fade_end) { return; }
-    lowlat_of<T>(h).swap_sets(h->levels);
-    h->fading = false;
-    h->staged = false;
+    if (h->fade.finish(h->position())) { s.swap_sets(h->levels); }
 }
 
 // positions [pos, end) of block block_pos for every channel: `in` / `out` point at position pos of channel 0. pos == 0, end == B is a
@@ -2149,14 +2118,13 @@ void lowlat_finish_fade(neo_b200_lowlat* h)
 // A segment with samples on both sides of a crossfade's start ... end runs the head twice: the B side outputs only, then the A side,
 // which commits the state as always and blends the two per sample.
 template<typename T>
-int lowlat_segment(neo_b200_lowlat* h, T const* in, size_t in_stride, T* out, size_t out_stride, size_t pos, size_t end)
+int lowlat_segment(neo_b200_lowlat* h, lowlat_state<T>& s, T const* in, size_t in_stride, T* out, size_t out_stride, size_t pos, size_t end)
 {
-    lowlat_state<T>& s   = lowlat_of<T>(h);
     cudaStream_t const st = h->stream.stream;
     size_t const C = h->cfg.channels, B = h->cfg.block, tb = h->block_pos;
     bool const completes = end == B;
-    bool const both      = h->fading && tb * B + pos < h->fade_end && tb * B + end > h->fade_start;
-    conv_fade const fade{tb * B, h->fade_start, h->fade_end - h->fade_start};
+    bool const both      = h->fade.overlaps(tb * B + pos, tb * B + end);
+    conv_fade const fade = h->fade.from(tb * B);
 
     // the partial output of level i for block tb comes from its frame tb / T_i - 2; the first segment of the block waits for it
     lowlat_levels<T> lv{}, lvb{};
@@ -2188,7 +2156,7 @@ int lowlat_segment(neo_b200_lowlat* h, T const* in, size_t in_stride, T* out, si
             lowlat_head_args<T> b = a;
             b.out                 = s.fade_y.template as<T>() + pos;
             b.out_stride          = B;
-            b.filter              = s.spare_head.template as<cx<T>>();
+            b.filter              = e.spare_filter.template as<cx<T>>();
             b.levels              = lvb;
             b.commit              = 0;
             NEO_TRY(launch(b));
@@ -2209,19 +2177,11 @@ int lowlat_segment(neo_b200_lowlat* h, T const* in, size_t in_stride, T* out, si
             blk        = s.window.template as<T>() + B;
             blk_stride = 2 * B;
         }
-        if (both) {  // one insert, the B side's MAC and inverse transform into fade_y, then the A side's MAC as forward() runs it
-            NEO_TRY(e.forward_r2c(blk, blk_stride, 1, 0, C, st));
-            {
-                use_spare const use_b(e.filter, s.spare_head);
-                NEO_TRY(e.forward_mac(1, 0, C, st));
-            }
-            NEO_TRY(e.inverse(e.acc_w(), 0, 1, s.fade_y.template as<T>(), B, 0, C, 1, st));
-            NEO_TRY(e.forward_mac(1, 0, C, st));
-            e.advance(1);
-        } else {
-            NEO_TRY(e.forward(blk, blk_stride, 1, st));
-        }
-        NEO_TRY(e.inverse(static_cast<cx<T> const*>(e.acc_r()), 0, 1, s.head_y.template as<T>(), B, 0, C, 1, st));
+        // one insert, the B side's MAC and inverse transform into fade_y inside a crossfade, the A side's into head_y, one advance
+        NEO_TRY(e.forward_r2c(blk, blk_stride, 1, 0, C, st));
+        if (both) { NEO_TRY(e.mac_inverse(true, 1, 0, C, s.fade_y.template as<T>(), B, st)); }
+        NEO_TRY(e.mac_inverse(false, 1, 0, C, s.head_y.template as<T>(), B, st));
+        e.advance(1);
         dim3 const grid(unsigned((B + 255) / 256), unsigned(C));
         lowlat_combine_kernel<T><<<grid, 256, 0, st>>>(s.head_y.template as<T>(), B, int(pos), int(B), blk, blk_stride, out, out_stride, ring_slot,
                                                        ring_stride, lv, both ? s.fade_y.template as<T>() : nullptr, lvb, fade);
@@ -2234,11 +2194,8 @@ int lowlat_segment(neo_b200_lowlat* h, T const* in, size_t in_stride, T* out, si
         lowlat_window_kernel<T><<<wgrid, 256, 0, st>>>(e.prev[e.prev_flip].template as<T>(), s.pending.template as<T>(), in, in_stride, int(B),
                                                        int(pos), int(end), s.window.template as<T>());
         NEO_TRY(check_launch("lowlat_window_kernel"));
-        NEO_TRY(e.window_step(s.window.template as<T>(), s.window_y.template as<T>(), false, st));
-        if (both) {
-            use_spare const use_b(e.filter, s.spare_head);
-            NEO_TRY(e.window_step(s.window.template as<T>(), s.fade_y.template as<T>(), false, st));
-        }
+        NEO_TRY(e.window_step(s.window.template as<T>(), s.window_y.template as<T>(), false, false, st));
+        if (both) { NEO_TRY(e.window_step(s.window.template as<T>(), s.fade_y.template as<T>(), false, true, st)); }
         dim3 const grid(unsigned((end + 255) / 256), unsigned(C));
         lowlat_combine_kernel<T><<<grid, 256, 0, st>>>(s.window_y.template as<T>() + B, 2 * B, int(pos), int(end), nullptr, 0, out, out_stride,
                                                        nullptr, 0, lv, both ? s.fade_y.template as<T>() + B : nullptr, lvb, fade);
@@ -2246,7 +2203,7 @@ int lowlat_segment(neo_b200_lowlat* h, T const* in, size_t in_stride, T* out, si
     }
     if (!completes) {
         h->sample_pos = end;
-        lowlat_finish_fade<T>(h);
+        lowlat_finish_fade(h, s);
         return NEO_B200_OK;
     }
     h->block_pos  = tb + 1;
@@ -2281,37 +2238,22 @@ int lowlat_segment(neo_b200_lowlat* h, T const* in, size_t in_stride, T* out, si
         conv_engine<T>& e   = s.level[i];
         T const* const frm  = s.in_ring.template as<T>() + ((f * ti) % h->ring_blocks) * B;
         size_t const first  = (f + 2) * ti * B, last = (f + 3) * ti * B;  // the samples this frame's output covers
-        bool const side_a   = !h->fading || first < h->fade_end;
-        bool const side_b   = h->fading && last > h->fade_start;
         size_t const slot   = (f % 2) * ti * B;
-        if (!side_b) {
-            NEO_TRY(e.forward(frm, ring_stride, ti, ls));
-            NEO_TRY(e.inverse(static_cast<cx<T> const*>(e.acc_r()), 0, 1, s.plane[i].template as<T>() + slot, 2 * ti * B, 0, C, ti, ls));
-        } else {
-            // one insert; the second forward_mac stores the same ring slot with the same bits; one advance
-            NEO_TRY(e.forward_r2c(frm, ring_stride, ti, 0, C, ls));
-            if (side_a) {
-                NEO_TRY(e.forward_mac(ti, 0, C, ls));
-                NEO_TRY(e.inverse(e.acc_w(), 0, 1, s.plane[i].template as<T>() + slot, 2 * ti * B, 0, C, ti, ls));
-            }
-            {
-                use_spare const use_b(e.filter2, s.spare_level[i]);
-                NEO_TRY(e.forward_mac(ti, 0, C, ls));
-            }
-            NEO_TRY(e.inverse(e.acc_w(), 0, 1, s.plane_b[i].template as<T>() + slot, 2 * ti * B, 0, C, ti, ls));
-            e.advance(ti);
-        }
+        // one insert, the A side into `plane` and inside a crossfade the B side into `plane_b` (below), one advance
+        NEO_TRY(e.forward_r2c(frm, ring_stride, ti, 0, C, ls));
+        if (!h->fade.fading || first < h->fade.end) { NEO_TRY(e.mac_inverse(false, ti, 0, C, s.plane[i].template as<T>() + slot, 2 * ti * B, ls)); }
+        if (h->fade.fading && last > h->fade.start) { NEO_TRY(e.mac_inverse(true, ti, 0, C, s.plane_b[i].template as<T>() + slot, 2 * ti * B, ls)); }
+        e.advance(ti);
         if (!h->sync) { NEO_CUDA_TRY(cudaEventRecord(h->done[i][f & 1], ls)); }
     }
-    lowlat_finish_fade<T>(h);
+    lowlat_finish_fade(h, s);
     return NEO_B200_OK;
 }
 
 // `samples` consecutive samples of every channel: [channels][samples] rows, cut into segments at block boundaries
 template<typename T>
-int lowlat_process(neo_b200_lowlat* h, void const* in, void* out, size_t samples, int memspace)
+int lowlat_process(neo_b200_lowlat* h, lowlat_state<T>& s, void const* in, void* out, size_t samples, int memspace)
 {
-    lowlat_state<T>& s   = lowlat_of<T>(h);
     cudaStream_t const st = h->stream.stream;
     size_t const B = h->cfg.block, stride = samples, bytes = h->cfg.channels * stride * sizeof(T);
     T const* din = static_cast<T const*>(in);
@@ -2325,7 +2267,7 @@ int lowlat_process(neo_b200_lowlat* h, void const* in, void* out, size_t samples
     }
     for (size_t done = 0; done < samples;) {
         size_t const pos = h->sample_pos, n = std::min(B - pos, samples - done);
-        NEO_TRY(lowlat_segment<T>(h, din + done, stride, dout + done, stride, pos, pos + n));
+        NEO_TRY(lowlat_segment(h, s, din + done, stride, dout + done, stride, pos, pos + n));
         done += n;
     }
     if (memspace == NEO_B200_HOST) {
@@ -2370,7 +2312,7 @@ int neo_b200_lowlat_create(neo_b200_lowlat** handle, neo_b200_lowlat_config cons
         NEO_CUDA_TRY(cudaStreamCreateWithPriority(&p->side[i], cudaStreamNonBlocking, prio));
         for (cudaEvent_t* ev : {&p->ready[i], &p->done[i][0], &p->done[i][1]}) { NEO_CUDA_TRY(cudaEventCreateWithFlags(ev, cudaEventDisableTiming)); }
     }
-    NEO_TRY(config->dtype == NEO_B200_F32 ? lowlat_init<float>(p.get()) : lowlat_init<double>(p.get()));
+    NEO_TRY(with_state(p.get(), [&](auto& s) { return lowlat_init(p.get(), s); }));
     NEO_CUDA_TRY(cudaStreamSynchronize(p->stream.stream));
     *handle = p.release();
     return NEO_B200_OK;
@@ -2379,9 +2321,8 @@ int neo_b200_lowlat_create(neo_b200_lowlat** handle, neo_b200_lowlat_config cons
 void neo_b200_lowlat_destroy(neo_b200_lowlat* handle) { delete handle; }
 
 extern "C++" template<typename T>
-int lowlat_set_filter_impl(neo_b200_lowlat* h, void const* H, void const* ir, size_t taps, int memspace)
+int lowlat_set_filter_impl(neo_b200_lowlat* h, lowlat_state<T>& s, void const* H, void const* ir, size_t taps, int memspace)
 {
-    lowlat_state<T>& s   = lowlat_of<T>(h);
     cudaStream_t const st = h->stream.stream;
     NEO_TRY(h->sync_all());
     h->has_filter = false;
@@ -2392,16 +2333,15 @@ int lowlat_set_filter_impl(neo_b200_lowlat* h, void const* H, void const* ir, si
         NEO_TRY(s.head.set_filter(H, memspace, st));
         for (size_t i = 0; i < h->levels; ++i) { NEO_TRY(s.level[i].set_filter(H, memspace, st)); }
     }
-    NEO_TRY(lowlat_clear<T>(h));
+    NEO_TRY(lowlat_clear(h, s));
     h->has_filter = true;
     return NEO_B200_OK;
 }
 
 // builds H / ir into the spare set on the staging stream; the current set, the delay lines and the position are not touched
 extern "C++" template<typename T>
-int lowlat_stage_impl(neo_b200_lowlat* h, void const* H, void const* ir, size_t taps, int memspace)
+int lowlat_stage_impl(neo_b200_lowlat* h, lowlat_state<T>& s, void const* H, void const* ir, size_t taps, int memspace)
 {
-    lowlat_state<T>& s   = lowlat_of<T>(h);
     size_t const C = h->cfg.channels, B = h->cfg.block;
     if (h->stage_stream == nullptr) {
         int least = 0, greatest = 0;
@@ -2410,12 +2350,8 @@ int lowlat_stage_impl(neo_b200_lowlat* h, void const* H, void const* ir, size_t 
         for (cudaEvent_t& ev : h->stage_after) { NEO_CUDA_TRY(cudaEventCreateWithFlags(&ev, cudaEventDisableTiming)); }
     }
     cudaStream_t const ss = h->stage_stream;
-    NEO_TRY(s.spare_head.reserve(s.head.filter.bytes));
     NEO_TRY(s.fade_y.reserve(C * (h->fused ? 1 : 2) * B * sizeof(T)));
-    for (size_t i = 0; i < h->levels; ++i) {
-        NEO_TRY(s.spare_level[i].reserve(s.level[i].filter2.bytes));
-        NEO_TRY(s.plane_b[i].reserve(s.plane[i].bytes));
-    }
+    for (size_t i = 0; i < h->levels; ++i) { NEO_TRY(s.plane_b[i].reserve(s.plane[i].bytes)); }
     // the spare set may still be read by enqueued work: the A side of a fade that has just ended
     NEO_CUDA_TRY(cudaEventRecord(h->stage_after[0], h->stream.stream));
     NEO_CUDA_TRY(cudaStreamWaitEvent(ss, h->stage_after[0], 0));
@@ -2423,54 +2359,40 @@ int lowlat_stage_impl(neo_b200_lowlat* h, void const* H, void const* ir, size_t 
         NEO_CUDA_TRY(cudaEventRecord(h->stage_after[1 + i], h->side[i]));
         NEO_CUDA_TRY(cudaStreamWaitEvent(ss, h->stage_after[1 + i], 0));
     }
-    h->staged = false;
-    {
-        use_spare const use(s.head.filter, s.spare_head);
-        NEO_TRY(ir != nullptr ? s.head.load_impulse(ir, taps, memspace, ss) : s.head.load_filter(H, memspace, ss));
-    }
-    for (size_t i = 0; i < h->levels; ++i) {
-        use_spare const use(s.level[i].filter2, s.spare_level[i]);
-        NEO_TRY(ir != nullptr ? s.level[i].load_impulse(ir, taps, memspace, ss) : s.level[i].load_filter(H, memspace, ss));
-    }
+    h->fade.staged = false;
+    NEO_TRY(s.head.stage(H, ir, taps, memspace, ss));
+    for (size_t i = 0; i < h->levels; ++i) { NEO_TRY(s.level[i].stage(H, ir, taps, memspace, ss)); }
     NEO_CUDA_TRY(cudaStreamSynchronize(ss));
-    h->staged = true;
+    h->fade.staged = true;
     return NEO_B200_OK;
 }
 
-extern "C++" static int lowlat_stage_check(neo_b200_lowlat* h)
+extern "C++" static int lowlat_stage(neo_b200_lowlat* h, void const* H, void const* ir, size_t taps, int memspace)
 {
+    if (ir != nullptr) { NEO_TRY(check_taps(taps, h->cfg.block, h->cfg.partitions, false)); }
     if (!h->has_filter) { return fail(NEO_B200_ERR_INVALID, "no filter set: stage needs a current filter to fade from"); }
-    if (h->fading) { return fail(NEO_B200_ERR_INVALID, "a crossfade is pending or running"); }
+    if (h->fade.fading) { return fail(NEO_B200_ERR_INVALID, "a crossfade is pending or running"); }
     NEO_CUDA_TRY(cudaSetDevice(h->device));
-    return NEO_B200_OK;
+    return with_state(h, [&](auto& s) { return lowlat_stage_impl(h, s, H, ir, taps, memspace); });
 }
 
 int neo_b200_lowlat_stage_filter(neo_b200_lowlat* handle, void const* H, int memspace)
 {
     if (handle == nullptr || H == nullptr) { return fail(NEO_B200_ERR_INVALID, "null argument"); }
-    NEO_TRY(lowlat_stage_check(handle));
-    if (handle->cfg.dtype == NEO_B200_F32) { return lowlat_stage_impl<float>(handle, H, nullptr, 0, memspace); }
-    return lowlat_stage_impl<double>(handle, H, nullptr, 0, memspace);
+    return lowlat_stage(handle, H, nullptr, 0, memspace);
 }
 
 int neo_b200_lowlat_stage_impulse(neo_b200_lowlat* handle, void const* ir, size_t taps, int memspace)
 {
     if (handle == nullptr || ir == nullptr) { return fail(NEO_B200_ERR_INVALID, "null argument"); }
-    if (taps < handle->cfg.block) { return fail(NEO_B200_ERR_INVALID, "impulse response shorter than one block"); }
-    if (neo_b200_num_partitions(taps, handle->cfg.block) > handle->cfg.partitions) {
-        return fail(NEO_B200_ERR_INVALID, "taps=%zu gives %zu partitions, the handle holds %zu", taps, neo_b200_num_partitions(taps, handle->cfg.block),
-                    handle->cfg.partitions);
-    }
-    NEO_TRY(lowlat_stage_check(handle));
-    if (handle->cfg.dtype == NEO_B200_F32) { return lowlat_stage_impl<float>(handle, nullptr, ir, taps, memspace); }
-    return lowlat_stage_impl<double>(handle, nullptr, ir, taps, memspace);
+    return lowlat_stage(handle, nullptr, ir, taps, memspace);
 }
 
 int neo_b200_lowlat_crossfade(neo_b200_lowlat* handle, size_t fade, size_t* start)
 {
     if (handle == nullptr) { return fail(NEO_B200_ERR_INVALID, "null argument"); }
-    if (handle->fading) { return fail(NEO_B200_ERR_INVALID, "a crossfade is already pending or running"); }
-    if (!handle->staged) { return fail(NEO_B200_ERR_INVALID, "nothing staged: call neo_b200_lowlat_stage_filter / _stage_impulse first"); }
+    if (handle->fade.fading) { return fail(NEO_B200_ERR_INVALID, "a crossfade is already pending or running"); }
+    if (!handle->fade.staged) { return fail(NEO_B200_ERR_INVALID, "nothing staged: call neo_b200_lowlat_stage_filter / _stage_impulse first"); }
     // level i's B side starts with the first frame released after this call, floor(b / T_i), whose output begins at block
     // (floor(b / T_i) + 2) T_i; b is the block holding the next sample. With no levels the head alone starts at the next sample.
     size_t at = handle->position();
@@ -2481,12 +2403,11 @@ int neo_b200_lowlat_crossfade(neo_b200_lowlat* handle, size_t fade, size_t* star
     }
     if (fade > SIZE_MAX - at) { return fail(NEO_B200_ERR_INVALID, "fade of %zu samples overflows the stream position", fade); }
     NEO_CUDA_TRY(cudaSetDevice(handle->device));
-    handle->fading     = true;
-    handle->fade_start = at;
-    handle->fade_end   = at + fade;
+    handle->fade.fading = true;
+    handle->fade.start  = at;
+    handle->fade.end    = at + fade;
     if (start != nullptr) { *start = at; }
-    if (handle->cfg.dtype == NEO_B200_F32) { lowlat_finish_fade<float>(handle); }
-    else { lowlat_finish_fade<double>(handle); }
+    with_state(handle, [&](auto& s) { lowlat_finish_fade(handle, s); });
     return NEO_B200_OK;
 }
 
@@ -2494,21 +2415,15 @@ int neo_b200_lowlat_set_filter(neo_b200_lowlat* handle, void const* H, int memsp
 {
     if (handle == nullptr || H == nullptr) { return fail(NEO_B200_ERR_INVALID, "null argument"); }
     NEO_CUDA_TRY(cudaSetDevice(handle->device));
-    if (handle->cfg.dtype == NEO_B200_F32) { return lowlat_set_filter_impl<float>(handle, H, nullptr, 0, memspace); }
-    return lowlat_set_filter_impl<double>(handle, H, nullptr, 0, memspace);
+    return with_state(handle, [&](auto& s) { return lowlat_set_filter_impl(handle, s, H, nullptr, 0, memspace); });
 }
 
 int neo_b200_lowlat_set_impulse(neo_b200_lowlat* handle, void const* ir, size_t taps, int memspace)
 {
     if (handle == nullptr || ir == nullptr) { return fail(NEO_B200_ERR_INVALID, "null argument"); }
-    if (taps < handle->cfg.block) { return fail(NEO_B200_ERR_INVALID, "impulse response shorter than one block"); }
-    if (neo_b200_num_partitions(taps, handle->cfg.block) != handle->cfg.partitions) {
-        return fail(NEO_B200_ERR_INVALID, "taps=%zu gives %zu partitions, handle was created for %zu", taps,
-                    neo_b200_num_partitions(taps, handle->cfg.block), handle->cfg.partitions);
-    }
+    NEO_TRY(check_taps(taps, handle->cfg.block, handle->cfg.partitions, true));
     NEO_CUDA_TRY(cudaSetDevice(handle->device));
-    if (handle->cfg.dtype == NEO_B200_F32) { return lowlat_set_filter_impl<float>(handle, nullptr, ir, taps, memspace); }
-    return lowlat_set_filter_impl<double>(handle, nullptr, ir, taps, memspace);
+    return with_state(handle, [&](auto& s) { return lowlat_set_filter_impl(handle, s, nullptr, ir, taps, memspace); });
 }
 
 int neo_b200_lowlat_reset(neo_b200_lowlat* handle)
@@ -2516,7 +2431,7 @@ int neo_b200_lowlat_reset(neo_b200_lowlat* handle)
     if (handle == nullptr) { return fail(NEO_B200_ERR_INVALID, "null argument"); }
     NEO_CUDA_TRY(cudaSetDevice(handle->device));
     NEO_TRY(handle->sync_all());
-    return handle->cfg.dtype == NEO_B200_F32 ? lowlat_clear<float>(handle) : lowlat_clear<double>(handle);
+    return with_state(handle, [&](auto& s) { return lowlat_clear(handle, s); });
 }
 
 int neo_b200_lowlat_process(neo_b200_lowlat* handle, void const* in, void* out, size_t blocks, int memspace)
@@ -2526,9 +2441,7 @@ int neo_b200_lowlat_process(neo_b200_lowlat* handle, void const* in, void* out, 
     if (in == nullptr || out == nullptr) { return fail(NEO_B200_ERR_INVALID, "null buffer"); }
     if (blocks == 0) { return fail(NEO_B200_ERR_INVALID, "blocks must be >= 1"); }
     NEO_CUDA_TRY(cudaSetDevice(handle->device));
-    size_t const samples = blocks * handle->cfg.block;
-    if (handle->cfg.dtype == NEO_B200_F32) { return lowlat_process<float>(handle, in, out, samples, memspace); }
-    return lowlat_process<double>(handle, in, out, samples, memspace);
+    return with_state(handle, [&](auto& s) { return lowlat_process(handle, s, in, out, blocks * handle->cfg.block, memspace); });
 }
 
 int neo_b200_lowlat_process_samples(neo_b200_lowlat* handle, void const* in, void* out, size_t samples, int memspace)
@@ -2538,8 +2451,7 @@ int neo_b200_lowlat_process_samples(neo_b200_lowlat* handle, void const* in, voi
     if (in == nullptr || out == nullptr) { return fail(NEO_B200_ERR_INVALID, "null buffer"); }
     if (samples == 0) { return fail(NEO_B200_ERR_INVALID, "samples must be >= 1"); }
     NEO_CUDA_TRY(cudaSetDevice(handle->device));
-    if (handle->cfg.dtype == NEO_B200_F32) { return lowlat_process<float>(handle, in, out, samples, memspace); }
-    return lowlat_process<double>(handle, in, out, samples, memspace);
+    return with_state(handle, [&](auto& s) { return lowlat_process(handle, s, in, out, samples, memspace); });
 }
 
 int neo_b200_lowlat_set_stream(neo_b200_lowlat* handle, void* cuda_stream)
@@ -2561,7 +2473,7 @@ int neo_b200_lowlat_synchronize(neo_b200_lowlat* handle)
 size_t neo_b200_lowlat_device_bytes(neo_b200_lowlat const* handle)
 {
     if (handle == nullptr) { return 0; }
-    return handle->cfg.dtype == NEO_B200_F32 ? handle->f32.device_bytes(handle->levels) : handle->f64.device_bytes(handle->levels);
+    return with_state(handle, [&](auto& s) { return s.device_bytes(handle->levels); });
 }
 
 }  // extern "C"

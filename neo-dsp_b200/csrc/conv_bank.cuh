@@ -229,13 +229,6 @@ struct neo_b200_bank
 namespace neo_b200 {
 namespace {
 
-template<typename F>
-int bank_with_engine(neo_b200_conv* conv, F&& f)
-{
-    if (conv->cfg.dtype == NEO_B200_F32) { return f(conv->f32); }
-    return f(conv->f64);
-}
-
 // shard gp of Gp over the partition axis; in frame mode shards start on frame boundaries (the delay of a shard is whole frames)
 inline void bank_partition_range(size_t parts, size_t frame, size_t shards, size_t gp, size_t* lo, size_t* hi)
 {
@@ -309,7 +302,7 @@ int bank_build_rank(neo_b200_bank* bank, bank_rank& r)
     NEO_CUDA_TRY(cudaMemsetAsync(r.xring.ptr, 0, r.xring.bytes, r.s_in));
     NEO_CUDA_TRY(cudaStreamSynchronize(r.s_in));
     bool fused = false;
-    (void)bank_with_engine(r.conv, [&](auto& e) {
+    (void)with_engine(r.conv, [&](auto& e) {
         fused = e.fused;
         return NEO_B200_OK;
     });
@@ -563,7 +556,7 @@ int bank_submit_impl(neo_b200_bank* bank, void const* const* in_rows, void* cons
         size_t const delay_slots = c.frame_blocks > 0 ? r.info.delay_blocks / c.frame_blocks : 0;
         size_t const read_slot   = (step + r.slots - delay_slots) % r.slots;  // zeros until the delayed step exists
         T const* const x         = r.xring.template as<T>() + read_slot * r.slot_elems;
-        NEO_TRY(bank_with_engine(r.conv, [&](auto& e) -> int {
+        NEO_TRY(with_engine(r.conv, [&](auto& e) -> int {
             using E = std::remove_reference_t<decltype(e)>;
             if constexpr (std::is_same_v<E, conv_engine<T>>) {
                 NEO_TRY(e.forward_r2c(x, pitch, blocks, 0, r.conv->cfg.inputs, r.s_cmp));
@@ -711,10 +704,10 @@ int bank_finish_impl(neo_b200_bank* bank, neo_b200_bank_step& st)
                 NEO_CUDA_TRY(cudaStreamWaitEvent(r.s_cmp, r.ev_out[(st.step - k_bank_depth) & 3U], 0));
             }
         }
-        NEO_TRY(bank_with_engine(r.conv, [&](auto& e) -> int {
+        NEO_TRY(with_engine(r.conv, [&](auto& e) -> int {
             using E = std::remove_reference_t<decltype(e)>;
             if constexpr (std::is_same_v<E, conv_engine<T>>) {
-                return e.inverse_sum(srcs, nsrc, dst, pitch, own_in_group, r.info.out_count, blocks, r.s_cmp);
+                return e.inverse(srcs, nsrc, dst, pitch, own_in_group, r.info.out_count, blocks, r.s_cmp);
             }
             return NEO_B200_OK;
         }));
@@ -1025,7 +1018,7 @@ int neo_b200_bank_profile_read(neo_b200_bank* bank, size_t local_index, double* 
     cudaGetDevice(&before);
     NEO_CUDA_TRY(cudaSetDevice(r.info.device));
     for (cudaStream_t s : {r.s_in, r.s_cmp, r.s_red, r.s_out}) { NEO_CUDA_TRY(cudaStreamSynchronize(s)); }
-    int const status = bank_with_engine(r.conv, [&](auto& e) { return e.read_profile(phase_ms, mac_launches, r.s_cmp); });
+    int const status = with_engine(r.conv, [&](auto& e) { return e.read_profile(phase_ms, mac_launches, r.s_cmp); });
     cudaSetDevice(before);
     return status;
 }
