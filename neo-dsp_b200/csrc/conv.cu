@@ -91,16 +91,10 @@ struct conv_engine
     bool has_filter{false};
 
     fft_tables<T> tables;
-    // float32, B = 1024 (the 2048-point real transforms of BASELINE config 5): one warp per transform, 32 points per thread, Hermitian
-    // split in registers, 128-bit accesses on the real side (fft_wide.cuh). NEO_B200_CONV_NO_WIDE keeps the 16-points-per-thread kernels.
-    // Measured (C5, frame mode T = 256, ms per step): c2r 0.668 -> 0.631 (15 % fewer instructions, 0.78 of HBM by its 12 bytes per sample);
-    // r2c 0.682 -> 0.699 (14 % fewer instructions, but 16 instead of 32 resident warps leave its loads exposed), so the forward side
-    // takes the wide kernel only with NEO_B200_CONV_WIDE_R2C.
+    // float32, B = 1024 (the 2048-point real transforms of BASELINE config 5): the inverse side runs one warp per transform, 32 points
+    // per thread, Hermitian split in registers, 128-bit stores on the real side (fft_wide.cuh, DESIGN.md section 4.1)
     wide_tables<10, 3, 3> wide10;
-    bool use_wide{false}, use_wide_r2c{false};
-    // resident CTAs the wide kernels are compiled for (NEO_B200_CONV_WIDE_R2C / _C2R = 4, 5, 6 -> 128 / 96 / 80 registers). Measured (C5, frame
-    // mode T = 256, ms per step, r2c / c2r): 4: 0.704 / 0.636, 5: 0.672 / 0.611, 6: 0.756 / 0.743 (spills), cta_fft r2c 0.689
-    int wide_minb_r2c{5}, wide_minb_c2r{5};
+    bool use_wide{false};
     device_buffer filter, fdl, prev[2], tail, acc, acc_alt, ola_y, stage_in, stage_out, stage_filter, tickets;
     // sparse filters (set_filter_csr): bitmap form of the reference's CSR matrices (conv_kernels.cuh, fdl_mac_sparse_kernel); the
     // dense filter buffer is released while they are in place
@@ -258,11 +252,8 @@ struct conv_engine
         nt      = m >> logw;
         NEO_TRY(tables.build(logb, true, stream));
         if constexpr (sizeof(T) == 4) {
-            use_wide = logb == 10 && std::getenv("NEO_B200_CONV_NO_WIDE") == nullptr;
+            use_wide = logb == 10;
             if (use_wide) { NEO_TRY(wide10.build(stream)); }
-            use_wide_r2c = use_wide && std::getenv("NEO_B200_CONV_WIDE_R2C") != nullptr;
-            if (char const* v = std::getenv("NEO_B200_CONV_WIDE_R2C")) { wide_minb_r2c = std::max(4, std::min(6, std::atoi(v))); }
-            if (char const* v = std::getenv("NEO_B200_CONV_WIDE_C2R")) { wide_minb_c2r = std::max(4, std::min(6, std::atoi(v))); }
         }
 
         size_t const csz = sizeof(cx<T>);
@@ -550,22 +541,10 @@ struct conv_engine
         return ir != nullptr ? load_impulse(ir, taps, memspace, stream) : load_filter(h, memspace, stream);
     }
 
-    // the wide kernels move the real rows with 128-bit accesses
+    // the wide c2r stores the real rows with 128-bit accesses, so it needs 16-byte aligned rows; the others take `cta_fft`'s c2r
     bool wide_rows_ok(void const* rows, size_t stride) const
     {
         return use_wide && (reinterpret_cast<std::uintptr_t>(rows) & 15U) == 0 && stride % 4 == 0;
-    }
-
-    template<int LOGM, class IO>
-    int run_r2c(IO const& io, bool wide, size_t batch, cudaStream_t stream)
-    {
-        if constexpr (sizeof(T) == 4 && LOGM == 10) {
-            if (wide) {
-                return launch_r2c_wide_io<10, 3, 3>(io, wide10.ta.template as<float2>(), wide10.tb_fwd.template as<float2>(),
-                                                    wide10.rtw.template as<float2>(), batch, stream, wide_minb_r2c);
-            }
-        }
-        return launch_r2c<T, LOGM>(io, tables.tw(), tables.rtw(), batch, stream);
     }
 
     template<int LOGM, class IO>
@@ -574,7 +553,7 @@ struct conv_engine
         if constexpr (sizeof(T) == 4 && LOGM == 10) {
             if (wide) {
                 return launch_c2r_wide_io<10, 3, 3>(io, wide10.ta.template as<float2>(), wide10.tb_bwd.template as<float2>(),
-                                                    wide10.rtw.template as<float2>(), batch, stream, wide_minb_c2r);
+                                                    wide10.rtw.template as<float2>(), batch, stream);
             }
         }
         return launch_c2r<T, LOGM>(io, tables.tw(), tables.rtw(), batch, stream);
@@ -591,12 +570,12 @@ struct conv_engine
                     conv_r2c_io<T, LOGM, true> io{in, in_stride, prev[prev_flip].template as<T>(), prev[prev_flip ^ 1].template as<T>(),
                                                   fdl.template as<cx<T>>(), ring, x1_half * frame, int(blocks),
                                                   cfg.kind == NEO_B200_UPOLA ? 1 : 0, logb, 1, chan0};
-                    status = run_r2c<LOGM>(io, use_wide_r2c && wide_rows_ok(in, in_stride), nchan * blocks, stream);
+                    status = launch_r2c<T, LOGM>(io, tables.tw(), tables.rtw(), nchan * blocks, stream);
                 } else {
                     conv_r2c_io<T, LOGM> io{in, in_stride, prev[prev_flip].template as<T>(), prev[prev_flip ^ 1].template as<T>(),
                                             fdl.template as<cx<T>>(), ring, int(write_pos), int(blocks),
                                             cfg.kind == NEO_B200_UPOLA ? 1 : 0, logw, nt, chan0};
-                    status = run_r2c<LOGM>(io, use_wide_r2c && wide_rows_ok(in, in_stride), nchan * blocks, stream);
+                    status = launch_r2c<T, LOGM>(io, tables.tw(), tables.rtw(), nchan * blocks, stream);
                 }
             }
         });

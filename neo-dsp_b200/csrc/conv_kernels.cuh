@@ -597,19 +597,6 @@ struct conv_r2c_io
         else { r.dst[((size_t(k >> logw) * ring) << logw) + (k & ((1 << logw) - 1))] = x; }
     }
     __device__ __forceinline__ void store_edges(row_state const& r, T dc, T nyq) const { r.dst[0] = mk<T>(dc, nyq); }
-    // the wide kernel's 128-bit accesses (float rows on 16-byte boundaries): complex pairs j, j + 1 of the lower (previous block) /
-    // upper (this block) half-window, j even and relative to the half
-    template<bool HI>
-    __device__ __forceinline__ float4 load_pair(row_state const& r, int j) const
-    {
-        static_assert(sizeof(T) == 4, "float rows");
-        if constexpr (HI) { return r.hi != nullptr ? *reinterpret_cast<float4 const*>(r.hi + j) : make_float4(0.0F, 0.0F, 0.0F, 0.0F); }
-        else { return *reinterpret_cast<float4 const*>(r.lo + j); }
-    }
-    __device__ __forceinline__ void keep_pair(row_state const& r, int j, float4 v) const
-    {
-        if (r.keep != nullptr) { *reinterpret_cast<float4*>(r.keep + j) = v; }
-    }
 };
 
 // neo::convolution::overlap_add_convolver (overlap_add_convolver.hpp:85-132) transforms its real window AS IT STANDS: after a call
@@ -714,8 +701,6 @@ struct conv_c2r_fade_io
     T scale;
     T const* yb;
     conv_fade fade;
-    // the wide c2r at 6 resident CTAs (80 registers) would spill the blend; a fade call runs it at 5 (96), same arithmetic
-    static constexpr int wide_max_minb = 5;
 
     struct row_state
     {

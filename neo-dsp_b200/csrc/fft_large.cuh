@@ -234,7 +234,7 @@ struct large_fft
     }
 };
 
-// ---- real transforms above the single-CTA range: half-size complex FFT + split pass over global memory --------------------
+// ---- real transforms past the one- and two-CTA forms: half-size complex FFT + split pass over global memory (rfft_engine) -------
 template<typename T, int DIR>
 __global__ void __launch_bounds__(256) split_pass_kernel(cx<T> const* __restrict__ in, size_t in_row, cx<T>* __restrict__ out, size_t out_row,
                                                          twiddle2_view<T> w2m, size_t m)
@@ -263,6 +263,7 @@ __global__ void __launch_bounds__(256) split_pass_kernel(cx<T> const* __restrict
     dst[k]        = DIR < 0 ? r2c_post(a, p, w) : c2r_pre(a, p, w);
 }
 
+// N = 1 (rfft_engine): the spectrum is the sample, and back
 template<typename T>
 __global__ void size_one_r2c_kernel(T const* in, cx<T>* out, size_t batch)
 {
@@ -276,67 +277,5 @@ __global__ void size_one_c2r_kernel(cx<T> const* in, size_t row_len, T* out, siz
     size_t const i = size_t(blockIdx.x) * blockDim.x + threadIdx.x;
     if (i < batch) { out[i] = in[i * row_len].x; }
 }
-
-template<typename T>
-struct large_rfft
-{
-    int order{0};
-    int logm{0};
-    large_fft<T> c2c;
-    twiddle2<T> w2m;
-    device_buffer zbuf;
-
-    int init(int order_, cudaStream_t stream)
-    {
-        order = order_;
-        logm  = order - 1;
-        NEO_TRY(c2c.init(logm, stream));
-        return w2m.build(order, stream);
-    }
-
-    int forward(T const* in, cx<T>* out, size_t batch, cudaStream_t stream)
-    {
-        size_t const m     = size_t(1) << logm;
-        size_t const chunk = std::max<size_t>(1, std::min(batch, (size_t(32) << 20) / (m * sizeof(cx<T>))));
-        NEO_TRY(zbuf.reserve(chunk * m * sizeof(cx<T>)));
-        cx<T>* const z = zbuf.template as<cx<T>>();
-        for (size_t first = 0; first < batch; first += chunk) {
-            size_t const cnt = std::min(chunk, batch - first);
-            NEO_TRY(c2c.exec(reinterpret_cast<cx<T> const*>(in) + first * m, z, cnt, -1, stream));
-            dim3 const grid(static_cast<unsigned>((m + 255) / 256), static_cast<unsigned>(cnt));
-            split_pass_kernel<T, -1><<<grid, 256, 0, stream>>>(z, m, out + first * (m + 1), m + 1, w2m.view(), m);
-            NEO_TRY(check_launch("split_pass_kernel"));
-        }
-        return NEO_B200_OK;
-    }
-
-    int backward(cx<T> const* in, size_t row_len, T* out, size_t batch, cudaStream_t stream)
-    {
-        size_t const m     = size_t(1) << logm;
-        size_t const chunk = std::max<size_t>(1, std::min(batch, (size_t(32) << 20) / (m * sizeof(cx<T>))));
-        NEO_TRY(zbuf.reserve(chunk * m * sizeof(cx<T>)));
-        cx<T>* const z = zbuf.template as<cx<T>>();
-        for (size_t first = 0; first < batch; first += chunk) {
-            size_t const cnt = std::min(chunk, batch - first);
-            dim3 const grid(static_cast<unsigned>((m + 255) / 256), static_cast<unsigned>(cnt));
-            split_pass_kernel<T, +1><<<grid, 256, 0, stream>>>(in + first * row_len, row_len, z, m, w2m.view(), m);
-            NEO_TRY(check_launch("split_pass_kernel"));
-            NEO_TRY(c2c.exec(z, reinterpret_cast<cx<T>*>(out) + first * m, cnt, +1, stream));
-        }
-        return NEO_B200_OK;
-    }
-
-    static int size_one_forward(T const* in, cx<T>* out, size_t batch, cudaStream_t stream)
-    {
-        size_one_r2c_kernel<T><<<static_cast<unsigned>((batch + 255) / 256), 256, 0, stream>>>(in, out, batch);
-        return check_launch("size_one_r2c_kernel");
-    }
-
-    static int size_one_backward(cx<T> const* in, size_t row_len, T* out, size_t batch, cudaStream_t stream)
-    {
-        size_one_c2r_kernel<T><<<static_cast<unsigned>((batch + 255) / 256), 256, 0, stream>>>(in, row_len, out, batch);
-        return check_launch("size_one_c2r_kernel");
-    }
-};
 
 }  // namespace neo_b200

@@ -5,15 +5,8 @@
 #include "fft_large.cuh"
 #include "fft_split.cuh"
 #include "fft_wide.cuh"
-// two forms of the 65536-point real transform that were measured and lost (DESIGN.md section 4.1): compiled only on request
-#ifdef NEO_B200_EXPERIMENTAL_FFT
-#include "fft_cluster.cuh"
-#include "fft_pair.cuh"
-#include "fft_stream.cuh"  // persistent CTAs fed by TMA bulk copies, N = 2^13 / 2^14 (NEO_B200_STREAM=1): 0.65/0.71 and 0.52/0.54 of HBM peak
-#endif
 
 #include <cmath>
-#include <cstdlib>
 #include <memory>
 
 namespace neo_b200 {
@@ -291,32 +284,22 @@ template<typename T>
 struct rfft_engine
 {
     int order;                   // real size N = 2^order, complex half size M = N/2
-    fft_tables<T> tables;        // single-CTA path: M-point plan; split path: M/2-point plan
-    fft_tables<T> tables_full;   // M = 2^max_cta as ONE CTA: only behind the NEO_B200_R2C_ONE_CTA / NEO_B200_C2R_ONE_CTA knobs
-    device_buffer w_n;           // split path: exp(-2 pi i k / N), k < M/2
-    large_rfft<T> large;
-    bool use_large{false};
+    fft_tables<T> tables;        // one-CTA path: M-point plan; two-CTA path: M/2-point plan
+    device_buffer w_n;           // two-CTA path: exp(-2 pi i k / N), k < M/2
     bool use_split{false};       // two CTAs per transform (fft_split.cuh)
-#ifdef NEO_B200_EXPERIMENTAL_FFT
-    bool use_cluster{false};     // float32, N = 2^14..2^16: persistent thread-block-cluster four-step (fft_cluster.cuh)
-    rfft_cluster_plan cluster;
-#endif
-    bool use_split15{false};     // float32, N = 2^16 as two 1024-thread CTAs of 2^14 points each (knob)
-    bool use_pair{false};        // float32, N = 2^16: one transform per CTA pair, exchange tile in distributed shared memory (fft_pair.cuh)
     bool use_big_cta{false};     // float32, M = 2^14: one 1024-thread CTA per transform (139 KB exchange tile)
-    bool use_wide{false};        // float32, N = 2^14 / 2^15: 32 points per thread, three stages, Hermitian split in registers (fft_wide.cuh)
-    wide_tables<12, 4, 4> wide12;
+    bool use_wide{false};        // float32, N = 2^14..2^16: 32 points per thread, three stages, Hermitian split in registers (fft_wide.cuh)
     wide_tables<13, 4, 5> wide13;
     wide_tables<14, 5, 5> wide14;
     wide_split_tables<14, 5, 5> wide15s;  // N = 2^16: two CTAs of 2^14 points per transform
-    bool use_two_pass{false};    // four-CTA split c2c into an L2-resident scratch + Hermitian split pass
-    c2c_engine<T> half;          // two-pass path: the half-size complex transform
+    bool use_two_pass{false};    // half-size complex transform into a chunked scratch + Hermitian split pass (split_pass_kernel)
+    c2c_engine<T> half;          // two-pass path: the half-size complex transform (four-CTA split or four-step)
     twiddle2<T> w2m;             // two-pass path: exp(-2 pi i k / N)
     device_buffer zbuf;
 
-    // half-size transforms of 2^(max_cta) and 2^(max_cta+1) points run as two CTAs of half that size each
-    static constexpr int k_split_lo = max_cta_logm<T>();
-    static constexpr int k_split_hi = max_cta_logm<T>() + 1;
+    // the half size that runs as two CTAs of half that size each: double the first one past a CTA; float the one after it, since
+    // M = 2^14 fits one 1024-thread CTA (use_big_cta)
+    static constexpr int k_split = max_cta_logm<T>() + (sizeof(T) == 4 ? 2 : 1);
 
     int init(int order_, cudaStream_t stream)
     {
@@ -324,63 +307,23 @@ struct rfft_engine
         if (order == 0) { return NEO_B200_OK; }
         int const logm = order - 1;
         if constexpr (sizeof(T) == 4) {
-            bool const w13 = order == 13 && std::getenv("NEO_B200_WIDE13") != nullptr;  // A/B knob: N = 8192 through the wide kernel too
-            if ((order == 14 || order == 15 || order == 16 || w13) && std::getenv("NEO_B200_NO_WIDE") == nullptr) {
+            if (order >= 14 && order <= 16) {
                 use_wide = true;
-                NEO_TRY(order == 13   ? wide12.build(stream)
-                        : order == 14 ? wide13.build(stream)
-                        : order == 15 ? wide14.build(stream)
-                                      : wide15s.build(stream));
+                NEO_TRY(order == 14 ? wide13.build(stream) : order == 15 ? wide14.build(stream) : wide15s.build(stream));
                 // no return: the 16-points-per-thread path below stays initialised for arrays that are not 16-byte aligned
             }
-        }
-        if constexpr (sizeof(T) == 4) {
-            // N = 2^16, measured fractions of HBM peak (r2c / c2r), all parity-tested:
-            //   two 1024-thread CTAs of 2^14 points each (fft_split.cuh, no communication)       0.39 / 0.36   <- shipped
-            //   persistent cluster four-step through an L2 scratch (fft_cluster.cuh)              0.26 / 0.29   NEO_B200_CLUSTER16
-            //   CTA pair, exchange tile in distributed shared memory (fft_pair.cuh)               0.19 / 0.18   NEO_B200_PAIR
-            //   four-CTA split c2c + Hermitian pass (two HBM-side passes)                          0.12 / 0.15   NEO_B200_NO_SPLIT15
-            // The DSMEM form loses because half of every exchange crosses the SM-to-SM network (~20 B/clk per SM) and each of its
-            // 8 exchanges ends in a cluster barrier; the cluster four-step because its phases serialise.
-#ifdef NEO_B200_EXPERIMENTAL_FFT
-            bool const all = std::getenv("NEO_B200_CLUSTER_ALL") != nullptr;
-            if (order == 16 && std::getenv("NEO_B200_PAIR") != nullptr) {
-                use_pair = true;
+            if (logm == 14) {
+                use_big_cta = true;
                 return tables.build(logm, true, stream);
             }
-            if (((order == 16 && std::getenv("NEO_B200_CLUSTER16") != nullptr) || (all && order >= 14 && order <= 16))
-                && std::getenv("NEO_B200_NO_CLUSTER") == nullptr) {
-                use_cluster = true;
-                return cluster.init(order, stream);
-            }
-#endif
-            if (order == 16 && std::getenv("NEO_B200_NO_SPLIT15") == nullptr) {
-                use_split15 = true;
-                NEO_TRY(tables.build(logm - 1, true, stream));
-                auto const wn      = make_split_twiddles<T>(logm);
-                size_t const bytes = (wn.size() / 2) * sizeof(cx<T>);
-                NEO_TRY(w_n.reserve(bytes));
-                NEO_CUDA_TRY(cudaMemcpyAsync(w_n.ptr, wn.data(), bytes, cudaMemcpyHostToDevice, stream));
-                NEO_CUDA_TRY(cudaStreamSynchronize(stream));
-                return NEO_B200_OK;
-            }
         }
-        // measured (N = 2^15): one 1024-thread CTA per transform 0.48 / 0.41 of HBM peak (r2c / c2r) against 0.37 / 0.36 for two
-        // 8192-point CTAs that each read the whole input
-        if (sizeof(T) == 4 && logm == 14 && std::getenv("NEO_B200_NO_BIG_CTA") == nullptr) {
-            use_big_cta = true;
-            return tables.build(logm, true, stream);
-        }
-        use_split      = logm >= k_split_lo && logm <= k_split_hi;
-        use_two_pass   = logm == k_split_hi + 1;
-        use_large      = logm > k_split_hi + 1;
-        if (use_large) { return large.init(order, stream); }
+        use_split    = logm == k_split;
+        use_two_pass = logm > k_split;
         if (use_two_pass) {
             NEO_TRY(half.init(logm, stream));
             return w2m.build(order, stream);
         }
         if (use_split) {
-            if (logm == k_split_lo) { NEO_TRY(tables_full.build(logm, true, stream)); }
             NEO_TRY(tables.build(logm - 1, true, stream));
             auto const wn = make_split_twiddles<T>(logm);  // exp(-i pi k / M) = exp(-2 pi i k / N); first M/2 entries used
             size_t const bytes = (wn.size() / 2) * sizeof(cx<T>);
@@ -392,19 +335,12 @@ struct rfft_engine
         return tables.build(logm, true, stream);
     }
 
-    // the TMA-staged persistent kernels want 16-byte aligned arrays (any cudaMalloc / torch allocation is); NEO_B200_NO_STREAM
-    // switches them off (A/B measurements)
-    static bool stream_ok(void const* a, void const* b)
-    {
-        static bool const on = std::getenv("NEO_B200_STREAM") != nullptr;
-        return on && (reinterpret_cast<std::uintptr_t>(a) & 15U) == 0 && (reinterpret_cast<std::uintptr_t>(b) & 15U) == 0;
-    }
-
-    // chunks keep the intermediate spectrum L2-resident between the two passes
-    size_t two_pass_chunk(size_t batch)
+    // chunks keep the intermediate spectrum L2-resident between the two passes: 48 MB behind the four-CTA split c2c, 32 MB behind
+    // the four-step (fft_large.cuh), which walks its own scratch in 32 MB chunks as well
+    size_t two_pass_chunk(size_t batch) const
     {
         size_t const bytes = (size_t(1) << (order - 1)) * sizeof(cx<T>);
-        static size_t const mb = std::getenv("NEO_B200_FFT_CHUNK_MB") ? size_t(std::atoi(std::getenv("NEO_B200_FFT_CHUNK_MB"))) : 48;
+        size_t const mb    = half.use_large ? 32 : 48;
         return std::max<size_t>(1, std::min(batch, (mb << 20) / bytes));
     }
 
@@ -442,46 +378,20 @@ struct rfft_engine
 
     int forward(T const* in, cx<T>* out, size_t batch, cudaStream_t stream)
     {
-        if (order == 0) { return large_rfft<T>::size_one_forward(in, out, batch, stream); }
+        if (order == 0) {
+            size_one_r2c_kernel<T><<<static_cast<unsigned>((batch + 255) / 256), 256, 0, stream>>>(in, out, batch);
+            return check_launch("size_one_r2c_kernel");
+        }
         if constexpr (sizeof(T) == 4) {
+            // the wide kernels need 16-byte aligned rows; the others take any 8-byte aligned array
             if (use_wide && wide_aligned(in)) {
                 if (order == 16) { return launch_r2c_wide_split(wide15s, in, out, batch, stream); }
-                return order == 13   ? launch_r2c_wide(wide12, in, out, batch, stream)
-                       : order == 14 ? launch_r2c_wide(wide13, in, out, batch, stream)
-                                     : launch_r2c_wide(wide14, in, out, batch, stream);
+                return order == 14 ? launch_r2c_wide(wide13, in, out, batch, stream) : launch_r2c_wide(wide14, in, out, batch, stream);
             }
-        }
-        if constexpr (sizeof(T) == 4) {
-            if (use_split15) { return launch_r2c_split2<T, 14>(in, out, tables.tw(), tables.rtw(), batch, stream); }
-#ifdef NEO_B200_EXPERIMENTAL_FFT
-            if (use_pair) { return launch_r2c_pair<15>(in, out, tables.tw(), tables.rtw(), batch, stream); }
-            if (use_cluster) { return cluster.forward(in, out, batch, stream); }
-#endif
-        }
-        if constexpr (sizeof(T) == 4) {
             if (use_big_cta) { return launch_r2c<T, 14>(r2c_plain_io<T, 14>{in, out}, tables.tw(), tables.rtw(), batch, stream); }
         }
-        if (use_large) { return large.forward(in, out, batch, stream); }
         if (use_two_pass) { return forward_two_pass(in, out, batch, stream); }
-#ifdef NEO_B200_EXPERIMENTAL_FFT
-        if constexpr (sizeof(T) == 4) {
-            // N = 2^13, 2^14: persistent CTAs fed by TMA bulk copies (fft_stream.cuh); needs 16-byte aligned arrays
-            if (stream_ok(in, out)) {
-                if (order == 13) { return launch_r2c_stream<12>(in, out, tables.tw(), tables.rtw(), batch, stream); }
-                if (order == 14) { return launch_r2c_stream<13>(in, out, tables_full.tw(), tables_full.rtw(), batch, stream); }
-            }
-        }
-#endif
-        if (use_split) {
-            if (order - 1 == k_split_lo) {
-                static bool const one_cta = std::getenv("NEO_B200_R2C_SPLIT14") == nullptr;  // tuning knob: two 4096-point CTAs instead
-                if (one_cta) {
-                    return launch_r2c<T, k_split_lo>(r2c_plain_io<T, k_split_lo>{in, out}, tables_full.tw(), tables_full.rtw(), batch, stream);
-                }
-                return launch_r2c_split2<T, k_split_lo - 1>(in, out, tables.tw(), tables.rtw(), batch, stream);
-            }
-            return launch_r2c_split2<T, k_split_hi - 1>(in, out, tables.tw(), tables.rtw(), batch, stream);
-        }
+        if (use_split) { return launch_r2c_split2<T, k_split - 1>(in, out, tables.tw(), tables.rtw(), batch, stream); }
         int status = NEO_B200_ERR_UNSUPPORTED;
         NEO_DISPATCH_LOGM(T, order - 1, {
             if constexpr (LOGM <= max_cta_logm<T>()) {
@@ -494,49 +404,24 @@ struct rfft_engine
 
     int backward(cx<T> const* in, size_t row_len, T* out, size_t batch, cudaStream_t stream)
     {
-        if (order == 0) { return large_rfft<T>::size_one_backward(in, row_len, out, batch, stream); }
+        if (order == 0) {
+            size_one_c2r_kernel<T><<<static_cast<unsigned>((batch + 255) / 256), 256, 0, stream>>>(in, row_len, out, batch);
+            return check_launch("size_one_c2r_kernel");
+        }
         if constexpr (sizeof(T) == 4) {
+            // the wide kernels need 16-byte aligned rows; the others take any 8-byte aligned array
             if (use_wide && wide_aligned(out)) {
                 if (order == 16) { return launch_c2r_wide_split(wide15s, in, row_len, out, batch, stream); }
-                return order == 13   ? launch_c2r_wide(wide12, in, row_len, out, batch, stream)
-                       : order == 14 ? launch_c2r_wide(wide13, in, row_len, out, batch, stream)
-                                     : launch_c2r_wide(wide14, in, row_len, out, batch, stream);
+                return order == 14 ? launch_c2r_wide(wide13, in, row_len, out, batch, stream)
+                                   : launch_c2r_wide(wide14, in, row_len, out, batch, stream);
             }
-        }
-        if constexpr (sizeof(T) == 4) {
-            if (use_split15) {
-                return launch_c2r_split2<T, 14>(in, row_len, out, tables.tw(), tables.rtw(), w_n.template as<cx<T>>(), batch, stream);
-            }
-#ifdef NEO_B200_EXPERIMENTAL_FFT
-            if (use_pair) { return launch_c2r_pair<15>(in, row_len, out, tables.tw(), tables.rtw(), batch, stream); }
-            if (use_cluster) { return cluster.backward(in, row_len, out, batch, stream); }
-#endif
-        }
-        if constexpr (sizeof(T) == 4) {
             if (use_big_cta) {
                 return launch_c2r<T, 14>(c2r_plain_io<T, 14>{in, out, row_len}, tables.tw(), tables.rtw(), batch, stream);
             }
         }
-        if (use_large) { return large.backward(in, row_len, out, batch, stream); }
         if (use_two_pass) { return backward_two_pass(in, row_len, out, batch, stream); }
-#ifdef NEO_B200_EXPERIMENTAL_FFT
-        if constexpr (sizeof(T) == 4) {
-            if (stream_ok(in, out)) {
-                if (order == 13) { return launch_c2r_stream<12>(in, row_len, out, tables.tw(), tables.rtw(), batch, stream); }
-                if (order == 14) { return launch_c2r_stream<13>(in, row_len, out, tables_full.tw(), tables_full.rtw(), batch, stream); }
-            }
-        }
-#endif
         if (use_split) {
-            auto const* wn = w_n.template as<cx<T>>();
-            if (order - 1 == k_split_lo) {
-                // measured with the register caps in place: two CTAs 0.48-0.49 of HBM peak, one 8192-point CTA 0.44-0.45
-                static bool const one_cta = std::getenv("NEO_B200_C2R_SPLIT14") == nullptr;  // tuning knob: two 4096-point CTAs instead
-                if (!one_cta) { return launch_c2r_split2<T, k_split_lo - 1>(in, row_len, out, tables.tw(), tables.rtw(), wn, batch, stream); }
-                return launch_c2r<T, k_split_lo>(c2r_plain_io<T, k_split_lo>{in, out, row_len}, tables_full.tw(), tables_full.rtw(), batch,
-                                                 stream);
-            }
-            return launch_c2r_split2<T, k_split_hi - 1>(in, row_len, out, tables.tw(), tables.rtw(), wn, batch, stream);
+            return launch_c2r_split2<T, k_split - 1>(in, row_len, out, tables.tw(), tables.rtw(), w_n.template as<cx<T>>(), batch, stream);
         }
         int status = NEO_B200_ERR_UNSUPPORTED;
         NEO_DISPATCH_LOGM(T, order - 1, {

@@ -359,7 +359,7 @@ struct wide_fft
 };
 
 // in: [batch][2M] reals (16-byte aligned), out: [batch][M+1] complex. ta: [LOGP][XS] W_M^(2^p x); tb: [R2][16]; rtw: W_2M^k, k < J/2
-// PF: persistent CTAs, and no warp ever waits on DRAM: the NEXT row travels into shared memory by bulk copies (TMA) while this row is
+// Persistent CTAs, and no warp ever waits on DRAM: the NEXT row travels into shared memory by bulk copies (TMA) while this row is
 // transformed. Its first three quarters go into a staging buffer behind the tile as soon as stage 1 has taken this row's inputs
 // (a whole row time ahead: at the SM's fair share of the HBM bandwidth a row needs about that long); the last quarter goes into the
 // tile itself, which is idle from the stage-3 loads on. Both copies signal one mbarrier (two arrivals per phase).
@@ -380,7 +380,7 @@ struct wide_stage
     __device__ __forceinline__ float2 get(int e) const { return e < ST ? stage[e] : tile[e - ST]; }
 };
 
-template<int LOGM, int LOGR1, int LOGR2, int MINCTAS, bool PF>
+template<int LOGM, int LOGR1, int LOGR2, int MINCTAS>
 __global__ void __launch_bounds__(wide_cfg<LOGM, LOGR1, LOGR2>::NT, MINCTAS)
     r2c_wide_kernel(float const* __restrict__ in, float2* __restrict__ out, float2 const* __restrict__ ta, float2 const* __restrict__ tb,
                     float2 const* __restrict__ rtw, size_t batch)
@@ -396,20 +396,18 @@ __global__ void __launch_bounds__(wide_cfg<LOGM, LOGR1, LOGR2>::NT, MINCTAS)
     unsigned parity = 0;
     using stage_t = wide_stage<M, cfg::ST_FWD>;
     stage_t const st{sm, sm + M};
-    float2* const tbs = sm + M + cfg::ST_FWD;  // stage-2 twiddles in shared memory (PF)
+    float2* const tbs = sm + M + cfg::ST_FWD;  // stage-2 twiddles in shared memory
     auto const zrow = [&](size_t row) { return reinterpret_cast<float2 const*>(in) + row * size_t(M); };
-    if constexpr (PF) {
-        static_assert(!PF || BF1 == 2 || BF1 == 1, "one pass over the staged row");
-        for (int i = t; i < cfg::TB_FWD; i += NT) { tbs[i] = __ldg(tb + i); }
-        if (t == 0) {
-            wtma::init(&bar, 2);
-            if (blockIdx.x < batch) {
-                st.fetch_early(zrow(blockIdx.x), &bar);
-                st.fetch_late(zrow(blockIdx.x), &bar);
-            }
+    static_assert(BF1 == 2 || BF1 == 1, "one pass over the staged row");
+    for (int i = t; i < cfg::TB_FWD; i += NT) { tbs[i] = __ldg(tb + i); }
+    if (t == 0) {
+        wtma::init(&bar, 2);
+        if (blockIdx.x < batch) {
+            st.fetch_early(zrow(blockIdx.x), &bar);
+            st.fetch_late(zrow(blockIdx.x), &bar);
         }
-        __syncthreads();
     }
+    __syncthreads();
 
     for (size_t b = blockIdx.x; b < batch; b += gridDim.x) {
         bool const more = b + gridDim.x < batch;
@@ -419,26 +417,16 @@ __global__ void __launch_bounds__(wide_cfg<LOGM, LOGR1, LOGR2>::NT, MINCTAS)
             for (int m = 0; m < BF1 / 2; ++m) {
                 int const n = 2 * t + 2 * NT * m;  // this thread's butterflies n and n + 1
                 float2 ua[R1], ub[R1];
-                if constexpr (PF) {
-                    wtma::wait(&bar, parity);
-                    parity ^= 1U;
-                    static_for<0, R1>([&](auto n1c) {
-                        constexpr int n1 = decltype(n1c)::value;
-                        float4 const q = *reinterpret_cast<float4 const*>(st.template at<(n1 * S1 >= cfg::ST_FWD)>(n + n1 * S1));
-                        ua[n1]         = make_float2(q.x, q.y);
-                        ub[n1]         = make_float2(q.z, q.w);
-                    });
-                    __syncthreads();  // every thread has its inputs: staging buffer and tile may be overwritten
-                    if (t == 0 && more) { st.fetch_early(zrow(b + gridDim.x), &bar); }
-                } else {
-                    float4 const* const src = reinterpret_cast<float4 const*>(in + b * (2 * size_t(M))) + (n >> 1);
-#pragma unroll
-                    for (int n1 = 0; n1 < R1; ++n1) {
-                        float4 const q = __ldcs(src + n1 * (S1 / 2));
-                        ua[n1]         = make_float2(q.x, q.y);
-                        ub[n1]         = make_float2(q.z, q.w);
-                    }
-                }
+                wtma::wait(&bar, parity);
+                parity ^= 1U;
+                static_for<0, R1>([&](auto n1c) {
+                    constexpr int n1 = decltype(n1c)::value;
+                    float4 const q = *reinterpret_cast<float4 const*>(st.template at<(n1 * S1 >= cfg::ST_FWD)>(n + n1 * S1));
+                    ua[n1]         = make_float2(q.x, q.y);
+                    ub[n1]         = make_float2(q.z, q.w);
+                });
+                __syncthreads();  // every thread has its inputs: staging buffer and tile may be overwritten
+                if (t == 0 && more) { st.fetch_early(zrow(b + gridDim.x), &bar); }
                 wdft<R1, -1>::run(ua);
                 wdft<R1, -1>::run(ub);
                 {
@@ -468,20 +456,14 @@ __global__ void __launch_bounds__(wide_cfg<LOGM, LOGR1, LOGR2>::NT, MINCTAS)
         } else {
             int const n = t;
             float2 u[R1];
-            if constexpr (PF) {
-                wtma::wait(&bar, parity);
-                parity ^= 1U;
-                static_for<0, R1>([&](auto n1c) {
-                    constexpr int n1 = decltype(n1c)::value;
-                    u[n1]            = *st.template at<(n1 * S1 >= cfg::ST_FWD)>(n + n1 * S1);
-                });
-                __syncthreads();
-                if (t == 0 && more) { st.fetch_early(zrow(b + gridDim.x), &bar); }
-            } else {
-                float2 const* const src = reinterpret_cast<float2 const*>(in + b * (2 * size_t(M))) + n;
-#pragma unroll
-                for (int n1 = 0; n1 < R1; ++n1) { u[n1] = __ldcs(src + n1 * S1); }
-            }
+            wtma::wait(&bar, parity);
+            parity ^= 1U;
+            static_for<0, R1>([&](auto n1c) {
+                constexpr int n1 = decltype(n1c)::value;
+                u[n1]            = *st.template at<(n1 * S1 >= cfg::ST_FWD)>(n + n1 * S1);
+            });
+            __syncthreads();
+            if (t == 0 && more) { st.fetch_early(zrow(b + gridDim.x), &bar); }
             wdft<R1, -1>::run(u);
             {
                 float2 w[R1];
@@ -499,8 +481,7 @@ __global__ void __launch_bounds__(wide_cfg<LOGM, LOGR1, LOGR2>::NT, MINCTAS)
         }
         __syncthreads();
         // ---- stage 2, in place
-        if constexpr (PF) { W::template stage2<-1, true>(sm, tbs, t); }
-        else { W::template stage2<-1>(sm, tb, t); }
+        W::template stage2<-1, true>(sm, tbs, t);
         __syncthreads();
         // ---- stage 3 + Hermitian split in registers
         {
@@ -510,9 +491,7 @@ __global__ void __launch_bounds__(wide_cfg<LOGM, LOGR1, LOGR2>::NT, MINCTAS)
             W::load_row(sm4, ja, za);
             W::load_row(sm4, jb, zb);
             __syncthreads();  // the tile is free for the next row
-            if constexpr (PF) {
-                if (t == 0 && more) { st.fetch_late(zrow(b + gridDim.x), &bar); }
-            }
+            if (t == 0 && more) { st.fetch_late(zrow(b + gridDim.x), &bar); }
             dft<16, -1>::run(za);
             dft<16, -1>::run(zb);
             float2* const row = out + b * (size_t(M) + 1);
@@ -526,9 +505,9 @@ __global__ void __launch_bounds__(wide_cfg<LOGM, LOGR1, LOGR2>::NT, MINCTAS)
 }
 
 // in: [batch][row_len] complex (first M+1 used), out: [batch][2M] reals (16-byte aligned), unnormalised. tb: [R1][R2]
-// PF: as in r2c_wide_kernel. A spectrum row of M+1 bins starts on an 8-byte boundary only, so the bulk copies take the M bins from
+// Persistent CTAs fed by bulk copies as in r2c_wide_kernel. A spectrum row of M+1 bins starts on an 8-byte boundary only, so the bulk copies take the M bins from
 // the row's first 16-byte boundary on (bins lo .. lo+M-1, lo = 0 or 1) and thread 0 fetches the one bin left out (X[M] or X[0]).
-template<int LOGM, int LOGR1, int LOGR2, int MINCTAS, bool PF>
+template<int LOGM, int LOGR1, int LOGR2, int MINCTAS>
 __global__ void __launch_bounds__(wide_cfg<LOGM, LOGR1, LOGR2>::NT, MINCTAS)
     c2r_wide_kernel(float2 const* __restrict__ in, size_t row_len, float* __restrict__ out, float2 const* __restrict__ ta,
                     float2 const* __restrict__ tb, float2 const* __restrict__ rtw, size_t batch)
@@ -551,17 +530,15 @@ __global__ void __launch_bounds__(wide_cfg<LOGM, LOGR1, LOGR2>::NT, MINCTAS)
         float2 const* const x = in + row * row_len;
         return x + ((reinterpret_cast<std::uintptr_t>(x) >> 3) & 1U);
     };
-    if constexpr (PF) {
-        for (int i = t; i < cfg::TB_BWD; i += NT) { tbs[i] = __ldg(tb + i); }
-        if (t == 0) {
-            wtma::init(&bar, 2);
-            if (blockIdx.x < batch) {
-                st.fetch_early(xrow(blockIdx.x), &bar);
-                st.fetch_late(xrow(blockIdx.x), &bar);
-            }
+    for (int i = t; i < cfg::TB_BWD; i += NT) { tbs[i] = __ldg(tb + i); }
+    if (t == 0) {
+        wtma::init(&bar, 2);
+        if (blockIdx.x < batch) {
+            st.fetch_early(xrow(blockIdx.x), &bar);
+            st.fetch_late(xrow(blockIdx.x), &bar);
         }
-        __syncthreads();
     }
+    __syncthreads();
 
     for (size_t b = blockIdx.x; b < batch; b += gridDim.x) {
         bool const more = b + gridDim.x < batch;
@@ -572,37 +549,29 @@ __global__ void __launch_bounds__(wide_cfg<LOGM, LOGR1, LOGR2>::NT, MINCTAS)
             float2 const wt = __ldg(rtw + t);
             float2 za[16], zb[16];
             float nyq = 0.0F;
-            if constexpr (PF) {
-                int const lo = int(xrow(b) - x);
-                float2 edge  = make_float2(0.0F, 0.0F);
-                if (t == 0) { edge = x[lo ? 0 : M]; }
-                wtma::wait(&bar, parity);
-                parity ^= 1U;
-                // bin k sits at staged element k - lo. For t > 0 both ja + J k3 - lo and jb + J k3 - lo stay inside [J k3, J (k3 + 1)),
-                // so the region follows from k3 alone (the staging boundary is K3T J)
-                if (t != 0) {
-                    static_for<0, 16>([&](auto k3c) {
-                        constexpr int k3 = decltype(k3c)::value;
-                        za[k3]           = *st.template at<(k3 >= K3T)>(ja + J * k3 - lo);
-                        zb[k3]           = *st.template at<(k3 >= K3T)>(jb + J * k3 - lo);
-                    });
-                } else {
-#pragma unroll
-                    for (int k3 = 1; k3 < 16; ++k3) { za[k3] = st.get(J * k3 - lo); }
-#pragma unroll
-                    for (int k3 = 0; k3 < 16; ++k3) { zb[k3] = st.get(J / 2 + J * k3 - lo); }
-                    za[0] = lo ? edge : st.get(0);
-                    nyq   = lo ? st.get(M - 1).x : edge.x;
-                }
-                __syncthreads();  // every thread has its inputs: staging buffer and tile may be overwritten
-                if (t == 0 && more) { st.fetch_early(xrow(b + gridDim.x), &bar); }
+            int const lo = int(xrow(b) - x);
+            float2 edge  = make_float2(0.0F, 0.0F);
+            if (t == 0) { edge = x[lo ? 0 : M]; }
+            wtma::wait(&bar, parity);
+            parity ^= 1U;
+            // bin k sits at staged element k - lo. For t > 0 both ja + J k3 - lo and jb + J k3 - lo stay inside [J k3, J (k3 + 1)),
+            // so the region follows from k3 alone (the staging boundary is K3T J)
+            if (t != 0) {
+                static_for<0, 16>([&](auto k3c) {
+                    constexpr int k3 = decltype(k3c)::value;
+                    za[k3]           = *st.template at<(k3 >= K3T)>(ja + J * k3 - lo);
+                    zb[k3]           = *st.template at<(k3 >= K3T)>(jb + J * k3 - lo);
+                });
             } else {
 #pragma unroll
-                for (int k3 = 0; k3 < 16; ++k3) { za[k3] = __ldcs(x + ja + J * k3); }
+                for (int k3 = 1; k3 < 16; ++k3) { za[k3] = st.get(J * k3 - lo); }
 #pragma unroll
-                for (int k3 = 0; k3 < 16; ++k3) { zb[k3] = __ldcs(x + jb + J * k3); }
-                nyq = t == 0 ? x[M].x : 0.0F;
+                for (int k3 = 0; k3 < 16; ++k3) { zb[k3] = st.get(J / 2 + J * k3 - lo); }
+                za[0] = lo ? edge : st.get(0);
+                nyq   = lo ? st.get(M - 1).x : edge.x;
             }
+            __syncthreads();  // every thread has its inputs: staging buffer and tile may be overwritten
+            if (t == 0 && more) { st.fetch_early(xrow(b + gridDim.x), &bar); }
             wide_c2r_pre<M>(za, zb, t, wt, nyq);
             dft<16, +1>::run(za);
             dft<16, +1>::run(zb);
@@ -620,8 +589,7 @@ __global__ void __launch_bounds__(wide_cfg<LOGM, LOGR1, LOGR2>::NT, MINCTAS)
         }
         __syncthreads();
         // ---- stage 2', in place
-        if constexpr (PF) { W::template stage2<+1, true>(sm, tbs, t); }
-        else { W::template stage2<+1>(sm, tb, t); }
+        W::template stage2<+1, true>(sm, tbs, t);
         __syncthreads();
         // ---- stage 1'
         if constexpr (BF1 >= 2) {
@@ -638,9 +606,7 @@ __global__ void __launch_bounds__(wide_cfg<LOGM, LOGR1, LOGR2>::NT, MINCTAS)
                 }
                 if (m == BF1 / 2 - 1) {
                     __syncthreads();  // the tile is free for the next row
-                    if constexpr (PF) {
-                        if (t == 0 && more) { st.fetch_late(xrow(b + gridDim.x), &bar); }
-                    }
+                    if (t == 0 && more) { st.fetch_late(xrow(b + gridDim.x), &bar); }
                 }
                 wdft<R1, +1>::run(ua);
                 wdft<R1, +1>::run(ub);
@@ -654,9 +620,7 @@ __global__ void __launch_bounds__(wide_cfg<LOGM, LOGR1, LOGR2>::NT, MINCTAS)
 #pragma unroll
             for (int k1 = 0; k1 < R1; ++k1) { u[k1] = sm[(k1 * R2 + a2) * 16 + ((((a >> 1) ^ (k1 & 7)) << 1) | (a & 1))]; }
             __syncthreads();
-            if constexpr (PF) {
-                if (t == 0 && more) { st.fetch_late(xrow(b + gridDim.x), &bar); }
-            }
+            if (t == 0 && more) { st.fetch_late(xrow(b + gridDim.x), &bar); }
             wdft<R1, +1>::run(u);
             float2* const dst = reinterpret_cast<float2*>(out + b * (2 * size_t(M))) + n;
 #pragma unroll
@@ -954,89 +918,12 @@ __global__ void __launch_bounds__(wide_cfg<LOGM2, LOGR1, LOGR2>::NT, 1)
     }
 }
 
-// ---- one WARP per transform (M = 1024: the convolver's 2048-point real transforms), load / store sides as policy objects like
-// r2c_kernel / c2r_kernel. The three stages only need __syncwarp(): warps never wait for each other, so their load, butterfly and
-// store phases drift apart and overlap. Policies provide (besides open / store / store_edges / load / load_edges of the narrow
-// kernels) the 128-bit accesses of the real side: load_pair<HI>(row, j), keep_pair(row, j, v), store_pair<HI>(row, j, z0, z1) with j
-// an even index inside the lower (HI = false) or upper half of the real row's complex pairs.
-template<int LOGM, int LOGR1, int LOGR2, int G, class IO, int MINB = 512 / (32 * G)>
-__global__ void __launch_bounds__(32 * G, MINB)
-    r2c_wide_io_kernel(IO io, float2 const* __restrict__ ta, float2 const* __restrict__ tb, float2 const* __restrict__ rtw, size_t batch)
-{
-    using W   = wide_fft<LOGM, LOGR1, LOGR2>;
-    using cfg = wide_cfg<LOGM, LOGR1, LOGR2>;
-    constexpr int M = cfg::M, R1 = cfg::R1, R2 = cfg::R2, NT = cfg::NT, S1 = cfg::S1, J = cfg::J, BF1 = cfg::BF1, XS = cfg::XS, H = M / 2;
-    static_assert(NT == 32 && BF1 >= 2, "one warp per transform, pairs of stage-1 butterflies");
-    extern __shared__ __align__(128) unsigned char wide_smem_raw[];
-    int const t      = threadIdx.x & 31;
-    size_t const b   = size_t(blockIdx.x) * G + (threadIdx.x >> 5);
-    if (b >= batch) { return; }  // whole warps leave: nothing below synchronises across warps
-    float2* const sm  = reinterpret_cast<float2*>(wide_smem_raw) + (threadIdx.x >> 5) * M;
-    float4* const sm4 = reinterpret_cast<float4*>(sm);
-    typename IO::row_state const row = io.open(b);
-
-    // the whole row first (all of a thread's 128-bit loads in flight together), then the stage-1 passes
-    float4 q[BF1 / 2][R1];
-#pragma unroll
-    for (int m = 0; m < BF1 / 2; ++m) {
-        int const n = 2 * t + 2 * NT * m;
-        static_for<0, R1>([&](auto n1c) {
-            constexpr int n1 = decltype(n1c)::value;
-            if constexpr (n1 < R1 / 2) { q[m][n1] = io.template load_pair<false>(row, n + S1 * n1); }
-            else { q[m][n1] = io.template load_pair<true>(row, n + S1 * n1 - H); }
-        });
-    }
-#pragma unroll
-    for (int m = 0; m < BF1 / 2; ++m) {
-        int const n = 2 * t + 2 * NT * m;
-        float2 ua[R1], ub[R1];
-#pragma unroll
-        for (int n1 = 0; n1 < R1; ++n1) {
-            if (n1 >= R1 / 2) { io.keep_pair(row, n + S1 * n1 - H, q[m][n1]); }
-            ua[n1] = make_float2(q[m][n1].x, q[m][n1].y);
-            ub[n1] = make_float2(q[m][n1].z, q[m][n1].w);
-        }
-        wdft<R1, -1>::run(ua);
-        wdft<R1, -1>::run(ub);
-        {
-            float4 const* const ta4 = reinterpret_cast<float4 const*>(ta) + (n >> 1);
-            float2 wa[R1], wb[R1];
-#pragma unroll
-            for (int q = 1; q < R1; ++q) {
-                int const hi = 1 << (31 - __clz(q));
-                if (q == hi) {
-                    float4 const w4 = __ldg(ta4 + (31 - __clz(q)) * (XS / 2));
-                    wa[q]           = make_float2(w4.x, w4.y);
-                    wb[q]           = make_float2(w4.z, w4.w);
-                } else {
-                    wa[q] = cmul(wa[hi], wa[q - hi]);
-                    wb[q] = cmul(wb[hi], wb[q - hi]);
-                }
-                ua[q] = cmul(ua[q], wa[q]);
-                ub[q] = cmul(ub[q], wb[q]);
-            }
-        }
-        int const a2 = n >> 4, ah = (n & 15) >> 1;
-#pragma unroll
-        for (int k1 = 0; k1 < R1; ++k1) { sm4[(k1 * R2 + a2) * 8 + (ah ^ (k1 & 7))] = make_float4(ua[k1].x, ua[k1].y, ub[k1].x, ub[k1].y); }
-    }
-    __syncwarp();
-    W::template stage2<-1>(sm, tb, t);
-    __syncwarp();
-    {
-        int const ja = t, jb = t == 0 ? J / 2 : J - t;
-        float2 const wt = __ldg(rtw + t);
-        float2 za[16], zb[16];
-        W::load_row(sm4, ja, za);
-        W::load_row(sm4, jb, zb);
-        dft<16, -1>::run(za);
-        dft<16, -1>::run(zb);
-        wide_r2c_post<M>(za, zb, t, wt, [&](int k, float2 x) { io.store(row, k, x); },
-                         [&](float dc, float nyq) { io.store_edges(row, dc, nyq); });
-    }
-}
-
-template<int LOGM, int LOGR1, int LOGR2, int G, class IO, int MINB = 512 / (32 * G)>
+// ---- inverse transform with one WARP per transform (M = 1024: the convolver's 2048-point real transforms), load / store sides as
+// policy objects like c2r_kernel. The three stages only need __syncwarp(): warps never wait for each other, so their load, butterfly
+// and store phases drift apart and overlap. Policies provide (besides open / load of the narrow kernel) the 128-bit stores of the
+// real side: store_pair<HI>(row, j, z0, z1) with j an even index inside the lower (HI = false) or upper half of the real row's
+// complex pairs. MINB: resident CTAs per SM the kernel is compiled for (5: 96 registers).
+template<int LOGM, int LOGR1, int LOGR2, int G, class IO, int MINB>
 __global__ void __launch_bounds__(32 * G, MINB)
     c2r_wide_io_kernel(IO io, float2 const* __restrict__ ta, float2 const* __restrict__ tb, float2 const* __restrict__ rtw, size_t batch)
 {
@@ -1099,54 +986,16 @@ __global__ void __launch_bounds__(32 * G, MINB)
     }
 }
 
-// minb: resident CTAs per SM the kernel is compiled for (4 = 128 registers, 5 = 96, 6 = 80: more warps to hide the loads behind, at the
-// price of spills) -- a measured choice per direction, see conv_engine
 template<int LOGM, int LOGR1, int LOGR2, class IO>
-int launch_r2c_wide_io(IO const& io, float2 const* ta, float2 const* tb, float2 const* rtw, size_t batch, cudaStream_t stream, int minb = 4)
+int launch_c2r_wide_io(IO const& io, float2 const* ta, float2 const* tb, float2 const* rtw, size_t batch, cudaStream_t stream)
 {
     using cfg       = wide_cfg<LOGM, LOGR1, LOGR2>;
     constexpr int G = 4;
     if (batch == 0) { return NEO_B200_OK; }
-    auto const go = [&](auto kernel) {
-        NEO_TRY(enable_smem(kernel, G * cfg::SMEM));
-        kernel<<<unsigned((batch + G - 1) / G), 32 * G, G * cfg::SMEM, stream>>>(io, ta, tb, rtw, batch);
-        return check_launch("r2c_wide_io_kernel");
-    };
-    if (minb == 5) { return go(r2c_wide_io_kernel<LOGM, LOGR1, LOGR2, G, IO, 5>); }
-    if (minb == 6) { return go(r2c_wide_io_kernel<LOGM, LOGR1, LOGR2, G, IO, 6>); }
-    return go(r2c_wide_io_kernel<LOGM, LOGR1, LOGR2, G, IO, 4>);
-}
-
-// the most resident CTAs a c2r policy may be compiled for: IO::wide_max_minb where a policy sets it (a policy whose store needs more
-// registers than 80 without spilling), else 6; a larger request runs at that bound
-template<class IO, class = void>
-struct wide_max_minb
-{
-    static constexpr int value = 6;
-};
-template<class IO>
-struct wide_max_minb<IO, std::void_t<decltype(IO::wide_max_minb)>>
-{
-    static constexpr int value = IO::wide_max_minb;
-};
-
-template<int LOGM, int LOGR1, int LOGR2, class IO>
-int launch_c2r_wide_io(IO const& io, float2 const* ta, float2 const* tb, float2 const* rtw, size_t batch, cudaStream_t stream, int minb = 4)
-{
-    using cfg       = wide_cfg<LOGM, LOGR1, LOGR2>;
-    constexpr int G = 4;
-    if (batch == 0) { return NEO_B200_OK; }
-    auto const go = [&](auto kernel) {
-        NEO_TRY(enable_smem(kernel, G * cfg::SMEM));
-        kernel<<<unsigned((batch + G - 1) / G), 32 * G, G * cfg::SMEM, stream>>>(io, ta, tb, rtw, batch);
-        return check_launch("c2r_wide_io_kernel");
-    };
-    if constexpr (wide_max_minb<IO>::value < 6) { minb = std::min(minb, wide_max_minb<IO>::value); }
-    if (minb == 5) { return go(c2r_wide_io_kernel<LOGM, LOGR1, LOGR2, G, IO, 5>); }
-    if constexpr (wide_max_minb<IO>::value >= 6) {
-        if (minb == 6) { return go(c2r_wide_io_kernel<LOGM, LOGR1, LOGR2, G, IO, 6>); }
-    }
-    return go(c2r_wide_io_kernel<LOGM, LOGR1, LOGR2, G, IO, 4>);
+    auto kernel = c2r_wide_io_kernel<LOGM, LOGR1, LOGR2, G, IO, 5>;
+    NEO_TRY(enable_smem(kernel, G * cfg::SMEM));
+    kernel<<<unsigned((batch + G - 1) / G), 32 * G, G * cfg::SMEM, stream>>>(io, ta, tb, rtw, batch);
+    return check_launch("c2r_wide_io_kernel");
 }
 
 // ---- tables + launchers --------------------------------------------------------------------------------------------------------------
@@ -1211,16 +1060,8 @@ constexpr int wide_min_ctas()
     return n > 0 ? n : 1;
 }
 
-// NEO_B200_WIDE_NO_PREFETCH: one CTA per row with plain global loads instead of persistent CTAs fed by bulk copies (A/B knob)
-inline bool wide_prefetch()
+inline unsigned wide_grid(size_t batch, int ctas_per_sm)
 {
-    static bool const on = std::getenv("NEO_B200_WIDE_NO_PREFETCH") == nullptr;
-    return on;
-}
-
-inline unsigned wide_grid(size_t batch, int ctas_per_sm, bool persist)
-{
-    if (!persist) { return unsigned(batch); }
     int dev = 0, sms = 148;
     cudaGetDevice(&dev);
     cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
@@ -1233,11 +1074,9 @@ int launch_r2c_wide(wide_tables<LOGM, LOGR1, LOGR2> const& tb, float const* in, 
     using cfg = wide_cfg<LOGM, LOGR1, LOGR2>;
     if (batch == 0) { return NEO_B200_OK; }
     constexpr int ctas = wide_min_ctas<LOGM, LOGR1, LOGR2>();
-    bool const pf      = wide_prefetch();
-    auto kernel        = pf ? r2c_wide_kernel<LOGM, LOGR1, LOGR2, ctas, true> : r2c_wide_kernel<LOGM, LOGR1, LOGR2, ctas, false>;
-    size_t const smem = pf ? cfg::SMEM_PF : cfg::SMEM;
-    NEO_TRY(enable_smem(kernel, smem));
-    kernel<<<wide_grid(batch, ctas, pf), cfg::NT, smem, stream>>>(in, out, tb.ta.template as<float2>(), tb.tb_fwd.template as<float2>(),
+    auto kernel        = r2c_wide_kernel<LOGM, LOGR1, LOGR2, ctas>;
+    NEO_TRY(enable_smem(kernel, cfg::SMEM_PF));
+    kernel<<<wide_grid(batch, ctas), cfg::NT, cfg::SMEM_PF, stream>>>(in, out, tb.ta.template as<float2>(), tb.tb_fwd.template as<float2>(),
                                                                        tb.rtw.template as<float2>(), batch);
     return check_launch("r2c_wide_kernel");
 }
@@ -1249,12 +1088,9 @@ int launch_c2r_wide(wide_tables<LOGM, LOGR1, LOGR2> const& tb, float2 const* in,
     using cfg = wide_cfg<LOGM, LOGR1, LOGR2>;
     if (batch == 0) { return NEO_B200_OK; }
     constexpr int ctas = wide_min_ctas<LOGM, LOGR1, LOGR2>();
-    // the bulk copy wants the first 16-byte boundary of every row inside it and 8-byte aligned rows
-    bool const pf = wide_prefetch() && (reinterpret_cast<std::uintptr_t>(in) & 7U) == 0;
-    auto kernel   = pf ? c2r_wide_kernel<LOGM, LOGR1, LOGR2, ctas, true> : c2r_wide_kernel<LOGM, LOGR1, LOGR2, ctas, false>;
-    size_t const smem = pf ? cfg::SMEM_PF : cfg::SMEM;
-    NEO_TRY(enable_smem(kernel, smem));
-    kernel<<<wide_grid(batch, ctas, pf), cfg::NT, smem, stream>>>(in, row_len, out, tb.ta.template as<float2>(),
+    auto kernel        = c2r_wide_kernel<LOGM, LOGR1, LOGR2, ctas>;
+    NEO_TRY(enable_smem(kernel, cfg::SMEM_PF));
+    kernel<<<wide_grid(batch, ctas), cfg::NT, cfg::SMEM_PF, stream>>>(in, row_len, out, tb.ta.template as<float2>(),
                                                                        tb.tb_bwd.template as<float2>(), tb.rtw.template as<float2>(), batch);
     return check_launch("c2r_wide_kernel");
 }

@@ -47,8 +47,7 @@ def test_rfft_irfft_match_oracle_every_order(gpu, orc, real, cplx):
 @pytest.mark.parametrize("order,batch", [(13, 701), (14, 333), (14, 1201), (15, 301), (15, 610), (16, 151)])
 def test_long_rfft_many_rows(gpu, orc, order, batch):
     # N = 2^13 / 2^14 (512-thread CTAs, two per SM): more rows than one wave of CTAs, odd and even rows (spectrum rows of N/2+1 bins
-    # alternate between 16-byte aligned and not), and N-long spectrum rows on the way back. Also the parity test of the TMA-staged
-    # persistent form (fft_stream.cuh) when the library is built with EXTRA=-DNEO_B200_EXPERIMENTAL_FFT and run with NEO_B200_STREAM=1.
+    # alternate between 16-byte aligned and not), and N-long spectrum rows on the way back.
     n = 1 << order
     x = np.stack([orc.noise(n, 2 + (b % 5), np.float32) * np.float32(1 + b % 3) for b in range(batch)])
     base = orc.rfft(x[:15])
@@ -184,19 +183,30 @@ def test_long_transforms_four_step(gpu, orc, order):
     rp.close()
 
 
-@pytest.mark.parametrize("knob", ["NEO_B200_NO_SPLIT15", None])
-def test_every_form_of_the_65536_point_rfft(gpu, orc, monkeypatch, knob):
-    # four implementations of N = 2^16 exist (fft_plan.cu, rfft_engine::init lists what each measured); the shipped one is two
-    # 2^14-point CTAs, the others are selected by environment knobs when the plan is created -- all must agree with the oracle
-    if knob is not None:
-        monkeypatch.setenv(knob, "1")
-    n = 1 << 16
-    x = np.stack([orc.noise(n, 40 + b, np.float32) for b in range(3)])
-    rp = gpu.RFFTPlan(16, np.float32)
-    S = rp.rfft(x)
-    assert rel_l2(S, orc.rfft(x)) <= 1e-5
-    assert rel_l2(rp.irfft(S) / n, x) <= 1e-5
-    rp.close()
+@pytest.mark.parametrize("order", [14, 15, 16])
+def test_long_rfft_device_rows_aligned_and_at_8_bytes(gpu, orc, order):
+    # float N = 2^14 .. 2^16 has two forms, chosen by the alignment of the real rows: the wide kernels (fft_wide.cuh) need 16 bytes, rows
+    # that are only 8-byte aligned take the cta_fft kernels (one 8192-point CTA, one 1024-thread CTA, two 2^14-point CTAs). Real rows
+    # are read and written as complex pairs, so an offset of two floats is the smallest one a device array may have.
+    import torch
+
+    n, batch = 1 << order, 3
+    x = np.stack([orc.noise(n, 40 + b, np.float32) for b in range(batch)])
+    want = orc.rfft(x)
+    plan = gpu.RFFTPlan(order, np.float32)
+    plan.set_stream(torch.cuda.current_stream())
+    spec = torch.from_numpy(want.astype(np.complex64)).cuda()
+    for offset in (0, 2):
+        rows = torch.empty(batch * n + offset, device="cuda")[offset:].view(batch, n)
+        back = torch.empty(batch * n + offset, device="cuda")[offset:].view(batch, n)
+        assert rows.data_ptr() % 16 == back.data_ptr() % 16 == 4 * offset
+        rows.copy_(torch.from_numpy(x))
+        got = plan.rfft(rows)
+        plan.irfft(spec, out=back)
+        torch.cuda.synchronize()
+        assert rel_l2(got.cpu().numpy(), want) <= 1e-5, (order, offset)
+        assert rel_l2(back.cpu().numpy(), orc.irfft(want, n)) <= 1e-5, (order, offset)
+    plan.close()
 
 
 @pytest.mark.parametrize("real,cplx", CASES)

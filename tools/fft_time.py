@@ -14,4 +14,4 @@ a.record()
 for _ in range(10): plan.rfft(x, out=spec)
 b.record(); torch.cuda.synchronize()
 ms = a.elapsed_time(b) / 10
-print(f"order {order} dbg {os.environ.get('NEO_B200_CLUSTER_DBG','0')}: {ms*1e3:.0f} us, {batch*(4*n+8*(n//2+1))/ms/1e6:.0f} GB/s")
+print(f"order {order}: {ms*1e3:.0f} us, {batch*(4*n+8*(n//2+1))/ms/1e6:.0f} GB/s")
